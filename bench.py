@@ -2,7 +2,7 @@
 """bench.py -- throughput of the grid smoke step (BASELINE.json metric: grid cell-updates/s and % of the
 HBM roofline) on N B200s, with the CPU restatement of the reference timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|c2|c2s|c3|c4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|c2|c2s|c3|c4] [--dump-outputs DIR]
 
 The printed line is the c2 measurement (BASELINE.json configs[1], the configuration the metric is quoted on):
 batched dataset generation, 256 independent 128x128 sequences per GPU, 40 Jacobi sweeps per time step, 20 time
@@ -344,11 +344,36 @@ class Ctx:
         return -self.max_over_ranks(-x)
 
 
-def timed_passes(ctx, device_step, e2e_step, steps, warmup, count_launches, flush_l2=False):
+DUMP_MAX_VALUES = 1 << 20          # per dumped array over all ranks (4 MB of fp32): --workload all dumps 14 arrays, 56 MB at most
+
+
+def dump_sample(t, max_values=DUMP_MAX_VALUES):
+    """A [..., cols] tensor on the host as fp32; above max_values values, the rows of a fixed seeded sample (sorted row
+    indices of the [-1, cols] view, the same for the same shape in every run)."""
+    import torch
+    cols = t.shape[-1]
+    if t.numel() <= max_values:
+        return t.float().cpu().numpy()
+    rows = t.flatten(0, -2)
+    idx = np.sort(np.random.default_rng(0).choice(rows.shape[0], max(1, max_values // cols), replace=False))
+    return rows.index_select(0, torch.from_numpy(idx).to(rows.device)).float().cpu().numpy()
+
+
+def dump_outputs(ctx, key, arrays):
+    """--dump-outputs: DIR/<workload>_<name>.npy (<workload>_rank<r>_<name>.npy on several GPUs, each rank within an equal
+    share of DUMP_MAX_VALUES) for every array."""
+    os.makedirs(ctx.args.dump_outputs, exist_ok=True)
+    prefix = key if ctx.world == 1 else "%s_rank%d" % (key, ctx.rank)
+    for name, t in arrays.items():
+        np.save(os.path.join(ctx.args.dump_outputs, "%s_%s.npy" % (prefix, name)), dump_sample(t, DUMP_MAX_VALUES // ctx.world))
+
+
+def timed_passes(ctx, device_step, e2e_step, steps, warmup, count_launches, flush_l2=False, after_timed=None):
     """The three measurement passes of one workload: device-resident throughput (CUDA events, max over ranks), the same
     steps once more with an event pair around every launch, and the end-to-end pass through the public API.
     flush_l2: the working set fits the L2, so a 256 MB buffer is written before every bench step (outside the events /
-    the clock: each step is then timed on its own and the times are added up)."""
+    the clock: each step is then timed on its own and the times are added up).
+    after_timed: called once right after the timed steps, before anything else runs on the state they left."""
     torch, _lib = ctx.torch, ctx._lib
     flush = torch.empty(64 << 20, dtype=torch.float32, device=ctx.dev) if flush_l2 else None
     for _ in range(warmup):
@@ -379,6 +404,8 @@ def timed_passes(ctx, device_step, e2e_step, steps, warmup, count_launches, flus
         ctx.barrier()
         ms = ctx.max_over_ranks(sum(a.elapsed_time(b) for a, b in evs))
     launches = count_launches() - n0
+    if after_timed is not None:
+        after_timed()
     # per-kernel shares: events around every launch (cannot be recorded inside a replayed graph: always eager)
     ctx.barrier()
     _lib.profile_begin(max_records=launches + 64)
@@ -525,9 +552,13 @@ def run_batched(ctx, key, steps, warmup):
     def e2e_step():
         return sim.generate_sequences(emitter_lists, T, to_host=True)      # returns after the last D2H copy
 
+    def dump():
+        dump_outputs(ctx, key, {"frames": frames[..., :w], "u": ns.u, "v": ns.v, "p": ns.p, "density": ns.density})
+
     ws = ns._arena.numel() * 4 + frames.numel() * 4
     fits_l2 = ws < L2_MB * 1e6
-    ms, launches, prof, clk, e2e_s, host_frames = timed_passes(ctx, device_step, e2e_step, steps, warmup, _lib.launch_count, flush_l2=fits_l2)
+    ms, launches, prof, clk, e2e_s, host_frames = timed_passes(ctx, device_step, e2e_step, steps, warmup, _lib.launch_count, flush_l2=fits_l2,
+                                                               after_timed=dump if args.dump_outputs else None)
     total_cells = ctx.world * B * h * w * T
     value = total_cells * steps / (ms * 1e-3)
     d2h_bytes = T * B * h * L.pitch_c * 4
@@ -646,7 +677,11 @@ def run_slab(ctx, key, steps, warmup):
             copied[k].record(copy_stream)
         return host_bufs[k].unsqueeze(0)          # complete after the synchronize that ends the timed region
 
-    ms, launches, prof, clk, e2e_s, host = timed_passes(ctx, device_step, e2e_step, steps, warmup, _lib.launch_count)
+    def dump():
+        dump_outputs(ctx, key, {name: slab.owned(k) for k, name in (("u", "u"), ("v", "v"), ("p", "p"), ("d", "density"))})
+
+    ms, launches, prof, clk, e2e_s, host = timed_passes(ctx, device_step, e2e_step, steps, warmup, _lib.launch_count,
+                                                        after_timed=dump if args.dump_outputs else None)
     slab.check()
     total_cells = h * w * T
     value = total_cells * steps / (ms * 1e-3)
@@ -745,8 +780,15 @@ def main():
                          "ncclSend/ncclRecv groups issued from C, auto = peer when every neighbour is peer-accessible")
     ap.add_argument("--step-kernel", default="auto", choices=["auto", "phases", "fused"],
                     help="auto: whole simulation on one SM for grids <= 128x128 (k_step_fused), else one kernel per phase")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="right after the timed steps of each workload, write what its last timed "
+                    "step left as DIR/<workload>_<name>.npy in fp32: c2 / c3 the frames and the u, v, p, density state of every "
+                    "sequence, c4 the u, v, p, density rows of the grid; an array of more than %d values as a fixed seeded sample "
+                    "of its rows (on N GPUs every rank writes its own files, within 1/N of that).  The inputs are seeded, so two builds run with the same arguments can be compared file by file"
+                    % DUMP_MAX_VALUES)
     args = ap.parse_args()
     main_key = "c2" if args.workload == "all" else args.workload
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes what the GPU path computed; --impl reference has none")
     if args.impl == "reference":
         return reference_arm(args, main_key)
     if args.warmup < 3:
@@ -754,7 +796,6 @@ def main():
 
     ctx = Ctx(args)
     world, rank = ctx.world, ctx.rank
-    sub_steps = min(args.steps, 20)
     if main_key == "c4":
         out = run_slab(ctx, "c4", args.steps, args.warmup)
     elif main_key == "c2s" and world == 1:
@@ -764,11 +805,11 @@ def main():
     if args.workload == "all":
         also = {}
         if world > 1:
-            also["c2_strong"] = run_batched(ctx, "c2s", sub_steps, args.warmup)
+            also["c2_strong"] = run_batched(ctx, "c2s", args.steps, args.warmup)
         else:
             also["c2_strong"] = {"same_as": "the main line: at N = 1 the 256 sequences of configs[1] are the 256 sequences per GPU"}
-            also["c3"] = run_batched(ctx, "c3", sub_steps, args.warmup)
-        also["c4"] = run_slab(ctx, "c4", sub_steps, args.warmup)
+            also["c3"] = run_batched(ctx, "c3", args.steps, args.warmup)
+        also["c4"] = run_slab(ctx, "c4", args.steps, args.warmup)
         if world > 1:
             also["c3"] = {"skipped": "one 1024x1024 grid does not shard: measured at N = 1 only"}
         out["also"] = also
