@@ -13,7 +13,9 @@
  *     smk_last_error_string() (thread-local) describes the last failure; nothing throws or exits
  *   - all work is enqueued asynchronously on `stream` (a cudaStream_t passed as void*); no hidden syncs
  *   - fields are fp32, row-major [row=y][col=x] with an element pitch that is a multiple of 4 and a
- *     16-byte aligned base (float4 access); `batch` independent simulations are `stride_*` elements apart
+ *     16-byte aligned base (float4 access); `batch` independent simulations are `stride_*` elements apart.
+ *     The frames of smk_step_ex / smk_run_steps_ex may be f16 or bf16 instead (SMK_FRAME_*): same layout,
+ *     pitch and strides counted in elements of the frame type, base aligned to 4 such elements
  *   - arithmetic follows the reference's fp32 association with no FMA contraction (built -fmad=false),
  *     true division for /dt, so results are bit-identical to the reference's CPU path
  */
@@ -182,6 +184,18 @@ SMK_API int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* p
 SMK_API int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
                   float* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
                   const float* fmul, void* stream);
+/*     the same with the frames in another element type: frame_format SMK_FRAME_F32 (what smk_step / smk_run_steps write),
+ *     SMK_FRAME_F16 or SMK_FRAME_BF16.  A half-precision frame element is the fp32 one rounded once to nearest-even
+ *     (overflow gives +-inf, subnormals are kept), converted in the kernel that writes the frame: no extra launch, and
+ *     the state is bit-identical whatever the format.  frame / frames: base aligned to 4 elements of the frame type;
+ *     strides in elements of that type, multiples of 4.  A format outside the enum or a misaligned frame is SMK_EINVAL,
+ *     before anything is enqueued. */
+enum { SMK_FRAME_F32 = 0, SMK_FRAME_F16 = 1, SMK_FRAME_BF16 = 2 };
+SMK_API int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
+                        void* frame, int64_t frame_stride, const float* fmul, int32_t frame_format, void* stream);
+SMK_API int smk_run_steps_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                             void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                             const float* fmul, int32_t frame_format, void* stream);
 /*     1 when a call of nsteps steps (smk_step: 1) would take the fused single-launch path for this grid and params */
 SMK_API int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nsteps, int32_t* fused_host);
 /* Host-only (no GPU needed): the time-sliced schedule smk_run_steps gives the fused kernel when `nsims` simulations of

@@ -6,6 +6,8 @@ import ctypes as C
 import os
 import threading
 
+import torch
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 SO_PATH = os.path.join(_HERE, "libsmoke_sm100.so")
 
@@ -39,6 +41,17 @@ class Params(C.Structure):                   # smk_params_t
 
 
 STEP_KERNELS = {"auto": 0, "phases": 1, "fused": 2}           # SMK_STEP_AUTO / _PHASES / _FUSED
+
+# element type of the frames smk_step_ex / smk_run_steps_ex write: SMK_FRAME_F32 / _F16 / _BF16
+FRAME_FORMATS = {torch.float32: 0, torch.float16: 1, torch.bfloat16: 2}
+
+
+def frame_format(dtype):
+    """SMK_FRAME_* code of a torch dtype; ValueError for anything but float32, float16 and bfloat16."""
+    fmt = FRAME_FORMATS.get(dtype)
+    if fmt is None:
+        raise ValueError("frame dtype must be one of torch.float32, torch.float16, torch.bfloat16; got %r" % (dtype,))
+    return fmt
 
 
 class HaloBlock(C.Structure):                # smk_halo_block_t
@@ -77,6 +90,8 @@ SIGNATURES = {
     "smk_advect_slab": [GP, c_p, c_p, c_i32, c_i32, c_i32, c_p, c_p, c_f, c_f, C.POINTER(SlabCheck), c_p],
     "smk_step": [GP, SP, PP, c_p, c_i64, c_p, c_p],
     "smk_run_steps": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_p],
+    "smk_step_ex": [GP, SP, PP, c_p, c_i64, c_p, c_i32, c_p],
+    "smk_run_steps_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p],
     "smk_step_is_fused": [GP, PP, c_i32, C.POINTER(c_i32)],
     "smk_fused_plan": [c_i32, c_i32, c_i32, C.POINTER(c_i32), c_i32, C.POINTER(c_i32)],
     "smk_div_norms": [GP, c_p, c_p, c_p, c_p],

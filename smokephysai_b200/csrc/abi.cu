@@ -357,9 +357,29 @@ int smk_fused_plan(int32_t nsims, int32_t nsteps, int32_t piece_len, int32_t* it
     return rc;
 }
 
+// frames of SMK_FRAME_F32 / _F16 / _BF16: bytes per element; the kernels store 4 elements at a time (16 or 8 bytes)
+static int frame_elem_size(int32_t fmt) { return fmt == SMK_FRAME_F32 ? 4 : 2; }
+static int check_frames(const char* who, const void* frames, int64_t stride0, int64_t stride1, int32_t fmt)
+{
+    if (fmt != SMK_FRAME_F32 && fmt != SMK_FRAME_F16 && fmt != SMK_FRAME_BF16)
+        return fail(SMK_EINVAL, "%s: frame_format %d is not SMK_FRAME_F32/_F16/_BF16", who, fmt);
+    if (!frames) return SMK_OK;
+    if (reinterpret_cast<uintptr_t>(frames) % (4u * frame_elem_size(fmt)))
+        return fail(SMK_EINVAL, "%s: frame base is not aligned to 4 elements of the frame type (%d B)", who, 4 * frame_elem_size(fmt));
+    if ((stride0 | stride1) & 3) return fail(SMK_EINVAL, "%s: frame strides must be multiples of 4 elements", who);
+    return SMK_OK;
+}
+
 int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, float* frame, int64_t frame_stride,
              const float* fmul, void* stream)
 {
+    return smk_step_ex(g, st, prm, frame, frame_stride, fmul, SMK_FRAME_F32, stream);
+}
+
+int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
+                const float* fmul, int32_t frame_format, void* stream)
+{
+    SMK_TRY(check_frames("smk_step", frame, frame_stride, 0, frame_format));
     SMK_TRY(check_grid(g, "smk_step"));
     if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
         return fail(SMK_EUNSUPPORTED, "smk_step: slab grids are stepped phase by phase with halo exchanges in between");
@@ -373,7 +393,7 @@ int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, floa
     SMK_TRY(pick_step_kernel(g, prm, 1, &fused));
     if (fused)
         return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], 1, frame, 0, frame_stride,
-                                  fmul, prm->dt, prm->c_uv, prm->c_d, prm->decay, prm->jacobi_iters, st->div, s);
+                                  fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay, prm->jacobi_iters, st->div, s);
     const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
     float *u0 = st->u[cu], *u1 = st->u[cu ^ 1], *v0 = st->v[cv], *v1 = st->v[cv ^ 1], *d0 = st->d[cd], *d1 = st->d[cd ^ 1];
     // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
@@ -391,20 +411,29 @@ int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, floa
     if (fuse) {
         SMK_TRY(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s, 1, pl, v0));
         SMK_TRY(launch_advect(g, v0, v1, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v0, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
-        SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v1, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s));
+        SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v1, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s,
+                              0, nullptr, nullptr, nullptr, frame_format));
         st->cur_v ^= 1;
         return SMK_OK;
     }
     SMK_TRY(launch_project(g, pl, u1, v1, prm->dt, s));
     SMK_TRY(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
     SMK_TRY(launch_advect(g, v1, v0, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
-    SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v0, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s));
+    SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v0, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s,
+                          0, nullptr, nullptr, nullptr, frame_format));
     return SMK_OK;
 }
 
 int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
                   float* frames, int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, void* stream)
 {
+    return smk_run_steps_ex(g, st, prm, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, SMK_FRAME_F32, stream);
+}
+
+int smk_run_steps_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                     int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format, void* stream)
+{
+    SMK_TRY(check_frames("smk_run_steps", frames, frame_step_stride, frame_batch_stride, frame_format));
     if (nsteps < 0) return fail(SMK_EINVAL, "smk_run_steps: negative nsteps");
     if (nsteps > 1 && g && st && prm) {
         // the fused kernel keeps the state on chip across all the steps of the call: one launch
@@ -417,12 +446,14 @@ int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
             if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "smk_run_steps: negative jacobi_iters");
             if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "smk_run_steps: dt must be non-zero");
             return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
-                                      frame_step_stride, frame_batch_stride, fmul, prm->dt, prm->c_uv, prm->c_d, prm->decay,
+                                      frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
                                       prm->jacobi_iters, st->div, (cudaStream_t)stream);
         }
     }
+    const int64_t step_bytes = frame_step_stride * frame_elem_size(frame_format);
     for (int t = 0; t < nsteps; ++t)
-        SMK_TRY(smk_step(g, st, prm, frames ? frames + (int64_t)t * frame_step_stride : nullptr, frame_batch_stride, fmul, stream));
+        SMK_TRY(smk_step_ex(g, st, prm, frames ? static_cast<char*>(frames) + (int64_t)t * step_bytes : nullptr, frame_batch_stride, fmul,
+                            frame_format, stream));
     return SMK_OK;
 }
 

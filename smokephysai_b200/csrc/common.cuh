@@ -5,10 +5,41 @@
 // nvcc never contracts a*b+c; division is IEEE (-prec-div=true default).  Do not add fast-math flags.
 #pragma once
 #include <cuda_runtime.h>
+#include <cuda_fp16.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 #include "../../include/smoke_b200.h"
 
 namespace smk {
+
+// ---- frame output in SMK_FRAME_F32 / _F16 / _BF16 ----------------------------------------------------------------
+// A frame element is the fp32 value the step computes (fractal factor applied), rounded once to the frame type,
+// round-to-nearest-even, just before the store (cvt.rn: overflow -> inf, subnormals kept, nothing saturates).  `frame`
+// points at the frame base, `k` counts elements of the frame type; `fmt` is uniform over the launch, so the branch
+// never diverges.  frame_st4 needs k to be a multiple of 4 (16-byte fp32 / 8-byte half stores).
+__device__ __forceinline__ unsigned pack_h2(const __half2 h) { return *reinterpret_cast<const unsigned*>(&h); }
+__device__ __forceinline__ unsigned pack_b2(const __nv_bfloat162 h) { return *reinterpret_cast<const unsigned*>(&h); }
+__device__ __forceinline__ void frame_st4(void* frame, const size_t k, const float4 v, const int fmt)
+{
+    if (fmt == SMK_FRAME_F16)
+        *reinterpret_cast<uint2*>(static_cast<__half*>(frame) + k) =
+            make_uint2(pack_h2(__floats2half2_rn(v.x, v.y)), pack_h2(__floats2half2_rn(v.z, v.w)));
+    else if (fmt == SMK_FRAME_BF16)
+        *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(frame) + k) =
+            make_uint2(pack_b2(__floats2bfloat162_rn(v.x, v.y)), pack_b2(__floats2bfloat162_rn(v.z, v.w)));
+    else
+        *reinterpret_cast<float4*>(static_cast<float*>(frame) + k) = v;
+}
+__device__ __forceinline__ void* frame_offset(void* frame, const size_t k, const int fmt)
+{
+    return static_cast<char*>(frame) + k * (fmt == SMK_FRAME_F32 ? 4 : 2);
+}
+__device__ __forceinline__ void frame_st1(void* frame, const size_t k, const float v, const int fmt)
+{
+    if (fmt == SMK_FRAME_F16)       static_cast<__half*>(frame)[k] = __float2half_rn(v);
+    else if (fmt == SMK_FRAME_BF16) static_cast<__nv_bfloat16*>(frame)[k] = __float2bfloat16_rn(v);
+    else                            static_cast<float*>(frame)[k] = v;
+}
 
 __device__ __forceinline__ int clampi(int a, int lo, int hi) { return min(max(a, lo), hi); }
 // torch.clamp(x, lo, hi) == min(max(x, lo), hi)
@@ -127,10 +158,11 @@ int launch_bilerp(const float* f, int rows, int cols, int pitch, const float* y,
 // part (tiled kernel only, see advect_is_tiled): band_n > 0 -> only the tile rows [band_lo, band_lo + band_n); else every tile row
 // except those of the (up to two, ascending, disjoint) bands [skip_lo[k], skip_lo[k] + skip_n[k])
 struct AdvectPart { int band_lo, band_n, skip_lo[2], skip_n[2]; };
+// frame / frame_stride / frame_format: the (fractal-scaled) copy of the result, SMK_FRAME_*, stride in elements of that type
 int launch_advect(const smk_grid_t* g, const float* field, float* out, int rows, int cols, int pitch, int64_t stride,
-                  const float* u, const float* v, float dt, float scale, float* frame, int64_t frame_stride,
+                  const float* u, const float* v, float dt, float scale, void* frame, int64_t frame_stride,
                   const float* fmul, const smk_slab_check_t* chk, cudaStream_t s, int proj = 0, const float* p = nullptr, float* vout = nullptr,
-                  const AdvectPart* part = nullptr);
+                  const AdvectPart* part = nullptr, int frame_format = SMK_FRAME_F32);
 bool advect_can_fuse_project(const smk_grid_t* g);
 // 128-byte CUtensorMap of a (pitch, rows, batch) fp32 tensor read / written in box_cols x box_rows x 1 boxes (jacobi.cu); false when
 // the driver entry point is missing or the shape cannot be encoded
@@ -147,8 +179,8 @@ int launch_frame_features(const float* frames, int64_t frame_stride, int nframes
 int launch_frame_distances(const float* frames, int64_t frame_stride, int nframes, int h, int w, int pitch, double* sumsq, cudaStream_t s);
 bool fused_supported(const smk_grid_t* g);
 int pick_cluster(int batch);          // CTAs per simulation k_step_cluster would use for `batch` 128 x 128 simulations (0: one CTA each)
-int launch_steps_fused(const smk_grid_t* g, float* u, float* v, float* d, float* p, int nsteps, float* frames,
-                       int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul,
+int launch_steps_fused(const smk_grid_t* g, float* u, float* v, float* d, float* p, int nsteps, void* frames,
+                       int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int frame_format,
                        float dt, float c_uv, float c_d, float decay, int K, float* scratch, cudaStream_t s);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);
 int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int cols, int pitch, int batch, int64_t stride, cudaStream_t s);

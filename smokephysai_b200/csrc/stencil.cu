@@ -428,7 +428,8 @@ struct AdvectArgs {
     const float* F; float* O; int rows, cols, pitch; long long stride;
     const float* U; const float* V; int h, w, pu, pv; long long su_, sv_;
     float dt; int has_scale; float scale;
-    float* frame; long long frame_stride; int frame_pitch; const float* fmul;
+    void* frame; long long frame_stride; int frame_pitch; const float* fmul;      // frame: SMK_FRAME_* elements (frame_format)
+    int frame_format;
     unsigned ngroups; unsigned long long magic;          // row = (idx * magic) >> 40 == idx / ngroups (+ fix-up)
     int row0, gh;                                        // slab: global row of local row 0, global cell rows
     int need_lo, need_hi, valid_lo, valid_hi; int* overflow;
@@ -525,7 +526,7 @@ k_advect(const AdvectArgs a)
             const float4 m = ld4(a.fmul + (size_t)i * a.frame_pitch + c0);
             fr.x = fr.x + m.x * fr.x; fr.y = fr.y + m.y * fr.y; fr.z = fr.z + m.z * fr.z; fr.w = fr.w + m.w * fr.w;
         }
-        st4(a.frame + b * a.frame_stride + (size_t)i * a.frame_pitch + c0, fr);
+        frame_st4(a.frame, b * a.frame_stride + (size_t)i * a.frame_pitch + c0, fr, a.frame_format);
     }
 }
 
@@ -592,6 +593,7 @@ __device__ __forceinline__ void advect_tile(const AdvectArgs& a, AdvectTile& T, 
 {
     const int tid = threadIdx.x, lane = tid & 31, wp = tid >> 5;
     const int w = a.w, rows = a.rows, cols = a.cols, pitch = a.pitch;
+    const int ffmt = PROJ ? SMK_FRAME_F32 : a.frame_format;          // the fused u advection writes no frame (a.frame is NULL)
 
     // ---- stage: field window rows [i0-4, i0+20) x columns [j0-4, j0+132), u rows [i0, i0+16), v rows [i0, i0+17) ----
     const int wy0 = INTERIOR ? i0 - AT_HB : max(i0 - AT_HB, 0), wy1 = INTERIOR ? i0 + AT_R + AT_HB : min(i0 + AT_R + AT_HB, rows);
@@ -834,16 +836,16 @@ __device__ __forceinline__ void advect_tile(const AdvectArgs& a, AdvectTile& T, 
 #pragma unroll
             for (int k = 0; k < 4; ++k) orow[jb + 32 * k] = val[k];
             if (a.frame) {                                                          // :173 (+ fractal_generator.py:62)
-                float* frow = a.frame + b * a.frame_stride + (unsigned)i * a.frame_pitch;
+                const size_t frow = b * a.frame_stride + (unsigned)i * a.frame_pitch;
 #pragma unroll
                 for (int k = 0; k < 4; ++k) {
                     float fr = val[k];
                     if (a.fmul) fr = fr + __ldg(a.fmul + (unsigned)i * a.frame_pitch + jb + 32 * k) * fr;
-                    frow[jb + 32 * k] = fr;
+                    frame_st1(a.frame, frow + jb + 32 * k, fr, ffmt);
                 }
             }
         } else {
-            float* frow = a.frame ? a.frame + b * a.frame_stride + (unsigned)i * a.frame_pitch : nullptr;
+            const size_t frow = b * a.frame_stride + (unsigned)i * a.frame_pitch;
             const float* mrow = a.fmul ? a.fmul + (unsigned)i * a.frame_pitch : nullptr;
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -851,10 +853,10 @@ __device__ __forceinline__ void advect_tile(const AdvectArgs& a, AdvectTile& T, 
                 if (j < pitch) {
                     const float x = (j < cols) ? val[k] : 0.0f;
                     orow[j] = x;
-                    if (frow && j < a.frame_pitch) {
+                    if (a.frame && j < a.frame_pitch) {
                         float fr = x;
                         if (mrow) fr = fr + __ldg(mrow + j) * fr;
-                        frow[j] = fr;
+                        frame_st1(a.frame, frow + j, fr, ffmt);
                     }
                 }
             }
@@ -927,16 +929,16 @@ bool advect_is_tiled(const smk_grid_t* g, int rows, int cols)
 int advect_tile_rows() { return AT_R; }
 
 int launch_advect(const smk_grid_t* g, const float* field, float* out, int rows, int cols, int pitch, int64_t stride,
-                  const float* u, const float* v, float dt, float scale, float* frame, int64_t frame_stride,
+                  const float* u, const float* v, float dt, float scale, void* frame, int64_t frame_stride,
                   const float* fmul, const smk_slab_check_t* chk, cudaStream_t s, int proj, const float* p, float* vout,
-                  const AdvectPart* part)
+                  const AdvectPart* part, int frame_format)
 {
     if ((int64_t)rows * pitch >= (1ll << 31)) return fail(SMK_EUNSUPPORTED, "smk_advect: field of %d x %d exceeds 2^31 elements", rows, pitch);
     AdvectArgs a;
     a.F = field; a.O = out; a.rows = rows; a.cols = cols; a.pitch = pitch; a.stride = stride;
     a.U = u; a.V = v; a.h = g->h; a.w = g->w; a.pu = g->pitch_u; a.pv = g->pitch_v; a.su_ = g->stride_u; a.sv_ = g->stride_v;
     a.dt = dt; a.has_scale = scale != 1.0f ? 1 : 0; a.scale = scale;
-    a.frame = frame; a.frame_stride = frame_stride; a.frame_pitch = g->pitch_c; a.fmul = fmul;
+    a.frame = frame; a.frame_stride = frame_stride; a.frame_pitch = g->pitch_c; a.fmul = fmul; a.frame_format = frame_format;
     a.ngroups = (unsigned)((cols + 3) / 4);
     a.magic = ((1ull << 40) + a.ngroups - 1) / a.ngroups;
     const bool slab = g->gh != 0 && (g->gh != g->h || g->row0 != 0);

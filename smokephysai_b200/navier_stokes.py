@@ -359,10 +359,17 @@ class NavierStokesSimulator(nn.Module):
         _lib.call("smk_project", g, self._ptr("p"), self._ptr("u"), self._ptr("v"), float(self.dt), s)
 
     # ------------------------------------------------------------------ a3-a11 (navier_stokes.py:151-173)
-    def _new_frames(self, nsteps=None):
+    def _new_frames(self, nsteps=None, dtype=torch.float32):
         L = self._layout
         shape = (L.batch, L.h, L.pitch_c) if nsteps is None else (L.batch, nsteps, L.h, L.pitch_c)
-        return torch.empty(shape, dtype=torch.float32, device=self._cuda)
+        return torch.empty(shape, dtype=dtype, device=self._cuda)
+
+    def _check_frame_buffer(self, name, t, shape):
+        """A caller-owned frame buffer: contiguous, `shape`, on this simulator's device, fp32 / fp16 / bf16 -> SMK_FRAME_*."""
+        if (tuple(t.shape) != shape or not t.is_contiguous() or t.dtype not in _lib.FRAME_FORMATS or t.device != self._cuda):
+            raise ValueError("%s must be a contiguous float32, float16 or bfloat16 %s tensor on %s"
+                             % (name, list(shape), self._cuda))
+        return _lib.frame_format(t.dtype)
 
     def _finish_frames(self, fr):
         L = self._layout
@@ -372,54 +379,60 @@ class NavierStokesSimulator(nn.Module):
             fr = fr[0]
         return self._to_out(fr)
 
-    def step(self, fmul=None):
+    def step(self, fmul=None, *, frame_dtype=torch.float32):
         """One time step; returns a copy of the new density ([h, w], or [batch, h, w]).
 
         fmul (optional, [h, pitch_c] device tensor) fuses the fractal multiply of SmokeSimulator.simulate_step
         into the returned copy: frame = d + fmul*d (fractal_generator.py:62); solver state is not perturbed.
+        frame_dtype torch.float16 / torch.bfloat16 returns that copy rounded once (to nearest even) by the kernel that
+        writes it, equal to the fp32 copy's .to(frame_dtype); the state is the same whatever the dtype.
         """
-        fr = self._new_frames()
+        fmt = _lib.frame_format(frame_dtype)
+        fr = self._new_frames(dtype=frame_dtype)
         prm = self._params()
-        _lib.call("smk_step", C.byref(self._grid), C.byref(self._state), C.byref(prm), fr.data_ptr(),
-                  self._layout.h * self._layout.pitch_c, fmul.data_ptr() if fmul is not None else None, self._stream())
+        _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), fr.data_ptr(),
+                  self._layout.h * self._layout.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
         return self._finish_frames(fr)
 
     def step_into(self, frame, fmul=None):
-        """One time step whose returned copy is written into `frame`, a contiguous fp32 [batch, h, pitch_c]
-        device tensor owned by the caller (no allocation, no sync)."""
+        """One time step whose returned copy is written into `frame`, a contiguous [batch, h, pitch_c] float32, float16
+        or bfloat16 device tensor owned by the caller (no allocation, no sync)."""
         L = self._layout
-        if (tuple(frame.shape) != (L.batch, L.h, L.pitch_c) or not frame.is_contiguous()
-                or frame.dtype != torch.float32 or frame.device != self._cuda):
-            raise ValueError("frame must be a contiguous fp32 [%d, %d, %d] tensor on %s" % (L.batch, L.h, L.pitch_c, self._cuda))
+        fmt = self._check_frame_buffer("frame", frame, (L.batch, L.h, L.pitch_c))
         prm = self._params()
-        _lib.call("smk_step", C.byref(self._grid), C.byref(self._state), C.byref(prm), frame.data_ptr(),
-                  L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, self._stream())
+        _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), frame.data_ptr(),
+                  L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
 
-    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None):
+    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None):
         """nsteps consecutive steps enqueued back to back; returns frames [batch, nsteps, h, w] ([nsteps, h, w] if batch == 1).
 
-        out: optional preallocated [batch, nsteps, h, pitch_c] fp32 device buffer to write the frames into."""
+        out: optional preallocated [batch, nsteps, h, pitch_c] device buffer to write the frames into (float32, float16 or
+        bfloat16).  frame_dtype: the frames' dtype (default float32; with `out`, out.dtype, and a different frame_dtype is
+        an error); half-precision frames are the fp32 ones rounded once to nearest even, as in step()."""
         L = self._layout
-        if out is not None and (tuple(out.shape) != (L.batch, nsteps, L.h, L.pitch_c) or not out.is_contiguous()
-                                or out.dtype != torch.float32 or out.device != self._cuda):
-            raise ValueError("out must be a contiguous fp32 [%d, %d, %d, %d] tensor on %s" % (L.batch, nsteps, L.h, L.pitch_c, self._cuda))
-        fr = out if out is not None else (self._new_frames(nsteps) if return_frames else None)
+        if out is not None:
+            fmt = self._check_frame_buffer("out", out, (L.batch, nsteps, L.h, L.pitch_c))
+            if frame_dtype is not None and frame_dtype != out.dtype:
+                raise ValueError("frame_dtype %s disagrees with out.dtype %s" % (frame_dtype, out.dtype))
+            fr = out
+        else:
+            frame_dtype = torch.float32 if frame_dtype is None else frame_dtype
+            fmt = _lib.frame_format(frame_dtype)
+            fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
         prm = self._params()
-        _lib.call("smk_run_steps", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
+        _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
                   fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c,
-                  fmul.data_ptr() if fmul is not None else None, self._stream())
+                  fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
         return self._finish_frames(fr) if fr is not None else None
 
     def run_steps_time_major(self, nsteps, out, fmul=None):
-        """nsteps consecutive steps whose frames go to `out`, a contiguous fp32 [nsteps, batch, h, pitch_c] device
-        buffer owned by the caller (time-major: the frames of one step are one contiguous block)."""
+        """nsteps consecutive steps whose frames go to `out`, a contiguous [nsteps, batch, h, pitch_c] float32, float16 or
+        bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block)."""
         L = self._layout
-        if (tuple(out.shape) != (nsteps, L.batch, L.h, L.pitch_c) or not out.is_contiguous()
-                or out.dtype != torch.float32 or out.device != self._cuda):
-            raise ValueError("out must be a contiguous fp32 [%d, %d, %d, %d] tensor on %s" % (nsteps, L.batch, L.h, L.pitch_c, self._cuda))
+        fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
         prm = self._params()
-        _lib.call("smk_run_steps", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps), out.data_ptr(),
-                  L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, self._stream())
+        _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps), out.data_ptr(),
+                  L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
 
     def divergence_norms(self):
         """(max|div|, ||div||_2) of the un-normalised divergence of the live (u, v), per simulation: [batch, 2] on the host."""

@@ -11,7 +11,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from . import chaos, hostmem
+from . import _lib, chaos, hostmem
 from .fractal_generator import FractalGenerator
 from .navier_stokes import NavierStokesSimulator
 
@@ -45,7 +45,8 @@ class SmokeSimulator(nn.Module):
         return density
 
     # -------------------------------------------------------------- batched generation (data_loader.py:37-99)
-    def generate_sequences(self, emitters, sequence_length=20, add_fractal=True, to_host=False, steps_per_copy=None):
+    def generate_sequences(self, emitters, sequence_length=20, add_fractal=True, to_host=False, steps_per_copy=None,
+                           frame_dtype=torch.float32):
         """Reset, splat one emitter list per simulation, run sequence_length steps.
 
         emitters[b] = [((x, y), intensity), ...] for simulation b (len == batch).  Returns frames
@@ -58,27 +59,38 @@ class SmokeSimulator(nn.Module):
         copy is one contiguous block.  steps_per_copy is the chunk length (default: 1 for the phase-per-kernel
         step, 2 when the fused kernel keeps the state on chip across the steps of a launch).  The returned
         tensor is the [batch, sequence_length, h, w] view of the pinned time-major buffer, which this
-        simulator owns and reuses on the next call."""
+        simulator owns and reuses on the next call of the same frame_dtype.
+
+        frame_dtype torch.float16 / torch.bfloat16: the frames are rounded once (to nearest even) by the kernels that
+        write them -- equal to the float32 frames' .to(frame_dtype) -- so half the bytes cross PCIe; the simulation
+        itself is the same whatever the dtype."""
         ns = self.ns_solver
         L = ns._layout
         B, T = ns.batch, int(sequence_length)
+        _lib.frame_format(frame_dtype)                     # ValueError for an unsupported dtype, before any work
         ns.setup_grid()
         src, off, _ = ns.upload_sources([[(x, y, 8, inten) for (x, y), inten in lst] for lst in emitters], pin=to_host)
         ns.splat_uploaded(src, off)
         fmul = self.fractal_gen.multiplier((ns.h, ns.w), 0.05) if add_fractal else None
         if not to_host:
-            fr = ns.run_steps(T, fmul=fmul)
+            fr = ns.run_steps(T, fmul=fmul, frame_dtype=frame_dtype)
             return fr if B > 1 else fr.unsqueeze(0)
-        key = (T,)
-        if getattr(self, "_gen_key", None) != key:
-            self._gen_dev = torch.empty(T, B, L.h, L.pitch_c, dtype=torch.float32, device=ns._cuda)
+        # one (device, pinned host) buffer pair per frame dtype, keyed (T, dtype): calls that alternate dtypes each keep
+        # their own buffers instead of reallocating pinned memory every call or handing one call's frames to the other
+        if not hasattr(self, "_gen_bufs"):
+            self._gen_bufs = {}
+            self._gen_copy_stream = torch.cuda.Stream(device=ns._cuda)
+        key = (T, frame_dtype)
+        bufs = self._gen_bufs.get(frame_dtype)
+        if bufs is None or bufs[0] != key:
+            dev = torch.empty(T, B, L.h, L.pitch_c, dtype=frame_dtype, device=ns._cuda)
             # pinned pages on the NUMA node of this GPU's PCIe root: with several ranks copying at once a buffer on the far
             # socket costs most of the D2H bandwidth (hostmem.py)
-            self._gen_host = hostmem.pinned_empty((T, B, L.h, L.pitch_c), torch.float32, ns._cuda)
+            host = hostmem.pinned_empty((T, B, L.h, L.pitch_c), frame_dtype, ns._cuda)
             self._gen_host_node = hostmem.gpu_locality(ns._cuda)[0]
-            self._gen_copy_stream = torch.cuda.Stream(device=ns._cuda)
-            self._gen_key = key
-        dev, host, cs = self._gen_dev, self._gen_host, self._gen_copy_stream
+            bufs = self._gen_bufs[frame_dtype] = (key, dev, host)
+        _, dev, host = bufs
+        cs = self._gen_copy_stream
         main = torch.cuda.current_stream(ns._cuda)
         cs.wait_stream(main)                      # the previous call's consumer is done with the buffers
         n = int(steps_per_copy) if steps_per_copy else (2 if ns.step_is_fused(2) else 1)
