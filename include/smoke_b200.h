@@ -310,6 +310,40 @@ SMK_API int smk_slab_step(const smk_grid_t* g, smk_state_t* st, const smk_params
 SMK_API int smk_project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
                                const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d, void* stream);
 
+/* ---- reverse mode: adjoints of the step's phases (csrc/adjoint.cu), composed by smokephysai_b200/autodiff.py -------------------
+ * Each entry is the transpose of one forward phase, linearised at the forward values it is given; gradients follow torch autograd
+ * through the reference's ops (floor: no gradient; torch.clamp passes it where lo <= x <= hi; bilinear weights from the clamped
+ * integer corners).  Gradient buffers have the layout of the field they belong to (pads zero).  No float atomics: two calls on the
+ * same inputs give bitwise-equal results.  SMK_EUNSUPPORTED on a slab grid (gh != 0). */
+
+/*     adjoint of smk_advect (field [batch][rows][cols] advected by (u, v)).  The effective output gradient is
+ *       e = (g_out + (g_frame + fmul*g_frame)) * scale      (g_out, g_frame and fmul may each be NULL: zero / no fractal)
+ *     with g_frame [batch][h][pitch_c] frame_stride apart and fmul [h][pitch_c] (cell-centred fields only).  g_field receives the
+ *     field gradient (written, or added when accumulate != 0); the gradients through the back-trace are added into g_u and g_v.
+ *     g_field may alias g_u or g_v and g_out may alias any output.  workspace: 16 + 32*batch*rows*cols bytes, 16-byte aligned. */
+SMK_API int smk_advect_adjoint(const smk_grid_t* g, const float* field, int32_t rows, int32_t cols, int32_t pitch, int64_t stride,
+                               const float* u, const float* v, float dt, float scale,
+                               const float* g_out, const float* g_frame, int64_t frame_stride, const float* fmul,
+                               float* g_field, int32_t accumulate, float* g_u, float* g_v, void* workspace, void* stream);
+/*     adjoint of smk_project: g_p = g_p_in + the transpose of the gradient subtract applied to (g_u, g_v); g_p_in may be NULL (zero).
+ *     The gradients of u and v pass through unchanged. */
+SMK_API int smk_project_adjoint(const smk_grid_t* g, const float* g_u, const float* g_v, const float* g_p_in, float* g_p, float dt,
+                                void* stream);
+/*     adjoint of K Jacobi sweeps (smk_jacobi): from the gradient g_p_in of the swept pressure, g_p (of the pressure before the sweeps,
+ *     ring cells included) and g_div (of the divergence).  T as smk_jacobi.  workspace: 5 fields of batch * F floats, F = stride_c
+ *     (h * pitch_c when batch == 1), 16-byte aligned; NULL allowed when K == 0. */
+SMK_API int smk_jacobi_adjoint(const smk_grid_t* g, const float* g_p_in, float* g_p, float* g_div, int32_t K, int32_t T,
+                               float* workspace, void* stream);
+/*     adjoint of smk_forces_diffuse_div: from the gradients of (u_out, v_out, d_out, div), those of (u, v, d) before the buoyancy and
+ *     the diffusions.  Outputs must not alias inputs. */
+SMK_API int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u_diff, const float* g_v_diff, const float* g_d_diff,
+                                           const float* g_div, float* g_u, float* g_v, float* g_d, float dt, float c_uv, float c_d,
+                                           void* stream);
+/*     intensity gradient of smk_splat_sources: g_intensity[k] = sum over emitter k's footprint of g_density * its splat weight,
+ *     for the nsources = offsets[batch] emitters of (sources, offsets); a fixed-order tree per emitter. */
+SMK_API int smk_splat_sources_adjoint(const smk_grid_t* g, const float* g_density, const smk_source_t* sources,
+                                      const int32_t* offsets, int32_t nsources, float* g_intensity, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

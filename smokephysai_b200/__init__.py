@@ -7,5 +7,6 @@ C ABI in include/smoke_b200.h (libsmoke_sm100.so); there is no CPU or eager-PyTo
 from .navier_stokes import NavierStokesSimulator, FieldLayout  # noqa: F401
 from .fractal_generator import FractalGenerator  # noqa: F401
 from .smoke_simulator import SmokeSimulator  # noqa: F401
+from . import autodiff  # noqa: F401
 
-__all__ = ["NavierStokesSimulator", "FractalGenerator", "SmokeSimulator", "FieldLayout"]
+__all__ = ["NavierStokesSimulator", "FractalGenerator", "SmokeSimulator", "FieldLayout", "autodiff"]

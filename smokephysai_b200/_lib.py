@@ -112,6 +112,12 @@ SIGNATURES = {
     "smk_peer_unpack": [C.POINTER(PeerComm), C.POINTER(c_p), c_p],
     "smk_slab_step": [GP, SP, PP, C.POINTER(PeerComm), c_i32, C.POINTER(SlabCheck), C.POINTER(SlabCheck), C.POINTER(SlabCheck), c_p],
     "smk_project_advect": [GP, SP, PP, C.POINTER(SlabCheck), C.POINTER(SlabCheck), C.POINTER(SlabCheck), c_p],
+    "smk_advect_adjoint": [GP, c_p, c_i32, c_i32, c_i32, c_i64, c_p, c_p, c_f, c_f, c_p, c_p, c_i64, c_p, c_p, c_i32, c_p, c_p,
+                           c_p, c_p],
+    "smk_project_adjoint": [GP, c_p, c_p, c_p, c_p, c_f, c_p],
+    "smk_jacobi_adjoint": [GP, c_p, c_p, c_p, c_i32, c_i32, c_p, c_p],
+    "smk_forces_diffuse_div_adjoint": [GP, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_f, c_f, c_p],
+    "smk_splat_sources_adjoint": [GP, c_p, c_p, c_p, c_i32, c_p, c_p],
 }
 
 _lib = None

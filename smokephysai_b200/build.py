@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 SO = os.path.join(HERE, "libsmoke_sm100.so")
-SOURCES = ["abi.cu", "jacobi.cu", "stencil.cu", "features.cu", "fused.cu", "nccl_halo.cu", "peer_halo.cu"]
+SOURCES = ["abi.cu", "jacobi.cu", "stencil.cu", "features.cu", "fused.cu", "nccl_halo.cu", "peer_halo.cu", "adjoint.cu"]
 HEADERS = ["common.cuh", "jacobi_core.cuh", os.path.join("..", "..", "include", "smoke_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
