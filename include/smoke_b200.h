@@ -196,6 +196,16 @@ SMK_API int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t
 SMK_API int smk_run_steps_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
                              void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
                              const float* fmul, int32_t frame_format, void* stream);
+/*     the same on a freshly reset state: u, v, p all zeros and the density zeros plus the emitters of smk_splat_sources(g,
+ *     density, sources, offsets) (sources and offsets may both be NULL: no emitters), whatever the live copies hold now.
+ *     When the call runs on k_step_fused (one SM per simulation), that kernel builds the reset state on chip instead of
+ *     reading it -- no memset, no splat launch -- and *consumed_host is 1; the live copies then hold the state after the
+ *     steps, and the other copies and div are left as they were.  Otherwise nothing is enqueued and *consumed_host is 0:
+ *     the caller resets, splats and runs smk_run_steps_ex itself.  nsteps = 1 with frame_step_stride 0 is smk_step_ex. */
+SMK_API int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                                   void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                                   const float* fmul, int32_t frame_format, const smk_source_t* sources,
+                                   const int32_t* offsets, int32_t* consumed_host, void* stream);
 /*     1 when a call of nsteps steps (smk_step: 1) would take the fused single-launch path for this grid and params */
 SMK_API int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nsteps, int32_t* fused_host);
 /* Host-only (no GPU needed): the time-sliced schedule smk_run_steps gives the fused kernel when `nsims` simulations of

@@ -457,6 +457,32 @@ int smk_run_steps_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* p
     return SMK_OK;
 }
 
+int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                           int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format,
+                           const smk_source_t* sources, const int32_t* offsets, int32_t* consumed_host, void* stream)
+{
+    if (!consumed_host) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: consumed_host is NULL");
+    *consumed_host = 0;
+    SMK_TRY(check_frames("smk_run_steps_reset_ex", frames, frame_step_stride, frame_batch_stride, frame_format));
+    if (!g || !st || !prm) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: grid/state/params NULL");
+    if ((sources == nullptr) != (offsets == nullptr)) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: sources and offsets go together");
+    if (nsteps < 1) return SMK_OK;
+    SMK_TRY(check_grid(g, "smk_run_steps_reset_ex"));
+    int fused = 0;
+    SMK_TRY(pick_step_kernel(g, prm, nsteps, &fused));
+    const bool full = g->h == 128 && g->w == 128 && g->pitch_u == 128 && g->pitch_v == 132 && g->pitch_c == 128;
+    if (!fused || (full && pick_cluster(g->batch) != 0)) return SMK_OK;          // not k_step_fused: the caller resets
+    SMK_TRY(check_ptrs("smk_run_steps_reset_ex", {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
+    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: cur_* must be 0 or 1");
+    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: negative jacobi_iters");
+    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: dt must be non-zero");
+    SMK_TRY(launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
+                               frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
+                               prm->jacobi_iters, st->div, (cudaStream_t)stream, true, sources, offsets));
+    *consumed_host = 1;
+    return SMK_OK;
+}
+
 int smk_div_norms(const smk_grid_t* g, const float* u, const float* v, float* out, void* stream)
 {
     SMK_TRY(check_grid(g, "smk_div_norms"));

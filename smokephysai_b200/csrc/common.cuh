@@ -113,6 +113,21 @@ inline void launch_chain(void (*kernel)(P...), const dim3 grid, const dim3 block
     (void)cudaLaunchKernelEx(&cfg, kernel, P(args)...);          // errors are picked up by check_launch()
 }
 
+// add_smoke_source at one cell (navier_stokes.py:45-48): acc plus emitter e's Gaussian when cell (i, j) lies within its radius.
+// k_splat and the reset start of k_step_fused add a cell's emitters through this, in list order: bit-identical densities.
+__device__ __forceinline__ float splat_add(float acc, const int i, const int j, const smk_source_t& e)
+{
+    const long long dx = (long long)j - e.x, dy = (long long)i - e.y;
+    const float dist = sqrtf((float)(dx * dx + dy * dy));            // navier_stokes.py:45
+    if (dist <= (float)e.radius) {                                   // :46
+        const double r3 = (double)e.radius / 3.0;
+        const float denom = (float)(2.0 * (r3 * r3));
+        const float d2 = dist * dist;
+        acc = acc + e.intensity * expf((-d2) / denom);               // :48
+    }
+    return acc;
+}
+
 // Tuning / test switches from the environment, read ONCE per process (getenv is not free and not thread-safe against
 // setenv; a launch must not pay for it) and again only on smk_reload_env(), which the tests call after changing a variable.
 // SMK_ENV_UNSET marks a variable that is not set: the launcher then picks by its own rule.
@@ -181,7 +196,8 @@ bool fused_supported(const smk_grid_t* g);
 int pick_cluster(int batch);          // CTAs per simulation k_step_cluster would use for `batch` 128 x 128 simulations (0: one CTA each)
 int launch_steps_fused(const smk_grid_t* g, float* u, float* v, float* d, float* p, int nsteps, void* frames,
                        int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int frame_format,
-                       float dt, float c_uv, float c_d, float decay, int K, float* scratch, cudaStream_t s);
+                       float dt, float c_uv, float c_d, float decay, int K, float* scratch, cudaStream_t s,
+                       bool reset = false, const smk_source_t* src = nullptr, const int32_t* src_off = nullptr);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);
 int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int cols, int pitch, int batch, int64_t stride, cudaStream_t s);
 

@@ -1040,17 +1040,7 @@ k_splat(float* __restrict__ Dn, const int h, const int w, const int pc, const lo
         for (int q = 0; q < 8; ++q) { if (q < wp) before += wcount[q]; total += wcount[q]; }
         if (hit) list[before + __popc(m & ((1u << lane) - 1u))] = k;
         __syncthreads();
-        for (int q = 0; q < total; ++q) {
-            const smk_source_t e = src[list[q]];
-            const long long dx = (long long)j - e.x, dy = (long long)i - e.y;
-            const float dist = sqrtf((float)(dx * dx + dy * dy));            // navier_stokes.py:45
-            if (dist <= (float)e.radius) {                                   // :46
-                const double r3 = (double)e.radius / 3.0;
-                const float denom = (float)(2.0 * (r3 * r3));
-                const float d2 = dist * dist;
-                acc = acc + e.intensity * expf((-d2) / denom);               // :48
-            }
-        }
+        for (int q = 0; q < total; ++q) acc = splat_add(acc, i, j, src[list[q]]);
         __syncthreads();
     }
     if (in) *cell = acc;

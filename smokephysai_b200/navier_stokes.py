@@ -115,11 +115,19 @@ class NavierStokesSimulator(nn.Module):
         self._arena = None
         self._state = State()
         self._mirrors = {}
+        # Deferred reset (see setup_grid): _pending is None, or the [(sources, offsets)] splats issued since a reset that is not
+        # applied yet; _stale: a run that consumed a reset left the non-live copies, div and boundary as they were before it.
+        self._pending = None
+        self._stale = False
         self.setup_grid()
 
     # ------------------------------------------------------------------ state (navier_stokes.py:24-35)
     def setup_grid(self):
-        """Reset u, v, p, density (and the unused boundary mask) to zero; drops the pressure warm start."""
+        """Reset u, v, p, density (and the unused boundary mask) to zero; drops the pressure warm start.
+
+        On an existing state the reset is deferred: the next step()/run_steps that runs on the fused kernel builds the zero
+        state (plus the density of a splat issued in between) on chip instead of reading it back from memory; anything else
+        that reads or launches on the state applies the reset first.  What a caller can observe is the same either way."""
         L = self._layout
         if self._arena is None:
             self._arena = torch.zeros(L.total, dtype=torch.float32, device=self._cuda)
@@ -132,11 +140,46 @@ class NavierStokesSimulator(nn.Module):
             st.div = base + 4 * L.offset["div"]
         else:
             self._mirrors.clear()
-            self._arena.zero_()
+            if L.gh == 0:
+                self._pending = []
+            else:
+                self._arena.zero_()                     # slabs are stepped phase by phase: never on the fused kernel
         self._state.cur_u = self._state.cur_v = self._state.cur_d = self._state.cur_p = 0
+
+    def _materialize(self):
+        """Apply a deferred reset and its splats (the eager memset + k_splat), or zero what a consumed reset left stale."""
+        pending, self._pending = self._pending, None
+        if pending is not None:
+            self._arena.zero_()
+            self._stale = False
+            for src, off in pending:
+                _lib.call("smk_splat_sources", C.byref(self._grid), self._ptr("d"), src.data_ptr(), off.data_ptr(),
+                          _lib.stream_on(self._cuda))
+        elif self._stale:
+            L = self._layout
+            for name in ("u1", "v1", "d1", "p1", "div", "boundary"):
+                off = L.offset[name]
+                self._arena[off: off + L.batch * L.stride_of(name)].zero_()
+            self._stale = False
+
+    def _run_reset(self, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, fmt):
+        """A pending reset with at most one splat, consumed by a k_step_fused launch of nsteps steps: True when it ran."""
+        if self._pending is None or len(self._pending) > 1:
+            return False
+        src, off = self._pending[0] if self._pending else (None, None)
+        done = C.c_int32(0)
+        _lib.call("smk_run_steps_reset_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                  frames, frame_step_stride, frame_batch_stride, fmul.data_ptr() if fmul is not None else None, fmt,
+                  src.data_ptr() if src is not None else None, off.data_ptr() if off is not None else None, C.byref(done),
+                  _lib.stream_on(self._cuda))
+        if done.value:
+            self._pending = None
+            self._stale = True
+        return bool(done.value)
 
     def _field(self, name):
         """Strided view [batch, rows, cols] (or [rows, cols] when batch == 1) of a field in the arena."""
+        self._materialize()
         L = self._layout
         rows, cols, pitch = L.shape_of(name)
         off = L.offset[name]
@@ -198,6 +241,7 @@ class NavierStokesSimulator(nn.Module):
     def _stream(self):
         """The stream to launch on.  Also the one place every launch passes through: host copies edited in place are
         written back here, and the library's (statically linked) CUDA runtime is pointed at this simulator's device."""
+        self._materialize()
         self._flush_mirrors()
         return _lib.stream_on(self._cuda)
 
@@ -280,6 +324,9 @@ class NavierStokesSimulator(nn.Module):
         return src_h.to(self._cuda), off_h.to(self._cuda), src_h.numel() + 4 * off_h.numel()
 
     def splat_uploaded(self, src, off):
+        if self._pending == []:                         # right after a reset: the fused launch that consumes it splats
+            self._pending.append((src, off))
+            return
         _lib.call("smk_splat_sources", C.byref(self._grid), self._ptr("d"), src.data_ptr(), off.data_ptr(), self._stream())
 
     def add_sources(self, per_sim):
@@ -389,6 +436,8 @@ class NavierStokesSimulator(nn.Module):
         """
         fmt = _lib.frame_format(frame_dtype)
         fr = self._new_frames(dtype=frame_dtype)
+        if self._run_reset(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt):
+            return self._finish_frames(fr)
         prm = self._params()
         _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), fr.data_ptr(),
                   self._layout.h * self._layout.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -399,6 +448,8 @@ class NavierStokesSimulator(nn.Module):
         or bfloat16 device tensor owned by the caller (no allocation, no sync)."""
         L = self._layout
         fmt = self._check_frame_buffer("frame", frame, (L.batch, L.h, L.pitch_c))
+        if self._run_reset(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt):
+            return
         prm = self._params()
         _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), frame.data_ptr(),
                   L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -419,10 +470,11 @@ class NavierStokesSimulator(nn.Module):
             frame_dtype = torch.float32 if frame_dtype is None else frame_dtype
             fmt = _lib.frame_format(frame_dtype)
             fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
-        prm = self._params()
-        _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
-                  fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c,
-                  fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
+        if not self._run_reset(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt):
+            prm = self._params()
+            _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
+                      fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c,
+                      fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
         return self._finish_frames(fr) if fr is not None else None
 
     def run_steps_time_major(self, nsteps, out, fmul=None):
@@ -430,6 +482,8 @@ class NavierStokesSimulator(nn.Module):
         bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block)."""
         L = self._layout
         fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
+        if self._run_reset(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt):
+            return
         prm = self._params()
         _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps), out.data_ptr(),
                   L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -457,7 +511,7 @@ class NavierStokesSimulator(nn.Module):
 
 
 # every method that launches runs with the simulator's device current and restores the caller's afterwards
-for _name in ("setup_grid", "add_sources", "splat_uploaded", "upload_sources", "diffusion_step", "advection_step", "_bilerp",
+for _name in ("setup_grid", "_materialize", "add_sources", "splat_uploaded", "upload_sources", "diffusion_step", "advection_step", "_bilerp",
               "pressure_projection", "step", "step_into", "run_steps", "run_steps_time_major", "divergence_norms",
               "jacobi_residual_norms", "step_is_fused"):
     setattr(NavierStokesSimulator, _name, _lib.scoped(getattr(NavierStokesSimulator, _name)))
