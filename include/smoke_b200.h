@@ -206,6 +206,22 @@ SMK_API int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const s
                                    void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
                                    const float* fmul, int32_t frame_format, const smk_source_t* sources,
                                    const int32_t* offsets, int32_t* consumed_host, void* stream);
+/*     smk_run_steps_ex with continuous sources: the emitters of (sources, offsets) -- smk_splat_sources' format, both NULL for
+ *     none -- are added to the density at the head of EVERY step, before the buoyancy, exactly as smk_splat_sources followed by
+ *     smk_step_ex would add them (bit-identical frames and state).  Frame t is the density after step t, written before the splat
+ *     of step t + 1; the state left after the call carries no trailing splat.  On k_step_fused and k_step_cluster the emitters
+ *     are splatted on chip (no extra launch); on the phase kernels one k_splat launch precedes each step.  The records are read
+ *     during the launch and must stay valid until it completes.
+ *     reset = 1: the call starts from a freshly reset state splatted with (reset_sources, reset_offsets) (both may be NULL), under
+ *     smk_run_steps_reset_ex's contract: consumed on chip by k_step_fused (*consumed_host = 1, one launch for the reset, the
+ *     one-shot splat and the continuous sources) or nothing is enqueued (*consumed_host = 0) and the caller resets, splats and
+ *     calls again with reset = 0.  Returns SMK_EINVAL before enqueuing anything for nsteps < 1, unpaired sources / offsets,
+ *     reset_sources without reset, or a NULL consumed_host. */
+SMK_API int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                                 void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                                 const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
+                                 int32_t reset, const smk_source_t* reset_sources, const int32_t* reset_offsets,
+                                 int32_t* consumed_host, void* stream);
 /*     1 when a call of nsteps steps (smk_step: 1) would take the fused single-launch path for this grid and params */
 SMK_API int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nsteps, int32_t* fused_host);
 /* Host-only (no GPU needed): the time-sliced schedule smk_run_steps gives the fused kernel when `nsims` simulations of
@@ -353,6 +369,11 @@ SMK_API int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u
  *     for the nsources = offsets[batch] emitters of (sources, offsets); a fixed-order tree per emitter. */
 SMK_API int smk_splat_sources_adjoint(const smk_grid_t* g, const float* g_density, const smk_source_t* sources,
                                       const int32_t* offsets, int32_t nsources, float* g_intensity, void* stream);
+/*     the same with accumulate = 1: g_intensity[k] += that sum (one rounded add per call, so successive calls sum in call order);
+ *     accumulate = 0 is smk_splat_sources_adjoint. */
+SMK_API int smk_splat_sources_adjoint_ex(const smk_grid_t* g, const float* g_density, const smk_source_t* sources,
+                                         const int32_t* offsets, int32_t nsources, int32_t accumulate, float* g_intensity,
+                                         void* stream);
 
 #ifdef __cplusplus
 }

@@ -2,6 +2,7 @@
 
     frames, (u, v, p, d) = autodiff.rollout((u0, v0, p0, d0), nsteps, dt=0.01, viscosity=0.001, jacobi_iters=20)
     d0 = autodiff.add_sources(d0, emitters, intensities)       # emitters[b] = [(x, y, radius), ...]
+    frames, state = autodiff.rollout(state, nsteps, sources=emitters, intensities=intensities)   # emitters at every step
 
 The reference simulator is eager PyTorch, so autograd runs through it: a user can fit emitter intensities to observed frames,
 optimise an initial state or train a model through the simulator.  This module gives the same capability on the CUDA path.
@@ -18,6 +19,12 @@ then apply the adjoint entries of csrc/adjoint.cu in reverse phase order (DESIGN
 and copies here; every gradient is computed by a CUDA kernel.  Gradients are deterministic (bitwise repeatable).
 
 With grad disabled, or when no input requires grad, rollout is run_steps: no checkpoints, no extra copies.
+
+Continuous sources (rollout(..., sources=, intensities=)): the emitters are added to the density at the head of every step, as
+NavierStokesSimulator.set_continuous_sources does, and the forward is that call's run_steps bit for bit.  Checkpoints stay the
+pre-splat states S_t; the backward re-applies the splat to a copy of S_t.d before the recompute.  The splat is an add, so the
+gradient of the splatted density passes unchanged to S_t.d, and the intensity gradient is the sum over steps, t = T-1 down to 0
+in that order, of the splat adjoint of that gradient (smk_splat_sources_adjoint_ex, accumulating): deterministic, no atomics.
 """
 import ctypes as C
 
@@ -82,6 +89,7 @@ class _Config:
         self.dt, self.viscosity, self.jacobi_iters = dt, viscosity, int(jacobi_iters)
         self.add_fractal, self.step_kernel, self.sweeps_per_launch = bool(add_fractal), step_kernel, int(sweeps_per_launch)
         self.B = 1 if batch is None else batch
+        self.src = None                 # continuous sources: (int32 [n, 4] device records with the intensities, offsets, n)
 
     def simulator(self, state):
         sim = NavierStokesSimulator((self.h, self.w), self.dt, self.viscosity, self.device, jacobi_iters=self.jacobi_iters,
@@ -90,6 +98,8 @@ class _Config:
             live = _arena_view(sim, name)
             rows, cols, _ = sim._layout.shape_of(_layout_name(name))
             live[:, :, :cols] = t.detach().reshape(self.B, rows, cols)
+        if self.src is not None:
+            sim._csrc = (None, self.src[0], self.src[1])          # set_continuous_sources with records already on the device
         return sim
 
     def fmul(self):
@@ -130,7 +140,7 @@ def _ptr(t):
 
 class _Rollout(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, cfg, u0, v0, p0, d0):
+    def forward(ctx, cfg, u0, v0, p0, d0, intensities):
         with _lib.on_device(cfg.device):
             sim = cfg.simulator((u0, v0, p0, d0))
             L = sim._layout
@@ -143,8 +153,11 @@ class _Rollout(torch.autograd.Function):
             fmul = cfg.fmul()
             prm = sim._params()
             for t in range(T):
-                _lib.call("smk_step_ex", C.byref(sim._grid), C.byref(sim._state), C.byref(prm),
-                          frames.data_ptr() + 4 * t * L.h * L.pitch_c, T * L.h * L.pitch_c, _ptr(fmul), 0, sim._stream())
+                if cfg.src is None:
+                    _lib.call("smk_step_ex", C.byref(sim._grid), C.byref(sim._state), C.byref(prm),
+                              frames.data_ptr() + 4 * t * L.h * L.pitch_c, T * L.h * L.pitch_c, _ptr(fmul), 0, sim._stream())
+                else:
+                    sim._run_src(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0)
                 for k in _FIELDS:
                     ck[k][t + 1].copy_(_arena_view(sim, k))
             ctx.cfg, ctx.ck, ctx.fmul, ctx.layout, ctx.params = cfg, ck, fmul, L, prm
@@ -160,7 +173,7 @@ class _Rollout(torch.autograd.Function):
         cfg, ck, L, prm = ctx.cfg, ctx.ck, ctx.layout, ctx.params
         with _lib.on_device(cfg.device):
             grads = _reverse(cfg, ck, L, prm, ctx.fmul, g_frames, {"u": g_u, "v": g_v, "p": g_p, "d": g_d})
-        return (None,) + grads
+        return (None,) + grads[:4] + (grads[4] if ctx.needs_input_grad[5] else None,)
 
 
 def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
@@ -185,8 +198,17 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
     ws_jac = torch.empty(5 * B * L.stride_c if cfg.jacobi_iters >= 1 else 4, dtype=torch.float32, device=dev)
     dt, c_uv, c_d = prm.dt, prm.c_uv, prm.c_d
     rows_u, rows_v, rows_c = L.h + 1, L.h, L.h
+    g_int = None
+    if cfg.src is not None:
+        rec, off, n = cfg.src
+        g_int = torch.zeros(n, dtype=torch.float32, device=dev)
+        dsp = zeros("d")                                        # S_t.d with the step's splat, the density the step started from
     for t in range(T - 1, -1, -1):
         u0, v0, d0 = ck["u"][t], ck["v"][t], ck["d"][t]
+        if g_int is not None:
+            dsp.copy_(d0)
+            _lib.call("smk_splat_sources", gp, dsp.data_ptr(), rec.data_ptr(), off.data_ptr(), s)
+            d0 = dsp
         u1, v1, p1 = ck["u"][t + 1], ck["v"][t + 1], ck["p"][t + 1]
         # recompute: buoyancy + diffusions, then the gradient subtract with the pressure the step projected with
         _lib.call("smk_forces_diffuse_div", gp, u0.data_ptr(), v0.data_ptr(), d0.data_ptr(), ud.data_ptr(), vd.data_ptr(),
@@ -212,22 +234,28 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         _lib.call("smk_forces_diffuse_div_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), gdd.data_ptr(), gdiv.data_ptr(),
                   Gn["u"].data_ptr(), Gn["v"].data_ptr(), Gn["d"].data_ptr(), dt, c_uv, c_d, s)
         G, Gn = Gn, G
+        if g_int is not None:   # G.d: the gradient of the splatted density, which is also that of S_t.d
+            _lib.call("smk_splat_sources_adjoint_ex", gp, G["d"].data_ptr(), rec.data_ptr(), off.data_ptr(), n, 1, g_int.data_ptr(), s)
     out = []
     for k in _FIELDS:
         rows, cols, _ = L.shape_of(_layout_name(k))
         out.append(cfg.shape_out(G[k][:, :, :cols].contiguous()))
-    return tuple(out)
+    return tuple(out) + (g_int,)
 
 
 def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fractal=False, step_kernel="auto",
-            sweeps_per_launch=0):
+            sweeps_per_launch=0, sources=None, intensities=None):
     """nsteps steps of NavierStokesSimulator from state = (u, v, p, d); differentiable with respect to all four fields.
 
     u [.., h+1, w], v [.., h, w+1], p [.., h, w], d [.., h, w]: float32 CUDA tensors on one device, with an optional leading
     batch dimension.  Returns (frames, (u, v, p, d)): frames [B, T, h, w] ([T, h, w] for 2-D inputs) and the final state in
     the input shapes, bit-identical to NavierStokesSimulator.run_steps on the same state and parameters (any step_kernel).
     add_fractal multiplies the frames by 1 + 0.05*F as SmokeSimulator.simulate_step does (square grids only).  Gradients of
-    outputs that are not used count as zero; higher-order gradients are not supported."""
+    outputs that are not used count as zero; higher-order gradients are not supported.
+
+    sources / intensities: continuous emitters, added to the density at the head of every step (set_continuous_sources).
+    sources[b] = [(x, y, radius), ...] for simulation b (for 2-D inputs one flat list is accepted too), intensities a 1-D float32
+    tensor on the state's device with one value per emitter in flattened order; differentiable with respect to intensities."""
     batch, h, w, device = _check_state(state)
     if int(nsteps) < 1:
         raise ValueError("nsteps must be >= 1, got %r" % (nsteps,))
@@ -236,8 +264,19 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
     if step_kernel not in _lib.STEP_KERNELS:
         raise ValueError("step_kernel must be one of %s, got %r" % (sorted(_lib.STEP_KERNELS), step_kernel))
     cfg = _Config(batch, h, w, device, nsteps, dt, viscosity, jacobi_iters, add_fractal, step_kernel, sweeps_per_launch)
-    if torch.is_grad_enabled() and any(t.requires_grad for t in state):
-        frames, *final = _Rollout.apply(cfg, *state)
+    if sources is None and intensities is not None:
+        raise ValueError("intensities without sources")
+    if sources is not None:
+        if intensities is None:
+            raise ValueError("sources need intensities: a 1-D float32 tensor, one value per emitter")
+        sources = _emitter_lists(sources, batch is None)
+        rec, off, n = _source_records(sources, cfg.B, device)
+        _check_intensities(intensities, n, device)
+        if n:
+            rec.view(torch.float32)[:n, 3].copy_(intensities.detach())           # smk_source_t.intensity
+            cfg.src = (rec, off, n)
+    if torch.is_grad_enabled() and (any(t.requires_grad for t in state) or (cfg.src is not None and intensities.requires_grad)):
+        frames, *final = _Rollout.apply(cfg, *state, intensities if cfg.src is not None else None)
         return frames, tuple(final)
     with _lib.on_device(device):
         sim = cfg.simulator(state)
@@ -259,12 +298,25 @@ def _source_records(emitters, batch, device):
     flat, offs = [], [0]
     for lst in emitters:
         for e in lst:
-            if len(e) != 3:
+            if not hasattr(e, "__len__") or len(e) != 3:
                 raise ValueError("an emitter is (x, y, radius), got %r" % (e,))
             flat.append([int(e[0]), int(e[1]), int(e[2]), 0])
         offs.append(len(flat))
     rec = torch.tensor(flat if flat else [[0, 0, 0, 0]], dtype=torch.int32).to(device)
     return rec, torch.tensor(offs, dtype=torch.int32).to(device), len(flat)
+
+
+def _emitter_lists(emitters, two_d):
+    """For a 2-D state or density, one flat list of (x, y, radius) stands for [that list]."""
+    if two_d and len(emitters) and len(emitters[0]) and not isinstance(emitters[0][0], (list, tuple)):
+        return [emitters]
+    return emitters
+
+
+def _check_intensities(intensities, n, device):
+    if not torch.is_tensor(intensities) or intensities.dim() != 1 or intensities.dtype != torch.float32 \
+            or intensities.device != device or intensities.numel() != n:
+        raise ValueError("intensities must be a 1-D float32 tensor of %d values on %s" % (n, device))
 
 
 class _AddSources(torch.autograd.Function):
@@ -309,11 +361,8 @@ def add_sources(d0, emitters, intensities):
     if not torch.is_tensor(d0) or d0.dtype != torch.float32 or d0.device.type != "cuda" or d0.dim() not in (2, 3):
         raise ValueError("d0 must be a float32 CUDA tensor [h, w] or [batch, h, w]")
     two_d = d0.dim() == 2
-    if two_d and len(emitters) and len(emitters[0]) and not isinstance(emitters[0][0], (list, tuple)):
-        emitters = [emitters]                           # a 2-D density with one flat list of (x, y, radius)
+    emitters = _emitter_lists(emitters, two_d)
     batch = 1 if two_d else int(d0.shape[0])
     rec, off, n = _source_records(emitters, batch, d0.device)
-    if not torch.is_tensor(intensities) or intensities.dim() != 1 or intensities.dtype != torch.float32 \
-            or intensities.device != d0.device or intensities.numel() != n:
-        raise ValueError("intensities must be a 1-D float32 tensor of %d values on %s" % (n, d0.device))
+    _check_intensities(intensities, n, d0.device)
     return _AddSources.apply(d0, rec, off, n, intensities, two_d)

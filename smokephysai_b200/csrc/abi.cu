@@ -376,8 +376,11 @@ int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, floa
     return smk_step_ex(g, st, prm, frame, frame_stride, fmul, SMK_FRAME_F32, stream);
 }
 
-int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
-                const float* fmul, int32_t frame_format, void* stream)
+}  // extern "C"
+
+// One step; csrc / coff (may be NULL): continuous emitters splatted into the live density at the head of the step.
+static int step_src(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
+                    const float* fmul, int32_t frame_format, const smk_source_t* csrc, const int32_t* coff, void* stream)
 {
     SMK_TRY(check_frames("smk_step", frame, frame_stride, 0, frame_format));
     SMK_TRY(check_grid(g, "smk_step"));
@@ -393,7 +396,9 @@ int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, v
     SMK_TRY(pick_step_kernel(g, prm, 1, &fused));
     if (fused)
         return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], 1, frame, 0, frame_stride,
-                                  fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay, prm->jacobi_iters, st->div, s);
+                                  fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay, prm->jacobi_iters, st->div, s,
+                                  false, nullptr, nullptr, csrc, coff);
+    if (csrc) SMK_TRY(launch_splat(g, st->d[st->cur_d], csrc, coff, s));        // add_smoke_source, then the step (bit-equal by construction)
     const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
     float *u0 = st->u[cu], *u1 = st->u[cu ^ 1], *v0 = st->v[cv], *v1 = st->v[cv ^ 1], *d0 = st->d[cd], *d1 = st->d[cd ^ 1];
     // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
@@ -422,6 +427,14 @@ int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, v
     SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v0, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s,
                           0, nullptr, nullptr, nullptr, frame_format));
     return SMK_OK;
+}
+
+extern "C" {
+
+int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
+                const float* fmul, int32_t frame_format, void* stream)
+{
+    return step_src(g, st, prm, frame, frame_stride, fmul, frame_format, nullptr, nullptr, stream);
 }
 
 int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
@@ -480,6 +493,52 @@ int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
                                frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
                                prm->jacobi_iters, st->div, (cudaStream_t)stream, true, sources, offsets));
     *consumed_host = 1;
+    return SMK_OK;
+}
+
+int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                         int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format,
+                         const smk_source_t* sources, const int32_t* offsets, int32_t reset, const smk_source_t* reset_sources,
+                         const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
+{
+    const char* who = "smk_run_steps_src_ex";
+    if (!consumed_host) return fail(SMK_EINVAL, "%s: consumed_host is NULL", who);
+    *consumed_host = 0;
+    SMK_TRY(check_frames(who, frames, frame_step_stride, frame_batch_stride, frame_format));
+    if (!g || !st || !prm) return fail(SMK_EINVAL, "%s: grid/state/params NULL", who);
+    if ((sources == nullptr) != (offsets == nullptr)) return fail(SMK_EINVAL, "%s: sources and offsets go together", who);
+    if ((reset_sources == nullptr) != (reset_offsets == nullptr)) return fail(SMK_EINVAL, "%s: reset_sources and reset_offsets go together", who);
+    if (reset != 0 && reset != 1) return fail(SMK_EINVAL, "%s: reset must be 0 or 1, got %d", who, reset);
+    if (!reset && reset_sources) return fail(SMK_EINVAL, "%s: reset_sources without a reset", who);
+    if (nsteps < 1) return fail(SMK_EINVAL, "%s: nsteps must be >= 1, got %d", who, nsteps);
+    SMK_TRY(check_grid(g, who));
+    if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
+        return fail(SMK_EUNSUPPORTED, "%s: slab grids are stepped phase by phase with halo exchanges in between", who);
+    SMK_TRY(check_ptrs(who, {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
+    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "%s: cur_* must be 0 or 1", who);
+    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "%s: negative jacobi_iters", who);
+    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "%s: dt must be non-zero", who);
+    int fused = 0;
+    SMK_TRY(pick_step_kernel(g, prm, nsteps, &fused));
+    cudaStream_t s = (cudaStream_t)stream;
+    if (reset) {
+        // consumed on chip by k_step_fused only (the reset splat, then the continuous emitters at the head of step 0): one launch
+        const bool full = g->h == 128 && g->w == 128 && g->pitch_u == 128 && g->pitch_v == 132 && g->pitch_c == 128;
+        if (!fused || (full && pick_cluster(g->batch) != 0)) return SMK_OK;          // not k_step_fused: the caller resets
+        SMK_TRY(launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
+                                   frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
+                                   prm->jacobi_iters, st->div, s, true, reset_sources, reset_offsets, sources, offsets));
+        *consumed_host = 1;
+        return SMK_OK;
+    }
+    if (fused)
+        return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
+                                  frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
+                                  prm->jacobi_iters, st->div, s, false, nullptr, nullptr, sources, offsets);
+    const int64_t step_bytes = frame_step_stride * frame_elem_size(frame_format);
+    for (int t = 0; t < nsteps; ++t)
+        SMK_TRY(step_src(g, st, prm, frames ? static_cast<char*>(frames) + (int64_t)t * step_bytes : nullptr, frame_batch_stride, fmul,
+                         frame_format, sources, offsets, stream));
     return SMK_OK;
 }
 

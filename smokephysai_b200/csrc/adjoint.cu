@@ -286,10 +286,11 @@ k_forces_diffuse_div_adj(DiffAdjIn A, float* __restrict__ gU, float* __restrict_
 // ---- a2 adjoint: add_smoke_source (navier_stokes.py:37-48) -------------------------------------------------------------
 // density += intensity * expf(-dist^2 / denom) over the footprint, so d/d(intensity) = sum g_d * expf(...), with the weight
 // computed exactly as k_splat computes it.  One CTA per emitter; each thread sums a fixed, strided share of the bounding box,
-// then a fixed-order shared-memory tree adds the 256 partial sums.
+// then a fixed-order shared-memory tree adds the 256 partial sums.  accumulate: gI[k] += the sum (one add per launch, so a
+// sequence of launches sums in launch order), else gI[k] = the sum.
 __global__ void __launch_bounds__(256)
 k_splat_adj(const float* __restrict__ gD, const int h, const int w, const int pc, const long long sc, const int batch,
-            const smk_source_t* __restrict__ src, const int32_t* __restrict__ off, float* __restrict__ gI)
+            const smk_source_t* __restrict__ src, const int32_t* __restrict__ off, float* __restrict__ gI, const int accumulate)
 {
     __shared__ float part[256];
     const int k = blockIdx.x, tid = threadIdx.x;
@@ -323,7 +324,7 @@ k_splat_adj(const float* __restrict__ gD, const int h, const int w, const int pc
         if (tid < s) part[tid] = part[tid] + part[tid + s];
         __syncthreads();
     }
-    if (tid == 0) gI[k] = part[0];
+    if (tid == 0) gI[k] = accumulate ? gI[k] + part[0] : part[0];
 }
 
 inline dim3 cells_grid(int rows, int cols, int batch) { return dim3((cols + 31) / 32, (rows + 7) / 8, batch); }
@@ -462,14 +463,21 @@ int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u_diff, c
 int smk_splat_sources_adjoint(const smk_grid_t* g, const float* g_density, const smk_source_t* sources, const int32_t* offsets,
                               int32_t nsources, float* g_intensity, void* stream)
 {
+    return smk_splat_sources_adjoint_ex(g, g_density, sources, offsets, nsources, 0, g_intensity, stream);
+}
+
+int smk_splat_sources_adjoint_ex(const smk_grid_t* g, const float* g_density, const smk_source_t* sources, const int32_t* offsets,
+                                 int32_t nsources, int32_t accumulate, float* g_intensity, void* stream)
+{
     SMK_TRY(adj_grid(g, "smk_splat_sources_adjoint"));
+    if (accumulate != 0 && accumulate != 1) return fail(SMK_EINVAL, "smk_splat_sources_adjoint_ex: accumulate must be 0 or 1");
     if (nsources < 0) return fail(SMK_EINVAL, "smk_splat_sources_adjoint: negative nsources");
     if (nsources == 0) return SMK_OK;
     if (!g_density || !sources || !offsets || !g_intensity) return fail(SMK_EINVAL, "smk_splat_sources_adjoint: NULL pointer");
     if (nsources > 0x7fffffff / 2) return fail(SMK_EUNSUPPORTED, "smk_splat_sources_adjoint: %d emitters", nsources);
     cudaStream_t s = (cudaStream_t)stream;
     ProfScope prof_(SMK_PH_OTHER, s);
-    k_splat_adj<<<nsources, 256, 0, s>>>(g_density, g->h, g->w, g->pitch_c, g->stride_c, g->batch, sources, offsets, g_intensity);
+    k_splat_adj<<<nsources, 256, 0, s>>>(g_density, g->h, g->w, g->pitch_c, g->stride_c, g->batch, sources, offsets, g_intensity, accumulate);
     return check_launch("k_splat_adj");
 }
 

@@ -114,7 +114,8 @@ inline void launch_chain(void (*kernel)(P...), const dim3 grid, const dim3 block
 }
 
 // add_smoke_source at one cell (navier_stokes.py:45-48): acc plus emitter e's Gaussian when cell (i, j) lies within its radius.
-// k_splat and the reset start of k_step_fused add a cell's emitters through this, in list order: bit-identical densities.
+// k_splat, the reset start of k_step_fused and the continuous emitters of k_step_fused / k_step_cluster add a cell's emitters
+// through this, in list order: bit-identical densities.
 __device__ __forceinline__ float splat_add(float acc, const int i, const int j, const smk_source_t& e)
 {
     const long long dx = (long long)j - e.x, dy = (long long)i - e.y;
@@ -197,7 +198,8 @@ int pick_cluster(int batch);          // CTAs per simulation k_step_cluster woul
 int launch_steps_fused(const smk_grid_t* g, float* u, float* v, float* d, float* p, int nsteps, void* frames,
                        int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int frame_format,
                        float dt, float c_uv, float c_d, float decay, int K, float* scratch, cudaStream_t s,
-                       bool reset = false, const smk_source_t* src = nullptr, const int32_t* src_off = nullptr);
+                       bool reset = false, const smk_source_t* src = nullptr, const int32_t* src_off = nullptr,
+                       const smk_source_t* csrc = nullptr, const int32_t* csrc_off = nullptr);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);
 int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int cols, int pitch, int batch, int64_t stride, cudaStream_t s);
 

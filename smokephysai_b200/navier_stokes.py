@@ -33,6 +33,42 @@ def _round4(n):
     return (int(n) + 3) & ~3
 
 
+def check_source_lists(per_sim, batch):
+    """per_sim[b] = [(x, y, radius, intensity), ...] for each of `batch` simulations -> the same as lists of
+    (int, int, int, float) tuples; ValueError for anything else."""
+    if isinstance(per_sim, (str, bytes)) or not hasattr(per_sim, "__len__") or len(per_sim) != batch:
+        raise ValueError("need one emitter list per simulation (%d), got %r" % (batch, per_sim if not hasattr(per_sim, "__len__") else len(per_sim)))
+    out = []
+    for b, lst in enumerate(per_sim):
+        if isinstance(lst, (str, bytes)) or not hasattr(lst, "__iter__"):
+            raise ValueError("emitter list %d is not a list: %r" % (b, lst))
+        recs = []
+        for e in lst:
+            if not hasattr(e, "__len__") or len(e) != 4:
+                raise ValueError("an emitter is (x, y, radius, intensity), got %r in list %d" % (e, b))
+            try:
+                recs.append((int(e[0]), int(e[1]), int(e[2]), float(e[3])))
+            except (TypeError, ValueError):
+                raise ValueError("an emitter is (x, y, radius, intensity) of numbers, got %r in list %d" % (e, b)) from None
+        out.append(recs)
+    return out
+
+
+def pack_sources(per_sim):
+    """Per-simulation emitter lists -> (smk_source_t records as a SOURCE_DTYPE array of at least one record, int32 offsets
+    [len(per_sim) + 1]): simulation b owns records offsets[b] .. offsets[b + 1] - 1, in list order."""
+    flat, offs = [], [0]
+    for lst in per_sim:
+        flat.extend(lst)
+        offs.append(len(flat))
+    rec = np.zeros(max(len(flat), 1), dtype=SOURCE_DTYPE)          # smk_source_t records, 16 B each
+    if flat:
+        arr = np.asarray(flat, dtype=np.float64).reshape(len(flat), 4)
+        rec["x"], rec["y"], rec["radius"] = arr[:, 0].astype(np.int32), arr[:, 1].astype(np.int32), arr[:, 2].astype(np.int32)
+        rec["intensity"] = arr[:, 3].astype(np.float32)
+    return rec, np.asarray(offs, dtype=np.int32)
+
+
 class FieldLayout:
     """Where each field lives inside the single fp32 arena (pure host arithmetic, testable without a GPU).
 
@@ -119,6 +155,9 @@ class NavierStokesSimulator(nn.Module):
         # applied yet; _stale: a run that consumed a reset left the non-live copies, div and boundary as they were before it.
         self._pending = None
         self._stale = False
+        # Continuous sources (set_continuous_sources): None, or (per-simulation lists, device records, device offsets), uploaded once
+        # and splatted at the head of every step by the kernels.
+        self._csrc = None
         self.setup_grid()
 
     # ------------------------------------------------------------------ state (navier_stokes.py:24-35)
@@ -164,14 +203,19 @@ class NavierStokesSimulator(nn.Module):
 
     def _run_reset(self, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, fmt):
         """A pending reset with at most one splat, consumed by a k_step_fused launch of nsteps steps: True when it ran."""
-        if self._pending is None or len(self._pending) > 1:
+        if self._pending is None or len(self._pending) > 1 or nsteps < 1:
             return False
         src, off = self._pending[0] if self._pending else (None, None)
         done = C.c_int32(0)
-        _lib.call("smk_run_steps_reset_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                  frames, frame_step_stride, frame_batch_stride, fmul.data_ptr() if fmul is not None else None, fmt,
-                  src.data_ptr() if src is not None else None, off.data_ptr() if off is not None else None, C.byref(done),
-                  _lib.stream_on(self._cuda))
+        fm = fmul.data_ptr() if fmul is not None else None
+        sp, op = (src.data_ptr(), off.data_ptr()) if src is not None else (None, None)
+        if self._csrc is None:
+            _lib.call("smk_run_steps_reset_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, frame_step_stride, frame_batch_stride, fm, fmt, sp, op, C.byref(done), _lib.stream_on(self._cuda))
+        else:
+            _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, frame_step_stride, frame_batch_stride, fm, fmt, self._csrc[1].data_ptr(), self._csrc[2].data_ptr(),
+                      1, sp, op, C.byref(done), _lib.stream_on(self._cuda))
         if done.value:
             self._pending = None
             self._stale = True
@@ -296,17 +340,9 @@ class NavierStokesSimulator(nn.Module):
         as one H2D copy of 16 B per emitter plus 4 B per simulation."""
         if len(per_sim) != self.batch:
             raise ValueError("need one emitter list per simulation (%d), got %d" % (self.batch, len(per_sim)))
-        flat, offs = [], [0]
-        for lst in per_sim:
-            flat.extend(lst)
-            offs.append(len(flat))
-        rec = np.zeros(max(len(flat), 1), dtype=SOURCE_DTYPE)          # smk_source_t records, 16 B each
-        if flat:
-            arr = np.asarray(flat, dtype=np.float64).reshape(len(flat), 4)
-            rec["x"], rec["y"], rec["radius"] = arr[:, 0].astype(np.int32), arr[:, 1].astype(np.int32), arr[:, 2].astype(np.int32)
-            rec["intensity"] = arr[:, 3].astype(np.float32)
+        rec, offs = pack_sources(per_sim)
         src_h = torch.from_numpy(rec.view(np.uint8))
-        off_h = torch.tensor(offs, dtype=torch.int32)
+        off_h = torch.from_numpy(offs)
         if pin:
             # one cached pinned staging buffer (cudaHostAlloc per call costs more than the copy); the previous
             # call's H2D copy has long been consumed by the splat that followed it on the same stream
@@ -328,6 +364,37 @@ class NavierStokesSimulator(nn.Module):
             self._pending.append((src, off))
             return
         _lib.call("smk_splat_sources", C.byref(self._grid), self._ptr("d"), src.data_ptr(), off.data_ptr(), self._stream())
+
+    def set_continuous_sources(self, per_sim):
+        """Emitters that keep injecting: per_sim[b] = [(x, y, radius, intensity), ...] is added to simulation b's density at the
+        head of every later step (step, step_into, run_steps, run_steps_time_major), before the buoyancy, in list order -- the
+        same cells and weights as add_smoke_source.  run_steps(n) then equals n rounds of add_sources(per_sim); step() bit for
+        bit, on one launch per call.  A frame is the density after its step (before the next step's splat); the state a call
+        leaves carries no trailing splat.  None clears the list.  The records are uploaded once, here; setup_grid() keeps them.
+        The reference's per-phase methods (diffusion_step, advection_step, pressure_projection, ...) do not apply them."""
+        if per_sim is None:
+            self._csrc = None
+            return
+        lists = check_source_lists(per_sim, self.batch)
+        if not any(lists):
+            self._csrc = None
+            return
+        src, off, _ = self.upload_sources(lists)
+        self._csrc = (lists, src, off)
+
+    @property
+    def continuous_sources(self):
+        """The per-simulation lists of set_continuous_sources (a copy), or None when no simulation has one."""
+        return None if self._csrc is None else [list(l) for l in self._csrc[0]]
+
+    def _run_src(self, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, fmt):
+        """nsteps steps with the continuous sources (smk_run_steps_src_ex, no reset)."""
+        if nsteps < 1:
+            return
+        done = C.c_int32(0)
+        _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                  frames, frame_step_stride, frame_batch_stride, fmul.data_ptr() if fmul is not None else None, fmt,
+                  self._csrc[1].data_ptr(), self._csrc[2].data_ptr(), 0, None, None, C.byref(done), self._stream())
 
     def add_sources(self, per_sim):
         """Batched splat: per_sim[b] is the ordered emitter list [(x, y, radius, intensity), ...] of simulation b."""
@@ -438,6 +505,9 @@ class NavierStokesSimulator(nn.Module):
         fr = self._new_frames(dtype=frame_dtype)
         if self._run_reset(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt):
             return self._finish_frames(fr)
+        if self._csrc is not None:
+            self._run_src(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt)
+            return self._finish_frames(fr)
         prm = self._params()
         _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), fr.data_ptr(),
                   self._layout.h * self._layout.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -450,6 +520,8 @@ class NavierStokesSimulator(nn.Module):
         fmt = self._check_frame_buffer("frame", frame, (L.batch, L.h, L.pitch_c))
         if self._run_reset(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt):
             return
+        if self._csrc is not None:
+            return self._run_src(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt)
         prm = self._params()
         _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), frame.data_ptr(),
                   L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -470,7 +542,12 @@ class NavierStokesSimulator(nn.Module):
             frame_dtype = torch.float32 if frame_dtype is None else frame_dtype
             fmt = _lib.frame_format(frame_dtype)
             fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
-        if not self._run_reset(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt):
+        fp = fr.data_ptr() if fr is not None else None
+        if self._run_reset(nsteps, fp, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt):
+            pass
+        elif self._csrc is not None:
+            self._run_src(nsteps, fp, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt)
+        else:
             prm = self._params()
             _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
                       fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c,
@@ -484,6 +561,8 @@ class NavierStokesSimulator(nn.Module):
         fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
         if self._run_reset(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt):
             return
+        if self._csrc is not None:
+            return self._run_src(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt)
         prm = self._params()
         _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps), out.data_ptr(),
                   L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
@@ -511,7 +590,7 @@ class NavierStokesSimulator(nn.Module):
 
 
 # every method that launches runs with the simulator's device current and restores the caller's afterwards
-for _name in ("setup_grid", "_materialize", "add_sources", "splat_uploaded", "upload_sources", "diffusion_step", "advection_step", "_bilerp",
+for _name in ("setup_grid", "_materialize", "add_sources", "set_continuous_sources", "splat_uploaded", "upload_sources", "diffusion_step", "advection_step", "_bilerp",
               "pressure_projection", "step", "step_into", "run_steps", "run_steps_time_major", "divergence_norms",
               "jacobi_residual_norms", "step_is_fused"):
     setattr(NavierStokesSimulator, _name, _lib.scoped(getattr(NavierStokesSimulator, _name)))

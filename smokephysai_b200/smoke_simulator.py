@@ -29,10 +29,19 @@ class SmokeSimulator(nn.Module):
         self.history = []          # smoke_simulator.py:23
         self.max_history = 100     # :24
 
-    def add_incense_source(self, positions, intensities):
-        """Add incense smoke sources: radius is fixed to 8 (smoke_simulator.py:26-29)."""
-        for (x, y), intensity in zip(positions, intensities):
-            self.ns_solver.add_smoke_source(x, y, radius=8, intensity=intensity)
+    def add_incense_source(self, positions, intensities, *, continuous=False):
+        """Add incense smoke sources: radius is fixed to 8 (smoke_simulator.py:26-29).
+
+        continuous=True: sticks that keep burning -- the emitters are appended to every simulation's continuous sources
+        (NavierStokesSimulator.set_continuous_sources) and inject at the head of every later step instead of once."""
+        if not continuous:
+            for (x, y), intensity in zip(positions, intensities):
+                self.ns_solver.add_smoke_source(x, y, radius=8, intensity=intensity)
+            return
+        ns = self.ns_solver
+        new = [(int(x), int(y), 8, float(i)) for (x, y), i in zip(positions, intensities)]
+        lists = ns.continuous_sources or [[] for _ in range(ns.batch)]
+        ns.set_continuous_sources([lst + new for lst in lists])
 
     def simulate_step(self, add_fractal=True):
         """One simulation step; returns the (fractal-scaled) density frame (smoke_simulator.py:31-45)."""
@@ -46,7 +55,7 @@ class SmokeSimulator(nn.Module):
 
     # -------------------------------------------------------------- batched generation (data_loader.py:37-99)
     def generate_sequences(self, emitters, sequence_length=20, add_fractal=True, to_host=False, steps_per_copy=None,
-                           frame_dtype=torch.float32):
+                           frame_dtype=torch.float32, continuous=False):
         """Reset, splat one emitter list per simulation, run sequence_length steps.
 
         emitters[b] = [((x, y), intensity), ...] for simulation b (len == batch).  Returns frames
@@ -63,15 +72,31 @@ class SmokeSimulator(nn.Module):
 
         frame_dtype torch.float16 / torch.bfloat16: the frames are rounded once (to nearest even) by the kernels that
         write them -- equal to the float32 frames' .to(frame_dtype) -- so half the bytes cross PCIe; the simulation
-        itself is the same whatever the dtype."""
+        itself is the same whatever the dtype.
+
+        continuous=True: every sample's emitters inject at the head of every step (a sustained plume) instead of once; frame 0
+        is the same as with continuous=False.  The simulator's own continuous sources are set aside for the call and restored."""
         ns = self.ns_solver
-        L = ns._layout
         B, T = ns.batch, int(sequence_length)
         _lib.frame_format(frame_dtype)                     # ValueError for an unsupported dtype, before any work
+        lists = [[(x, y, 8, inten) for (x, y), inten in lst] for lst in emitters]
         ns.setup_grid()
-        src, off, _ = ns.upload_sources([[(x, y, 8, inten) for (x, y), inten in lst] for lst in emitters], pin=to_host)
-        ns.splat_uploaded(src, off)
+        src, off, _ = ns.upload_sources(lists, pin=to_host)
         fmul = self.fractal_gen.multiplier((ns.h, ns.w), 0.05) if add_fractal else None
+        if not continuous:
+            ns.splat_uploaded(src, off)
+            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype)
+        saved = ns._csrc
+        ns._csrc = (lists, src, off)
+        try:
+            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype)
+        finally:
+            ns._csrc = saved
+
+    def _run_sequences(self, T, fmul, to_host, steps_per_copy, frame_dtype):
+        ns = self.ns_solver
+        L = ns._layout
+        B = ns.batch
         if not to_host:
             fr = ns.run_steps(T, fmul=fmul, frame_dtype=frame_dtype)
             return fr if B > 1 else fr.unsqueeze(0)

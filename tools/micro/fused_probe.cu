@@ -28,7 +28,7 @@ int main(int argc, char** argv)
     cudaMalloc(&fr, (size_t)B * nsteps * nc * 4); cudaMalloc(&ticks, 8 * 8);
     cudaMemset(u, 0, B * nu * 4); cudaMemset(v, 0, B * nv * 4); cudaMemset(p, 0, B * nc * 4);
     cudaMemcpy(d, hd.data(), B * nc * 4, cudaMemcpyHostToDevice);
-    cudaFuncSetAttribute(k_step_fused<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FZ_SMEM);
+    cudaFuncSetAttribute(k_step_fused<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)FZ_SMEM);
     FusedArgs a;
     a.U = u; a.V = v; a.D = d; a.P = p; a.frames = fr; a.fmul = nullptr;
     a.h = 128; a.w = 128; a.pu = 128; a.pv = 132; a.pc = 128; a.su_ = nu; a.sv_ = nv; a.sc_ = nc;
@@ -37,7 +37,7 @@ int main(int argc, char** argv)
     a.ticks = ticks;
     for (int rep = 0; rep < 3; ++rep) {
         cudaMemset(ticks, 0, 64);
-        k_step_fused<true><<<B, FZ_THREADS, FZ_SMEM>>>(a);
+        k_step_fused<true, false><<<B, FZ_THREADS, FZ_SMEM>>>(a);
         cudaDeviceSynchronize();
     }
     long long t[8];
