@@ -178,7 +178,10 @@ SMK_API int smk_advect_slab(const smk_grid_t* g, const float* field, float* out,
 
 /* a3-a11 one full step() / n steps (navier_stokes.py:151-173) over the state.  frames (may be NULL):
  *     [batch][nsteps][h][pitch_c] returned copies, multiplied by (1+fmul) when fmul != NULL.
- *     Not available on a slab grid (the host interleaves halo exchanges between the phases). */
+ *     Not available on a slab grid (the host interleaves halo exchanges between the phases).
+ *     Every step entry point (smk_step, smk_step_ex, smk_run_steps, smk_run_steps_ex, smk_run_steps_reset_ex,
+ *     smk_run_steps_src_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
+ *     jacobi_iters, dt, step_kernel -- and refuses a malformed one before anything is enqueued. */
 SMK_API int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
              float* frame, int64_t frame_stride, const float* fmul, void* stream);
 SMK_API int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,

@@ -7,7 +7,7 @@
 The reference simulator is eager PyTorch, so autograd runs through it: a user can fit emitter intensities to observed frames,
 optimise an initial state or train a model through the simulator.  This module gives the same capability on the CUDA path.
 
-Forward: the existing step (smk_step_ex, phase or fused kernels), one step at a time; after each step the state
+Forward: the simulator's own step (phase or fused kernels), one step at a time; after each step the state
 S_t = (u, v, p, d) is copied into a [T+1, ...] checkpoint buffer, four plain device copies per step.  Frames and final state are
 bit-identical to NavierStokesSimulator.run_steps.  Checkpoint memory, in bytes:
 
@@ -153,11 +153,7 @@ class _Rollout(torch.autograd.Function):
             fmul = cfg.fmul()
             prm = sim._params()
             for t in range(T):
-                if cfg.src is None:
-                    _lib.call("smk_step_ex", C.byref(sim._grid), C.byref(sim._state), C.byref(prm),
-                              frames.data_ptr() + 4 * t * L.h * L.pitch_c, T * L.h * L.pitch_c, _ptr(fmul), 0, sim._stream())
-                else:
-                    sim._run_src(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0)
+                sim._steps(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0)
                 for k in _FIELDS:
                     ck[k][t + 1].copy_(_arena_view(sim, k))
             ctx.cfg, ctx.ck, ctx.fmul, ctx.layout, ctx.params = cfg, ck, fmul, L, prm

@@ -1,5 +1,5 @@
 // abi.cu -- the extern "C" surface of libsmoke_sm100.so (include/smoke_b200.h): argument validation,
-// thread-local error string, and the whole-step orchestration of navier_stokes.py:151-173.
+// thread-local error string, and the one runner behind the step entry points (navier_stokes.py:151-173).
 #include <atomic>
 #include <mutex>
 #include <cstdarg>
@@ -305,13 +305,17 @@ int smk_advect_slab(const smk_grid_t* g, const float* field, float* out, int32_t
     return launch_advect(g, field, out, rows, cols, pitch, 0, u, v, dt, scale, nullptr, 0, nullptr, chk, (cudaStream_t)stream);
 }
 
+// The kernels a step call runs on: one launch per phase per step, or all the steps in one launch of k_step_fused (one CTA per
+// simulation, or the time-sliced schedule) or of k_step_cluster (a cluster of CTAs per simulation).
+enum StepPlan { PLAN_PHASES, PLAN_FUSED, PLAN_CLUSTER };
+
 // SMK_STEP_AUTO: the fused kernel runs one simulation per SM, so it pays off when a call carries enough work per
 // launch -- several steps (the state stays on chip between them), or a single step of at least 32 simulations.
 // One step of a few simulations is faster spread over all SMs by the phase kernels (tools/step_latency.py: 37 us
 // against 45 us per step() at batch 1; the fused launch also reads and writes the state, ~10 us).
-static int pick_step_kernel(const smk_grid_t* g, const smk_params_t* prm, int nsteps, int* fused)
+static int pick_step_kernel(const smk_grid_t* g, const smk_params_t* prm, int nsteps, StepPlan* plan)
 {
-    *fused = 0;
+    *plan = PLAN_PHASES;
     if (prm->step_kernel == SMK_STEP_PHASES) return SMK_OK;
     if (prm->step_kernel != SMK_STEP_AUTO && prm->step_kernel != SMK_STEP_FUSED)
         return fail(SMK_EINVAL, "smk_step: step_kernel %d is not SMK_STEP_AUTO/_PHASES/_FUSED", prm->step_kernel);
@@ -324,11 +328,12 @@ static int pick_step_kernel(const smk_grid_t* g, const smk_params_t* prm, int ns
         // the phase path always wins (64 x 64: 52 against 65 us per step of 148 simulations).
         // Round 2: a few full-size simulations (up to 33) run on clusters of four CTAs (k_step_cluster): 27.3 us per step at K = 40 for
         // 1 .. 32 simulations against 36.6 .. 48.4 on the phase path (tools/cluster_latency.py), so those take the fused path too.
-        const bool full = g->h == 128 && g->w == 128 && g->pitch_u == 128 && g->pitch_v == 132 && g->pitch_c == 128;
+        const bool full = fused_full_size(g);
         const bool big_enough = (long)g->h * g->w >= 96L * 96L;
         const int need = full ? (nsteps >= 2 ? 12 : 48) : 96;
         const bool clustered = full && pick_cluster(g->batch) != 0;
-        *fused = (prm->step_kernel == SMK_STEP_FUSED || clustered || (big_enough && g->batch >= need)) ? 1 : 0;
+        if (prm->step_kernel == SMK_STEP_FUSED || clustered || (big_enough && g->batch >= need))
+            *plan = clustered ? PLAN_CLUSTER : PLAN_FUSED;
         return SMK_OK;
     }
     if (prm->step_kernel == SMK_STEP_FUSED)
@@ -340,9 +345,9 @@ int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nste
 {
     SMK_TRY(check_grid(g, "smk_step_is_fused"));
     if (!prm || !fused_host) return fail(SMK_EINVAL, "smk_step_is_fused: NULL");
-    int f = 0;
-    SMK_TRY(pick_step_kernel(g, prm, nsteps, &f));
-    *fused_host = f;
+    StepPlan plan = PLAN_PHASES;
+    SMK_TRY(pick_step_kernel(g, prm, nsteps, &plan));
+    *fused_host = plan != PLAN_PHASES;
     return SMK_OK;
 }
 
@@ -370,71 +375,56 @@ static int check_frames(const char* who, const void* frames, int64_t stride0, in
     return SMK_OK;
 }
 
+}  // extern "C"
+
+// The one body behind every step entry point: checks the whole call before anything is enqueued, then runs it on the kernels
+// pick_step_kernel chose.  A reset is consumed (*consumed = 1) only on k_step_fused; elsewhere nothing is enqueued and the
+// caller resets and calls again without one.
+static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const StepCall& c,
+                     int32_t* consumed, cudaStream_t s)
+{
+    SMK_TRY(check_frames(who, c.frames, c.frame_step_stride, c.frame_batch_stride, c.frame_format));
+    if (c.nsteps < 0) return fail(SMK_EINVAL, "%s: negative nsteps", who);
+    if (!g || !st || !prm) return fail(SMK_EINVAL, "%s: grid/state/params NULL", who);
+    if ((c.csrc == nullptr) != (c.coff == nullptr)) return fail(SMK_EINVAL, "%s: sources and offsets go together", who);
+    if ((c.rsrc == nullptr) != (c.roff == nullptr)) return fail(SMK_EINVAL, "%s: reset_sources and reset_offsets go together", who);
+    if (!c.reset && c.rsrc) return fail(SMK_EINVAL, "%s: reset_sources without a reset", who);
+    SMK_TRY(check_grid(g, who));
+    if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
+        return fail(SMK_EUNSUPPORTED, "%s: slab grids are stepped phase by phase with halo exchanges in between", who);
+    SMK_TRY(check_ptrs(who, {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
+    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "%s: cur_* must be 0 or 1", who);
+    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "%s: negative jacobi_iters", who);
+    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "%s: dt must be non-zero", who);
+    StepPlan plan = PLAN_PHASES;
+    SMK_TRY(pick_step_kernel(g, prm, c.nsteps, &plan));
+    if (c.nsteps == 0 || (c.reset && plan != PLAN_FUSED)) return SMK_OK;
+    if (plan != PLAN_PHASES) {
+        SMK_TRY(launch_steps_fused(g, st, prm, c, s));
+        if (c.reset) *consumed = 1;
+        return SMK_OK;
+    }
+    const int64_t step_bytes = c.frame_step_stride * frame_elem_size(c.frame_format);
+    for (int t = 0; t < c.nsteps; ++t)
+        SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff, c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
+                           c.frame_batch_stride, c.fmul, c.frame_format, nullptr, nullptr, nullptr, nullptr, s));
+    return SMK_OK;
+}
+
+extern "C" {
+
 int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, float* frame, int64_t frame_stride,
              const float* fmul, void* stream)
 {
     return smk_step_ex(g, st, prm, frame, frame_stride, fmul, SMK_FRAME_F32, stream);
 }
 
-}  // extern "C"
-
-// One step; csrc / coff (may be NULL): continuous emitters splatted into the live density at the head of the step.
-static int step_src(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
-                    const float* fmul, int32_t frame_format, const smk_source_t* csrc, const int32_t* coff, void* stream)
-{
-    SMK_TRY(check_frames("smk_step", frame, frame_stride, 0, frame_format));
-    SMK_TRY(check_grid(g, "smk_step"));
-    if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
-        return fail(SMK_EUNSUPPORTED, "smk_step: slab grids are stepped phase by phase with halo exchanges in between");
-    if (!st || !prm) return fail(SMK_EINVAL, "smk_step: state/params NULL");
-    SMK_TRY(check_ptrs("smk_step", {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
-    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "smk_step: cur_* must be 0 or 1");
-    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "smk_step: negative jacobi_iters");
-    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "smk_step: dt must be non-zero");
-    cudaStream_t s = (cudaStream_t)stream;
-    int fused = 0;
-    SMK_TRY(pick_step_kernel(g, prm, 1, &fused));
-    if (fused)
-        return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], 1, frame, 0, frame_stride,
-                                  fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay, prm->jacobi_iters, st->div, s,
-                                  false, nullptr, nullptr, csrc, coff);
-    if (csrc) SMK_TRY(launch_splat(g, st->d[st->cur_d], csrc, coff, s));        // add_smoke_source, then the step (bit-equal by construction)
-    const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
-    float *u0 = st->u[cu], *u1 = st->u[cu ^ 1], *v0 = st->v[cv], *v1 = st->v[cv ^ 1], *d0 = st->d[cd], *d1 = st->d[cd ^ 1];
-    // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
-    SMK_TRY(launch_forces_diffuse_div(g, u0, v0, d0, u1, v1, d1, st->div, prm->dt, prm->c_uv, prm->c_d, s));
-    // 3. Jacobi sweeps + gradient subtract                                     :139-149
-    int flip = 0;
-    SMK_TRY(launch_jacobi(g, st->div, st->p[st->cur_p], st->p[st->cur_p ^ 1], prm->jacobi_iters, prm->sweeps_per_launch, &flip, s));
-    st->cur_p ^= flip;
-    // On big grids the gradient subtract is fused into the u advection (k_advect_tiled<.., 1>: u, v are projected in shared memory
-    // from a staged pressure window; the projected u is never written, the projected v goes to the spare copy v0, and the v
-    // advection then runs v0 -> v1: the live v ends up in the other copy); else k_project runs on its own.
-    const float* pl = st->p[st->cur_p];
-    const bool fuse = advect_can_fuse_project(g);
-    // 4. sequential advection: u, then v with the new u, then density with both :166-168; 5. decay :171; copy :173
-    if (fuse) {
-        SMK_TRY(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s, 1, pl, v0));
-        SMK_TRY(launch_advect(g, v0, v1, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v0, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
-        SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v1, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s,
-                              0, nullptr, nullptr, nullptr, frame_format));
-        st->cur_v ^= 1;
-        return SMK_OK;
-    }
-    SMK_TRY(launch_project(g, pl, u1, v1, prm->dt, s));
-    SMK_TRY(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
-    SMK_TRY(launch_advect(g, v1, v0, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v1, prm->dt, 1.0f, nullptr, 0, nullptr, nullptr, s));
-    SMK_TRY(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v0, prm->dt, prm->decay, frame, frame_stride, fmul, nullptr, s,
-                          0, nullptr, nullptr, nullptr, frame_format));
-    return SMK_OK;
-}
-
-extern "C" {
-
 int smk_step_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
                 const float* fmul, int32_t frame_format, void* stream)
 {
-    return step_src(g, st, prm, frame, frame_stride, fmul, frame_format, nullptr, nullptr, stream);
+    StepCall c;
+    c.frames = frame; c.frame_batch_stride = frame_stride; c.fmul = fmul; c.frame_format = frame_format;
+    return run_steps("smk_step", g, st, prm, c, nullptr, (cudaStream_t)stream);
 }
 
 int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
@@ -446,28 +436,10 @@ int smk_run_steps(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
 int smk_run_steps_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
                      int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format, void* stream)
 {
-    SMK_TRY(check_frames("smk_run_steps", frames, frame_step_stride, frame_batch_stride, frame_format));
-    if (nsteps < 0) return fail(SMK_EINVAL, "smk_run_steps: negative nsteps");
-    if (nsteps > 1 && g && st && prm) {
-        // the fused kernel keeps the state on chip across all the steps of the call: one launch
-        SMK_TRY(check_grid(g, "smk_run_steps"));
-        int fused = 0;
-        SMK_TRY(pick_step_kernel(g, prm, nsteps, &fused));
-        if (fused) {
-            SMK_TRY(check_ptrs("smk_run_steps", {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1]}));
-            if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "smk_run_steps: cur_* must be 0 or 1");
-            if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "smk_run_steps: negative jacobi_iters");
-            if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "smk_run_steps: dt must be non-zero");
-            return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
-                                      frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
-                                      prm->jacobi_iters, st->div, (cudaStream_t)stream);
-        }
-    }
-    const int64_t step_bytes = frame_step_stride * frame_elem_size(frame_format);
-    for (int t = 0; t < nsteps; ++t)
-        SMK_TRY(smk_step_ex(g, st, prm, frames ? static_cast<char*>(frames) + (int64_t)t * step_bytes : nullptr, frame_batch_stride, fmul,
-                            frame_format, stream));
-    return SMK_OK;
+    StepCall c;
+    c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
+    c.fmul = fmul; c.frame_format = frame_format;
+    return run_steps("smk_run_steps", g, st, prm, c, nullptr, (cudaStream_t)stream);
 }
 
 int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
@@ -476,24 +448,10 @@ int smk_run_steps_reset_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
 {
     if (!consumed_host) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: consumed_host is NULL");
     *consumed_host = 0;
-    SMK_TRY(check_frames("smk_run_steps_reset_ex", frames, frame_step_stride, frame_batch_stride, frame_format));
-    if (!g || !st || !prm) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: grid/state/params NULL");
-    if ((sources == nullptr) != (offsets == nullptr)) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: sources and offsets go together");
-    if (nsteps < 1) return SMK_OK;
-    SMK_TRY(check_grid(g, "smk_run_steps_reset_ex"));
-    int fused = 0;
-    SMK_TRY(pick_step_kernel(g, prm, nsteps, &fused));
-    const bool full = g->h == 128 && g->w == 128 && g->pitch_u == 128 && g->pitch_v == 132 && g->pitch_c == 128;
-    if (!fused || (full && pick_cluster(g->batch) != 0)) return SMK_OK;          // not k_step_fused: the caller resets
-    SMK_TRY(check_ptrs("smk_run_steps_reset_ex", {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
-    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: cur_* must be 0 or 1");
-    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: negative jacobi_iters");
-    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "smk_run_steps_reset_ex: dt must be non-zero");
-    SMK_TRY(launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
-                               frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
-                               prm->jacobi_iters, st->div, (cudaStream_t)stream, true, sources, offsets));
-    *consumed_host = 1;
-    return SMK_OK;
+    StepCall c;
+    c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
+    c.fmul = fmul; c.frame_format = frame_format; c.reset = true; c.rsrc = sources; c.roff = offsets;
+    return run_steps("smk_run_steps_reset_ex", g, st, prm, c, consumed_host, (cudaStream_t)stream);
 }
 
 int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
@@ -504,42 +462,13 @@ int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_
     const char* who = "smk_run_steps_src_ex";
     if (!consumed_host) return fail(SMK_EINVAL, "%s: consumed_host is NULL", who);
     *consumed_host = 0;
-    SMK_TRY(check_frames(who, frames, frame_step_stride, frame_batch_stride, frame_format));
-    if (!g || !st || !prm) return fail(SMK_EINVAL, "%s: grid/state/params NULL", who);
-    if ((sources == nullptr) != (offsets == nullptr)) return fail(SMK_EINVAL, "%s: sources and offsets go together", who);
-    if ((reset_sources == nullptr) != (reset_offsets == nullptr)) return fail(SMK_EINVAL, "%s: reset_sources and reset_offsets go together", who);
     if (reset != 0 && reset != 1) return fail(SMK_EINVAL, "%s: reset must be 0 or 1, got %d", who, reset);
-    if (!reset && reset_sources) return fail(SMK_EINVAL, "%s: reset_sources without a reset", who);
     if (nsteps < 1) return fail(SMK_EINVAL, "%s: nsteps must be >= 1, got %d", who, nsteps);
-    SMK_TRY(check_grid(g, who));
-    if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
-        return fail(SMK_EUNSUPPORTED, "%s: slab grids are stepped phase by phase with halo exchanges in between", who);
-    SMK_TRY(check_ptrs(who, {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
-    if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "%s: cur_* must be 0 or 1", who);
-    if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "%s: negative jacobi_iters", who);
-    if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "%s: dt must be non-zero", who);
-    int fused = 0;
-    SMK_TRY(pick_step_kernel(g, prm, nsteps, &fused));
-    cudaStream_t s = (cudaStream_t)stream;
-    if (reset) {
-        // consumed on chip by k_step_fused only (the reset splat, then the continuous emitters at the head of step 0): one launch
-        const bool full = g->h == 128 && g->w == 128 && g->pitch_u == 128 && g->pitch_v == 132 && g->pitch_c == 128;
-        if (!fused || (full && pick_cluster(g->batch) != 0)) return SMK_OK;          // not k_step_fused: the caller resets
-        SMK_TRY(launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
-                                   frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
-                                   prm->jacobi_iters, st->div, s, true, reset_sources, reset_offsets, sources, offsets));
-        *consumed_host = 1;
-        return SMK_OK;
-    }
-    if (fused)
-        return launch_steps_fused(g, st->u[st->cur_u], st->v[st->cur_v], st->d[st->cur_d], st->p[st->cur_p], nsteps, frames,
-                                  frame_step_stride, frame_batch_stride, fmul, frame_format, prm->dt, prm->c_uv, prm->c_d, prm->decay,
-                                  prm->jacobi_iters, st->div, s, false, nullptr, nullptr, sources, offsets);
-    const int64_t step_bytes = frame_step_stride * frame_elem_size(frame_format);
-    for (int t = 0; t < nsteps; ++t)
-        SMK_TRY(step_src(g, st, prm, frames ? static_cast<char*>(frames) + (int64_t)t * step_bytes : nullptr, frame_batch_stride, fmul,
-                         frame_format, sources, offsets, stream));
-    return SMK_OK;
+    StepCall c;
+    c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
+    c.fmul = fmul; c.frame_format = frame_format; c.csrc = sources; c.coff = offsets;
+    c.reset = reset == 1; c.rsrc = reset_sources; c.roff = reset_offsets;
+    return run_steps(who, g, st, prm, c, consumed_host, (cudaStream_t)stream);
 }
 
 int smk_div_norms(const smk_grid_t* g, const float* u, const float* v, float* out, void* stream)

@@ -194,12 +194,31 @@ int launch_frame_features(const float* frames, int64_t frame_stride, int nframes
                           const float* edges, int nbins, float lo, float hi, int* box_counts, int* hist, float* mean_out, cudaStream_t s);
 int launch_frame_distances(const float* frames, int64_t frame_stride, int nframes, int h, int w, int pitch, double* sumsq, cudaStream_t s);
 bool fused_supported(const smk_grid_t* g);
+bool fused_full_size(const smk_grid_t* g);   // 128 x 128 cells at the natural pitches: the k_step_fused<true, ..> / k_step_cluster grid
 int pick_cluster(int batch);          // CTAs per simulation k_step_cluster would use for `batch` 128 x 128 simulations (0: one CTA each)
-int launch_steps_fused(const smk_grid_t* g, float* u, float* v, float* d, float* p, int nsteps, void* frames,
-                       int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int frame_format,
-                       float dt, float c_uv, float c_d, float decay, int K, float* scratch, cudaStream_t s,
-                       bool reset = false, const smk_source_t* src = nullptr, const int32_t* src_off = nullptr,
-                       const smk_source_t* csrc = nullptr, const int32_t* csrc_off = nullptr);
+
+// One call of the step entry points (smk_step*, smk_run_steps*), everything but the grid, state and params: abi.cu's
+// run_steps validates it and runs it on the phase kernels or on launch_steps_fused.
+struct StepCall {
+    int nsteps = 1;
+    void* frames = nullptr;                   // may be NULL; strides in elements of frame_format (SMK_FRAME_*)
+    int64_t frame_step_stride = 0, frame_batch_stride = 0;
+    const float* fmul = nullptr;
+    int frame_format = SMK_FRAME_F32;
+    const smk_source_t* csrc = nullptr;       // continuous emitters splatted at the head of every step (NULL: none)
+    const int32_t* coff = nullptr;
+    bool reset = false;                       // start from a reset state splatted once with (rsrc, roff): k_step_fused only
+    const smk_source_t* rsrc = nullptr;
+    const int32_t* roff = nullptr;
+};
+int launch_steps_fused(const smk_grid_t* g, const smk_state_t* st, const smk_params_t* prm, const StepCall& c, cudaStream_t s);
+// One step on the phase kernels (peer_halo.cu), for a whole grid or a row slab whose ghost rows are current: the continuous
+// emitters (csrc / coff), buoyancy + diffusion + divergence, the Jacobi sweeps, the gradient subtract and the three advections.
+// All per-call inputs may be NULL: the frame (whole grids), the reach guards chk_* and the comm of the tail push (slabs).
+int phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
+               void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+               const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
+               const smk_peer_comm_t* push_comm, cudaStream_t s);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);
 int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int cols, int pitch, int batch, int64_t stride, cudaStream_t s);
 

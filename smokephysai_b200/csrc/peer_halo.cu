@@ -1,4 +1,5 @@
-// peer_halo.cu -- the slab halo exchange (SURVEY.md s8e) as direct peer stores over NVLink, and the whole slab step issued from C.
+// peer_halo.cu -- the slab halo exchange (SURVEY.md s8e) as direct peer stores over NVLink, and the phase-kernel step that whole
+// grids (abi.cu's run_steps) and row slabs (smk_slab_step) share.
 //
 // Why.  A row slab of an 8192 x 8192 grid on eight GPUs runs ~250 us of kernels per step; the ncclSend / ncclRecv group of
 // nccl_halo.cu costs ~85 us of stream time per exchange for ~10 us of data (NCCL's proxy and FIFO protocol are built for
@@ -16,8 +17,9 @@
 // slot exchange n overwrites.  Counters only grow, so nothing is ever reset between steps or after setup_grid().
 //
 // Both kernels read the exchange number from device memory (seq[0]), not from a launch argument: a captured CUDA graph of the step
-// replays correctly.  smk_slab_step issues exchange + forces/diffusion/divergence + the Jacobi launches + gradient subtract + the
-// three advections from one C call; the results are those of the phase entry points called one by one (same launchers).
+// replays correctly.  smk_slab_step issues the exchange, then phase_step: forces/diffusion/divergence + the Jacobi launches +
+// gradient subtract + the three advections, from one C call; the results are those of the phase entry points called one by one
+// (same launchers).
 #include <cuda.h>
 #include <cstring>
 #include "common.cuh"
@@ -199,16 +201,19 @@ using namespace smk;
 
 #define SMK_TRY_(x) do { const int rc_ = (x); if (rc_ != SMK_OK) return rc_; } while (0)
 
-// The density advection of a step, optionally with the NEXT step's halo push issued from the middle of it (push_comm != NULL):
-// the tile rows that hold the rows this rank sends to its neighbours are advected first (two short launches), then k_halo_push
-// copies the boundary rows of the new u, v, density and of p into the neighbours' mailboxes, then the rest of the field is
-// advected -- the NVLink transfer, the counters' flight and the neighbours' skew hide behind that last launch and the
-// neighbour's own, instead of heading the next step.  new_base: the live u, v, density, p once this step is complete.
+// The density advection of a step, writing the frame (may be NULL) as it goes, or -- slabs, no frame -- with the NEXT step's
+// halo push issued from the middle of it (push_comm != NULL): the tile rows that hold the rows this rank sends to its neighbours
+// are advected first (two short launches), then k_halo_push copies the boundary rows of the new u, v, density and of p into the
+// neighbours' mailboxes, then the rest of the field is advected -- the NVLink transfer, the counters' flight and the neighbours'
+// skew hide behind that last launch and the neighbour's own, instead of heading the next step.  new_base: the live u, v,
+// density, p once this step is complete.
 static int advect_density(const smk_grid_t* g, const float* d_in, float* d_out, const float* u, const float* v, const smk_params_t* prm,
+                          void* frame, int64_t frame_stride, const float* fmul, int frame_format,
                           const smk_slab_check_t* chk_d, cudaStream_t s, const smk_peer_comm_t* push_comm, float* const* new_base)
 {
     if (!push_comm)
-        return launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, 0, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s);
+        return launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, g->stride_c, u, v, prm->dt, prm->decay, frame, frame_stride, fmul,
+                             chk_d, s, 0, nullptr, nullptr, nullptr, frame_format);
     AdvectPart rest = {0, 0, {0, 0}, {0, 0}};
     int nb = 0;
     if (advect_is_tiled(g, g->h, g->w)) {
@@ -227,14 +232,14 @@ static int advect_density(const smk_grid_t* g, const float* d_in, float* d_out, 
         if (nb == 2 && lo[1] < hi[0]) { hi[0] = hi[0] > hi[1] ? hi[0] : hi[1]; nb = 1; }          // overlapping bands: one
         for (int k = 0; k < nb; ++k) {
             const AdvectPart band = {lo[k], hi[k] - lo[k], {0, 0}, {0, 0}};
-            SMK_TRY_(launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, 0, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s,
-                                   0, nullptr, nullptr, &band));
+            SMK_TRY_(launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, g->stride_c, u, v, prm->dt, prm->decay, nullptr, 0, nullptr,
+                                   chk_d, s, 0, nullptr, nullptr, &band));
             rest.skip_lo[k] = lo[k]; rest.skip_n[k] = hi[k] - lo[k];
         }
     }
     if (nb == 0) {
         // small field (direct kernel) or nothing to send: advect everything, then push
-        SMK_TRY_(launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, 0, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s));
+        SMK_TRY_(launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, g->stride_c, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s));
         return peer_xfer(push_comm, new_base, true, s);
     }
     // the push on the side stream (after the bands), the rest of the advection on the caller's; SMK_PUSH_STREAM=0: one stream
@@ -247,17 +252,19 @@ static int advect_density(const smk_grid_t* g, const float* d_in, float* d_out, 
         (void)cudaGetLastError();
         SMK_TRY_(peer_xfer(push_comm, new_base, true, s));
     }
-    return launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, 0, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s,
+    return launch_advect(g, d_in, d_out, g->h, g->w, g->pitch_c, g->stride_c, u, v, prm->dt, prm->decay, nullptr, 0, nullptr, chk_d, s,
                          0, nullptr, nullptr, &rest);
 }
 
-// The tail of a step on a (slab) grid whose live u, v, density are the outputs of forces + diffusion and whose live p holds the
-// K sweeps: gradient subtract (navier_stokes.py:148-149), sequential advection of u, v, density (:166-168), decay (:171).
-// The live copies of u and density flip; so does v's, except on big fields, where the gradient subtract runs inside the u
-// advection (k_advect_tiled<.., 1>, stencil.cu), the projected v passes through the spare copy and the live v ends where it was.
-static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
-                          const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d, cudaStream_t s,
-                          const smk_peer_comm_t* push_comm = nullptr)
+// The tail of a step on a grid or slab whose live u, v, density are the outputs of forces + diffusion and whose live p holds the
+// K sweeps: gradient subtract (navier_stokes.py:148-149), sequential advection of u, v, density (:166-168), decay (:171), the
+// frame copy (:173).  The live copies of u and density flip; so does v's, except on big fields, where the gradient subtract runs
+// inside the u advection (k_advect_tiled<.., 1>, stencil.cu), the projected v passes through the spare copy and the live v ends
+// where it was.
+static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
+                          const float* fmul, int frame_format,
+                          const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
+                          const smk_peer_comm_t* push_comm, cudaStream_t s)
 {
     const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
     float *u1 = st->u[cu], *u0 = st->u[cu ^ 1], *v1 = st->v[cv], *v0 = st->v[cv ^ 1], *d1 = st->d[cd], *d0 = st->d[cd ^ 1];
@@ -265,20 +272,39 @@ static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params
     if (advect_can_fuse_project(g)) {
         // u advection with the gradient subtract inside; it leaves the projected v in the spare copy v0, so the v advection runs
         // v0 -> v1 and the live v stays in the copy it was in
-        SMK_TRY_(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, 0, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_u, s, 1, pl, v0));
-        SMK_TRY_(launch_advect(g, v0, v1, g->h, g->w + 1, g->pitch_v, 0, u0, v0, prm->dt, 1.0f, nullptr, 0, nullptr, chk_v, s));
+        SMK_TRY_(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_u, s, 1, pl, v0));
+        SMK_TRY_(launch_advect(g, v0, v1, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v0, prm->dt, 1.0f, nullptr, 0, nullptr, chk_v, s));
         float* nb_[4] = {u0, v1, d0, pl};
-        SMK_TRY_(advect_density(g, d1, d0, u0, v1, prm, chk_d, s, push_comm, nb_));
+        SMK_TRY_(advect_density(g, d1, d0, u0, v1, prm, frame, frame_stride, fmul, frame_format, chk_d, s, push_comm, nb_));
         st->cur_u = cu ^ 1; st->cur_d = cd ^ 1;
         return SMK_OK;
     }
     SMK_TRY_(launch_project(g, pl, u1, v1, prm->dt, s));
-    SMK_TRY_(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, 0, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_u, s));
-    SMK_TRY_(launch_advect(g, v1, v0, g->h, g->w + 1, g->pitch_v, 0, u0, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_v, s));
+    SMK_TRY_(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_u, s));
+    SMK_TRY_(launch_advect(g, v1, v0, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_v, s));
     float* nb_[4] = {u0, v0, d0, pl};
-    SMK_TRY_(advect_density(g, d1, d0, u0, v0, prm, chk_d, s, push_comm, nb_));
+    SMK_TRY_(advect_density(g, d1, d0, u0, v0, prm, frame, frame_stride, fmul, frame_format, chk_d, s, push_comm, nb_));
     st->cur_u = cu ^ 1; st->cur_v = cv ^ 1; st->cur_d = cd ^ 1;
     return SMK_OK;
+}
+
+int smk::phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
+                    void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+                    const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
+                    const smk_peer_comm_t* push_comm, cudaStream_t s)
+{
+    if (csrc) SMK_TRY_(launch_splat(g, st->d[st->cur_d], csrc, coff, s));     // add_smoke_source, then the step (bit-equal by construction)
+    const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
+    // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
+    SMK_TRY_(launch_forces_diffuse_div(g, st->u[cu], st->v[cv], st->d[cd], st->u[cu ^ 1], st->v[cv ^ 1], st->d[cd ^ 1], st->div,
+                                       prm->dt, prm->c_uv, prm->c_d, s));
+    st->cur_u = cu ^ 1; st->cur_v = cv ^ 1; st->cur_d = cd ^ 1;
+    // 3. Jacobi sweeps                                                         :139-145
+    int flip = 0;
+    SMK_TRY_(launch_jacobi(g, st->div, st->p[st->cur_p], st->p[st->cur_p ^ 1], prm->jacobi_iters, prm->sweeps_per_launch, &flip, s));
+    st->cur_p ^= flip;
+    // 4-5. gradient subtract + the three advections + decay + frame            :148-149, :166-173
+    return project_advect(g, st, prm, frame, frame_stride, fmul, frame_format, chk_u, chk_v, chk_d, push_comm, s);
 }
 
 #define SMK_TRY(x) do { const int rc_ = (x); if (rc_ != SMK_OK) return rc_; } while (0)
@@ -369,18 +395,9 @@ int smk_slab_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
         if (flags & SMK_SLAB_PUSH_HEAD) SMK_TRY(peer_xfer(comm, base, true, s));
         SMK_TRY(peer_xfer(comm, base, false, s));
     }
-    const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
-    // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
-    SMK_TRY(launch_forces_diffuse_div(g, st->u[cu], st->v[cv], st->d[cd], st->u[cu ^ 1], st->v[cv ^ 1], st->d[cd ^ 1], st->div,
-                                      prm->dt, prm->c_uv, prm->c_d, s));
-    st->cur_u = cu ^ 1; st->cur_v = cv ^ 1; st->cur_d = cd ^ 1;
-    // 3. Jacobi sweeps                                                         :139-145
-    int flip = 0;
-    SMK_TRY(launch_jacobi(g, st->div, st->p[st->cur_p], st->p[st->cur_p ^ 1], prm->jacobi_iters, prm->sweeps_per_launch, &flip, s));
-    st->cur_p ^= flip;
-    // 4-5. gradient subtract + the three advections + decay                    :148-149, :166-171
-    //    SMK_SLAB_PUSH_TAIL: the ghost rows of the NEXT step leave from the middle of the density advection
-    return project_advect(g, st, prm, chk_u, chk_v, chk_d, s, (comm && (flags & SMK_SLAB_PUSH_TAIL)) ? comm : nullptr);
+    // SMK_SLAB_PUSH_TAIL: the ghost rows of the NEXT step leave from the middle of the density advection
+    return phase_step(g, st, prm, nullptr, nullptr, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d,
+                      (comm && (flags & SMK_SLAB_PUSH_TAIL)) ? comm : nullptr, s);
 }
 
 int smk_project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
@@ -395,7 +412,7 @@ int smk_project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t*
     if ((st->cur_u | st->cur_v | st->cur_d | st->cur_p) & ~1) return fail(SMK_EINVAL, "smk_project_advect: cur_* must be 0 or 1");
     for (const smk_slab_check_t* c : {chk_u, chk_v, chk_d})
         if (c && (!c->overflow_flag || c->need_lo > c->need_hi || c->valid_lo > c->valid_hi)) return fail(SMK_EINVAL, "smk_project_advect: bad check ranges");
-    return project_advect(g, st, prm, chk_u, chk_v, chk_d, (cudaStream_t)stream);
+    return project_advect(g, st, prm, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d, nullptr, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -201,26 +201,6 @@ class NavierStokesSimulator(nn.Module):
                 self._arena[off: off + L.batch * L.stride_of(name)].zero_()
             self._stale = False
 
-    def _run_reset(self, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, fmt):
-        """A pending reset with at most one splat, consumed by a k_step_fused launch of nsteps steps: True when it ran."""
-        if self._pending is None or len(self._pending) > 1 or nsteps < 1:
-            return False
-        src, off = self._pending[0] if self._pending else (None, None)
-        done = C.c_int32(0)
-        fm = fmul.data_ptr() if fmul is not None else None
-        sp, op = (src.data_ptr(), off.data_ptr()) if src is not None else (None, None)
-        if self._csrc is None:
-            _lib.call("smk_run_steps_reset_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                      frames, frame_step_stride, frame_batch_stride, fm, fmt, sp, op, C.byref(done), _lib.stream_on(self._cuda))
-        else:
-            _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                      frames, frame_step_stride, frame_batch_stride, fm, fmt, self._csrc[1].data_ptr(), self._csrc[2].data_ptr(),
-                      1, sp, op, C.byref(done), _lib.stream_on(self._cuda))
-        if done.value:
-            self._pending = None
-            self._stale = True
-        return bool(done.value)
-
     def _field(self, name):
         """Strided view [batch, rows, cols] (or [rows, cols] when batch == 1) of a field in the arena."""
         self._materialize()
@@ -387,15 +367,6 @@ class NavierStokesSimulator(nn.Module):
         """The per-simulation lists of set_continuous_sources (a copy), or None when no simulation has one."""
         return None if self._csrc is None else [list(l) for l in self._csrc[0]]
 
-    def _run_src(self, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, fmt):
-        """nsteps steps with the continuous sources (smk_run_steps_src_ex, no reset)."""
-        if nsteps < 1:
-            return
-        done = C.c_int32(0)
-        _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                  frames, frame_step_stride, frame_batch_stride, fmul.data_ptr() if fmul is not None else None, fmt,
-                  self._csrc[1].data_ptr(), self._csrc[2].data_ptr(), 0, None, None, C.byref(done), self._stream())
-
     def add_sources(self, per_sim):
         """Batched splat: per_sim[b] is the ordered emitter list [(x, y, radius, intensity), ...] of simulation b."""
         if not any(len(l) for l in per_sim):
@@ -493,6 +464,35 @@ class NavierStokesSimulator(nn.Module):
             fr = fr[0]
         return self._to_out(fr)
 
+    def _offer_reset(self):
+        """The pending reset to hand to the next step call, as (reset sources, offsets) device pointers, or None: a reset with
+        at most one splat can be built on chip; anything else is applied eagerly by _materialize."""
+        if self._pending is None or len(self._pending) > 1:
+            return None
+        return tuple(t.data_ptr() for t in self._pending[0]) if self._pending else (None, None)
+
+    def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt):
+        """nsteps steps of the state, frames (a device pointer or None) at the given strides in elements of frame format fmt.
+
+        One smk_run_steps_src_ex call, with the continuous sources if any.  A pending reset is offered to it first (reset = 1,
+        on the current stream without materializing anything); when the call does not consume it (not on k_step_fused),
+        nothing was enqueued, and the reset is applied eagerly before the call is made again without it."""
+        if nsteps == 0:
+            return                                      # (a negative count goes on to the library, which refuses it)
+        src, off = (self._csrc[1].data_ptr(), self._csrc[2].data_ptr()) if self._csrc is not None else (None, None)
+        fm = fmul.data_ptr() if fmul is not None else None
+        done = C.c_int32(0)
+        offer = self._offer_reset()
+        for reset in ((True, False) if offer is not None else (False,)):
+            rsrc, roff = offer if reset else (None, None)
+            _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, step_stride, batch_stride, fm, fmt, src, off, int(reset), rsrc, roff, C.byref(done),
+                      _lib.stream_on(self._cuda) if reset else self._stream())
+            if done.value:
+                self._pending = None
+                self._stale = True
+                return
+
     def step(self, fmul=None, *, frame_dtype=torch.float32):
         """One time step; returns a copy of the new density ([h, w], or [batch, h, w]).
 
@@ -503,14 +503,7 @@ class NavierStokesSimulator(nn.Module):
         """
         fmt = _lib.frame_format(frame_dtype)
         fr = self._new_frames(dtype=frame_dtype)
-        if self._run_reset(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt):
-            return self._finish_frames(fr)
-        if self._csrc is not None:
-            self._run_src(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt)
-            return self._finish_frames(fr)
-        prm = self._params()
-        _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), fr.data_ptr(),
-                  self._layout.h * self._layout.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
+        self._steps(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt)
         return self._finish_frames(fr)
 
     def step_into(self, frame, fmul=None):
@@ -518,13 +511,7 @@ class NavierStokesSimulator(nn.Module):
         or bfloat16 device tensor owned by the caller (no allocation, no sync)."""
         L = self._layout
         fmt = self._check_frame_buffer("frame", frame, (L.batch, L.h, L.pitch_c))
-        if self._run_reset(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt):
-            return
-        if self._csrc is not None:
-            return self._run_src(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt)
-        prm = self._params()
-        _lib.call("smk_step_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), frame.data_ptr(),
-                  L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
+        self._steps(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt)
 
     def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None):
         """nsteps consecutive steps enqueued back to back; returns frames [batch, nsteps, h, w] ([nsteps, h, w] if batch == 1).
@@ -542,16 +529,7 @@ class NavierStokesSimulator(nn.Module):
             frame_dtype = torch.float32 if frame_dtype is None else frame_dtype
             fmt = _lib.frame_format(frame_dtype)
             fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
-        fp = fr.data_ptr() if fr is not None else None
-        if self._run_reset(nsteps, fp, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt):
-            pass
-        elif self._csrc is not None:
-            self._run_src(nsteps, fp, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt)
-        else:
-            prm = self._params()
-            _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps),
-                      fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c,
-                      fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
+        self._steps(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt)
         return self._finish_frames(fr) if fr is not None else None
 
     def run_steps_time_major(self, nsteps, out, fmul=None):
@@ -559,13 +537,7 @@ class NavierStokesSimulator(nn.Module):
         bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block)."""
         L = self._layout
         fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
-        if self._run_reset(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt):
-            return
-        if self._csrc is not None:
-            return self._run_src(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt)
-        prm = self._params()
-        _lib.call("smk_run_steps_ex", C.byref(self._grid), C.byref(self._state), C.byref(prm), int(nsteps), out.data_ptr(),
-                  L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul.data_ptr() if fmul is not None else None, fmt, self._stream())
+        self._steps(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt)
 
     def divergence_norms(self):
         """(max|div|, ||div||_2) of the un-normalised divergence of the live (u, v), per simulation: [batch, 2] on the host."""

@@ -382,3 +382,66 @@ def test_rejections_before_any_launch():
                dict(sources=[[(1, 2)], []], intensities=torch.ones(1, device=DEV))):
         with pytest.raises(ValueError):
             autodiff.rollout(tuple(st), 2, **kw)
+
+
+@pytest.mark.parametrize("kernel", ["phases", "fused"])
+def test_every_step_entry_refuses_the_same_malformed_calls_before_any_launch(kernel):
+    """smk_step, smk_step_ex, smk_run_steps, smk_run_steps_ex, smk_run_steps_reset_ex and smk_run_steps_src_ex check a call the
+    same way, whichever kernel it would run on: each malformed grid, state, params or frame below is refused by every one of
+    them with nothing enqueued, and the well-formed calls then run."""
+    from smokephysai_b200 import _lib
+    h, w, B = (128, 128, 48) if kernel == "fused" else (32, 32, 2)      # 48 full-size simulations: k_step_fused, not clusters
+    ns = make(h, w, B, 20, step_kernel=kernel)
+    assert ns.step_is_fused(1) == ns.step_is_fused(2) == (kernel == "fused")
+    L, lib = ns._layout, _lib.load()
+    fr = torch.empty(B, 2, L.h, L.pitch_c, device=DEV)
+    src, off, _ = ns.upload_sources([[(5, 5, 3, 1.0)] for _ in range(B)])
+    s = _lib.stream_on(ns._cuda)
+    step, batch = L.h * L.pitch_c, 2 * L.h * L.pitch_c
+    done = C.c_int32(0)
+    entries = {
+        "smk_step": lambda g, st, prm, f: lib.smk_step(g, st, prm, f, batch, None, s),
+        "smk_step_ex": lambda g, st, prm, f: lib.smk_step_ex(g, st, prm, f, batch, None, 0, s),
+        "smk_run_steps": lambda g, st, prm, f: lib.smk_run_steps(g, st, prm, 2, f, step, batch, None, s),
+        "smk_run_steps_ex": lambda g, st, prm, f: lib.smk_run_steps_ex(g, st, prm, 2, f, step, batch, None, 0, s),
+        "smk_run_steps_reset_ex": lambda g, st, prm, f: lib.smk_run_steps_reset_ex(g, st, prm, 2, f, step, batch, None, 0,
+                                                                                   src.data_ptr(), off.data_ptr(), C.byref(done), s),
+        "smk_run_steps_src_ex": lambda g, st, prm, f: lib.smk_run_steps_src_ex(g, st, prm, 2, f, step, batch, None, 0, src.data_ptr(),
+                                                                               off.data_ptr(), 0, None, None, C.byref(done), s),
+    }
+
+    def edit(x, **fields):
+        y = type(x).from_buffer_copy(x)
+        for k, v in fields.items():
+            if isinstance(v, tuple):                # (copy index, pointer) of a ping-pong pair
+                getattr(y, k)[v[0]] = v[1]
+            else:
+                setattr(y, k, v)
+        return y
+    G, S, P, F = ns._grid, ns._state, ns._params(), fr.data_ptr()
+    bad = {
+        "NULL grid": (None, S, P, F),
+        "NULL state": (G, None, P, F),
+        "NULL params": (G, S, None, F),
+        "batch 0": (edit(G, batch=0), S, P, F),
+        "slab grid": (edit(G, gh=G.h + 8, row0=4), S, P, F),
+        "NULL div": (G, edit(S, div=None), P, F),
+        "NULL spare u": (G, edit(S, u=(S.cur_u ^ 1, None)), P, F),
+        "misaligned spare density": (G, edit(S, d=(S.cur_d ^ 1, S.d[S.cur_d ^ 1] + 4)), P, F),
+        "cur_v 2": (G, edit(S, cur_v=2), P, F),
+        "negative jacobi_iters": (G, S, edit(P, jacobi_iters=-1), F),
+        "dt 0": (G, S, edit(P, dt=0.0), F),
+        "unknown step_kernel": (G, S, edit(P, step_kernel=7), F),
+        "misaligned frames": (G, S, P, F + 4),
+    }
+    ref = lambda x: C.byref(x) if x is not None else None
+    torch.cuda.synchronize()
+    n0 = _lib.launch_count()
+    for name, call in entries.items():
+        for what, (g, st, prm, f) in bad.items():
+            assert call(ref(g), ref(st), ref(prm), f) != 0, "%s accepted a call with %s" % (name, what)
+            assert _lib.launch_count() == n0, "%s launched on a call with %s" % (name, what)
+    for name, call in entries.items():
+        assert call(ref(G), ref(S), ref(P), F) == 0, "%s: %s" % (name, lib.smk_last_error_string())
+    torch.cuda.synchronize()
+    assert _lib.launch_count() > n0

@@ -23,8 +23,9 @@ def make(h, w, B, K, device="cuda:0", **kw):
 
 
 def eager(ns):
-    """Force the eager reset: no launch consumes the pending reset, so the next launch applies it with memset + k_splat."""
-    ns._run_reset = lambda *args: False
+    """Force the eager reset: the pending reset is never offered to a step call, so the next launch applies it with memset +
+    k_splat."""
+    ns._offer_reset = lambda: None
     return ns
 
 
