@@ -180,7 +180,7 @@ SMK_API int smk_advect_slab(const smk_grid_t* g, const float* field, float* out,
  *     [batch][nsteps][h][pitch_c] returned copies, multiplied by (1+fmul) when fmul != NULL.
  *     Not available on a slab grid (the host interleaves halo exchanges between the phases).
  *     Every step entry point (smk_step, smk_step_ex, smk_run_steps, smk_run_steps_ex, smk_run_steps_reset_ex,
- *     smk_run_steps_src_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
+ *     smk_run_steps_src_ex, smk_run_steps_sched_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
  *     jacobi_iters, dt, step_kernel -- and refuses a malformed one before anything is enqueued. */
 SMK_API int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
              float* frame, int64_t frame_stride, const float* fmul, void* stream);
@@ -225,6 +225,18 @@ SMK_API int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk
                                  const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
                                  int32_t reset, const smk_source_t* reset_sources, const int32_t* reset_offsets,
                                  int32_t* consumed_host, void* stream);
+/*     smk_run_steps_src_ex with a source schedule: emitters that move or change intensity from step to step.  With
+ *     offsets_step_stride = g->batch, offsets holds nsteps * batch + 1 entries, step-major, and step t (0 .. nsteps - 1 of this
+ *     call) of simulation b adds records [offsets[t * batch + b], offsets[t * batch + b + 1]) at its head, exactly as
+ *     smk_splat_sources with that row followed by smk_step_ex would (bit-identical frames and state, same frame and reset
+ *     contract as smk_run_steps_src_ex).  An emitter with radius < 0 adds
+ *     nothing, which pads rows of different lengths to one width.  Any other stride, or a non-zero stride without sources,
+ *     is SMK_EINVAL before anything is enqueued.  smk_run_steps_src_ex is this entry with offsets_step_stride = 0. */
+SMK_API int smk_run_steps_sched_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                                   void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                                   const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
+                                   int32_t offsets_step_stride, int32_t reset, const smk_source_t* reset_sources,
+                                   const int32_t* reset_offsets, int32_t* consumed_host, void* stream);
 /*     1 when a call of nsteps steps (smk_step: 1) would take the fused single-launch path for this grid and params */
 SMK_API int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nsteps, int32_t* fused_host);
 /* Host-only (no GPU needed): the time-sliced schedule smk_run_steps gives the fused kernel when `nsims` simulations of

@@ -3,6 +3,7 @@
     frames, (u, v, p, d) = autodiff.rollout((u0, v0, p0, d0), nsteps, dt=0.01, viscosity=0.001, jacobi_iters=20)
     d0 = autodiff.add_sources(d0, emitters, intensities)       # emitters[b] = [(x, y, radius), ...]
     frames, state = autodiff.rollout(state, nsteps, sources=emitters, intensities=intensities)   # emitters at every step
+    frames, state = autodiff.rollout(state, nsteps, schedule=(xy, radius), intensities=I)       # an emission history, I [T, B, E]
 
 The reference simulator is eager PyTorch, so autograd runs through it: a user can fit emitter intensities to observed frames,
 optimise an initial state or train a model through the simulator.  This module gives the same capability on the CUDA path.
@@ -25,6 +26,11 @@ NavierStokesSimulator.set_continuous_sources does, and the forward is that call'
 pre-splat states S_t; the backward re-applies the splat to a copy of S_t.d before the recompute.  The splat is an add, so the
 gradient of the splatted density passes unchanged to S_t.d, and the intensity gradient is the sum over steps, t = T-1 down to 0
 in that order, of the splat adjoint of that gradient (smk_splat_sources_adjoint_ex, accumulating): deterministic, no atomics.
+
+Source schedules (rollout(..., schedule=(xy, radius), intensities=I)): row t of the schedule is added at the head of step t, as
+NavierStokesSimulator.run_steps(schedule=) does, and the forward is that call bit for bit.  The backward splats a copy of S_t.d with
+row t, and the gradient of step t's intensities is the splat adjoint of that step alone (smk_splat_sources_adjoint_ex on row t's
+records, not accumulating), so I.grad[t] is exactly that of step t and padded entries (radius < 0) get exactly 0.
 """
 import ctypes as C
 
@@ -32,7 +38,7 @@ import torch
 
 from . import _lib
 from .fractal_generator import FractalGenerator
-from .navier_stokes import FieldLayout, NavierStokesSimulator
+from .navier_stokes import FieldLayout, NavierStokesSimulator, pack_schedule, schedule_offsets
 
 __all__ = ["rollout", "add_sources"]
 
@@ -90,6 +96,7 @@ class _Config:
         self.add_fractal, self.step_kernel, self.sweeps_per_launch = bool(add_fractal), step_kernel, int(sweeps_per_launch)
         self.B = 1 if batch is None else batch
         self.src = None                 # continuous sources: (int32 [n, 4] device records with the intensities, offsets, n)
+        self.sched = None               # schedule: (int32 [T * B * E, 4] device records with the intensities, offsets [T * B + 1], E)
 
     def simulator(self, state):
         sim = NavierStokesSimulator((self.h, self.w), self.dt, self.viscosity, self.device, jacobi_iters=self.jacobi_iters,
@@ -101,6 +108,12 @@ class _Config:
         if self.src is not None:
             sim._csrc = (None, self.src[0], self.src[1])          # set_continuous_sources with records already on the device
         return sim
+
+    def step_sched(self, t0):
+        """_steps' schedule argument for a call whose step 0 is step t0 of the rollout (None without a schedule)."""
+        if self.sched is None:
+            return None
+        return self.sched[:2] + (t0,)
 
     def fmul(self):
         if not self.add_fractal:
@@ -153,7 +166,7 @@ class _Rollout(torch.autograd.Function):
             fmul = cfg.fmul()
             prm = sim._params()
             for t in range(T):
-                sim._steps(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0)
+                sim._steps(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0, cfg.step_sched(t))
                 for k in _FIELDS:
                     ck[k][t + 1].copy_(_arena_view(sim, k))
             ctx.cfg, ctx.ck, ctx.fmul, ctx.layout, ctx.params = cfg, ck, fmul, L, prm
@@ -199,11 +212,16 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         rec, off, n = cfg.src
         g_int = torch.zeros(n, dtype=torch.float32, device=dev)
         dsp = zeros("d")                                        # S_t.d with the step's splat, the density the step started from
+    elif cfg.sched is not None:
+        rec, off, E = cfg.sched
+        g_int = torch.zeros(T, B, E, dtype=torch.float32, device=dev)
+        row_off = schedule_offsets(1, B, E, dev)                # one row of B lists of E entries, for the per-step adjoint
+        dsp = zeros("d")
     for t in range(T - 1, -1, -1):
         u0, v0, d0 = ck["u"][t], ck["v"][t], ck["d"][t]
         if g_int is not None:
             dsp.copy_(d0)
-            _lib.call("smk_splat_sources", gp, dsp.data_ptr(), rec.data_ptr(), off.data_ptr(), s)
+            _lib.call("smk_splat_sources", gp, dsp.data_ptr(), rec.data_ptr(), off.data_ptr() + (4 * t * B if cfg.sched else 0), s)
             d0 = dsp
         u1, v1, p1 = ck["u"][t + 1], ck["v"][t + 1], ck["p"][t + 1]
         # recompute: buoyancy + diffusions, then the gradient subtract with the pressure the step projected with
@@ -230,8 +248,12 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         _lib.call("smk_forces_diffuse_div_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), gdd.data_ptr(), gdiv.data_ptr(),
                   Gn["u"].data_ptr(), Gn["v"].data_ptr(), Gn["d"].data_ptr(), dt, c_uv, c_d, s)
         G, Gn = Gn, G
-        if g_int is not None:   # G.d: the gradient of the splatted density, which is also that of S_t.d
+        # G.d: the gradient of the splatted density, which is also that of S_t.d
+        if cfg.src is not None:
             _lib.call("smk_splat_sources_adjoint_ex", gp, G["d"].data_ptr(), rec.data_ptr(), off.data_ptr(), n, 1, g_int.data_ptr(), s)
+        elif cfg.sched is not None:
+            _lib.call("smk_splat_sources_adjoint_ex", gp, G["d"].data_ptr(), rec.data_ptr() + 16 * t * B * E, row_off.data_ptr(),
+                      B * E, 0, g_int[t].data_ptr(), s)
     out = []
     for k in _FIELDS:
         rows, cols, _ = L.shape_of(_layout_name(k))
@@ -240,7 +262,7 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
 
 
 def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fractal=False, step_kernel="auto",
-            sweeps_per_launch=0, sources=None, intensities=None):
+            sweeps_per_launch=0, sources=None, intensities=None, schedule=None):
     """nsteps steps of NavierStokesSimulator from state = (u, v, p, d); differentiable with respect to all four fields.
 
     u [.., h+1, w], v [.., h, w+1], p [.., h, w], d [.., h, w]: float32 CUDA tensors on one device, with an optional leading
@@ -251,7 +273,11 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
 
     sources / intensities: continuous emitters, added to the density at the head of every step (set_continuous_sources).
     sources[b] = [(x, y, radius), ...] for simulation b (for 2-D inputs one flat list is accepted too), intensities a 1-D float32
-    tensor on the state's device with one value per emitter in flattened order; differentiable with respect to intensities."""
+    tensor on the state's device with one value per emitter in flattened order; differentiable with respect to intensities.
+
+    schedule = (xy, radius) / intensities: an emission history, row t added at the head of step t (run_steps(schedule=)).
+    xy integer [T, B, E, 2], radius integer [T, B, E] (B = 1 for 2-D inputs; radius < 0 pads), intensities float32 [T, B, E]
+    on the state's device, differentiable.  Exclusive with sources=."""
     batch, h, w, device = _check_state(state)
     if int(nsteps) < 1:
         raise ValueError("nsteps must be >= 1, got %r" % (nsteps,))
@@ -260,9 +286,13 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
     if step_kernel not in _lib.STEP_KERNELS:
         raise ValueError("step_kernel must be one of %s, got %r" % (sorted(_lib.STEP_KERNELS), step_kernel))
     cfg = _Config(batch, h, w, device, nsteps, dt, viscosity, jacobi_iters, add_fractal, step_kernel, sweeps_per_launch)
-    if sources is None and intensities is not None:
-        raise ValueError("intensities without sources")
-    if sources is not None:
+    if sources is not None and schedule is not None:
+        raise ValueError("sources= and schedule= do not combine: fold the constant emitters into the schedule")
+    if sources is None and schedule is None and intensities is not None:
+        raise ValueError("intensities without sources or a schedule")
+    if schedule is not None:
+        cfg.sched = _schedule_records(schedule, intensities, cfg.nsteps, cfg.B, device)
+    elif sources is not None:
         if intensities is None:
             raise ValueError("sources need intensities: a 1-D float32 tensor, one value per emitter")
         sources = _emitter_lists(sources, batch is None)
@@ -271,12 +301,13 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
         if n:
             rec.view(torch.float32)[:n, 3].copy_(intensities.detach())           # smk_source_t.intensity
             cfg.src = (rec, off, n)
-    if torch.is_grad_enabled() and (any(t.requires_grad for t in state) or (cfg.src is not None and intensities.requires_grad)):
-        frames, *final = _Rollout.apply(cfg, *state, intensities if cfg.src is not None else None)
+    differentiable = cfg.src is not None or cfg.sched is not None
+    if torch.is_grad_enabled() and (any(t.requires_grad for t in state) or (differentiable and intensities.requires_grad)):
+        frames, *final = _Rollout.apply(cfg, *state, intensities if differentiable else None)
         return frames, tuple(final)
     with _lib.on_device(device):
         sim = cfg.simulator(state)
-        frames = sim.run_steps(cfg.nsteps, fmul=cfg.fmul())
+        frames = sim._run_steps(cfg.nsteps, cfg.fmul(), True, None, None, cfg.step_sched(0))
         if batch is not None and cfg.B == 1:
             frames = frames.unsqueeze(0)
         final = []
@@ -300,6 +331,27 @@ def _source_records(emitters, batch, device):
         offs.append(len(flat))
     rec = torch.tensor(flat if flat else [[0, 0, 0, 0]], dtype=torch.int32).to(device)
     return rec, torch.tensor(offs, dtype=torch.int32).to(device), len(flat)
+
+
+def _schedule_records(schedule, intensities, T, B, device):
+    """(xy, radius) and the intensities [T, B, E] -> (int32 [T * B * E, 4] device records with the intensities, offsets, E), or
+    None for E == 0.  ValueError for anything pack_schedule refuses or intensities of another shape, dtype or device."""
+    if not isinstance(schedule, (tuple, list)) or len(schedule) != 2:
+        raise ValueError("rollout's schedule is (xy, radius); the intensities go in intensities=")
+    if intensities is None:
+        raise ValueError("a schedule needs intensities: a float32 [T, B, E] tensor")
+    xy, radius = schedule
+    shape = tuple(getattr(radius, "shape", ()))
+    if not torch.is_tensor(intensities) or intensities.dtype != torch.float32 or intensities.device != device \
+            or tuple(intensities.shape) != shape:
+        raise ValueError("intensities must be a float32 tensor on %s shaped like radius %s" % (device, shape))
+    rdev = radius.device if torch.is_tensor(radius) else torch.device("cpu")
+    rec, E = pack_schedule((xy, radius, torch.zeros(shape, dtype=torch.float32, device=rdev)), T, B)
+    if rec is None:
+        return None
+    rec = rec.to(device)
+    rec[:, 3] = intensities.detach().reshape(-1).view(torch.int32)           # smk_source_t.intensity bits
+    return rec, schedule_offsets(T, B, E, device), E
 
 
 def _emitter_lists(emitters, two_d):

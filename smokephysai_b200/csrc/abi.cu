@@ -387,6 +387,8 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
     if (c.nsteps < 0) return fail(SMK_EINVAL, "%s: negative nsteps", who);
     if (!g || !st || !prm) return fail(SMK_EINVAL, "%s: grid/state/params NULL", who);
     if ((c.csrc == nullptr) != (c.coff == nullptr)) return fail(SMK_EINVAL, "%s: sources and offsets go together", who);
+    if (c.cstride != 0 && (!c.csrc || c.cstride != g->batch))
+        return fail(SMK_EINVAL, "%s: offsets_step_stride must be 0 or the batch (%d) with sources, got %d", who, g->batch, c.cstride);
     if ((c.rsrc == nullptr) != (c.roff == nullptr)) return fail(SMK_EINVAL, "%s: reset_sources and reset_offsets go together", who);
     if (!c.reset && c.rsrc) return fail(SMK_EINVAL, "%s: reset_sources without a reset", who);
     SMK_TRY(check_grid(g, who));
@@ -406,7 +408,7 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
     }
     const int64_t step_bytes = c.frame_step_stride * frame_elem_size(c.frame_format);
     for (int t = 0; t < c.nsteps; ++t)
-        SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff, c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
+        SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff ? c.coff + (int64_t)t * c.cstride : nullptr, c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
                            c.frame_batch_stride, c.fmul, c.frame_format, nullptr, nullptr, nullptr, nullptr, s));
     return SMK_OK;
 }
@@ -459,14 +461,23 @@ int smk_run_steps_src_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_
                          const smk_source_t* sources, const int32_t* offsets, int32_t reset, const smk_source_t* reset_sources,
                          const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
 {
-    const char* who = "smk_run_steps_src_ex";
+    return smk_run_steps_sched_ex(g, st, prm, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, frame_format, sources,
+                                  offsets, 0, reset, reset_sources, reset_offsets, consumed_host, stream);
+}
+
+int smk_run_steps_sched_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                           int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format,
+                           const smk_source_t* sources, const int32_t* offsets, int32_t offsets_step_stride, int32_t reset,
+                           const smk_source_t* reset_sources, const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
+{
+    const char* who = "smk_run_steps_sched_ex";
     if (!consumed_host) return fail(SMK_EINVAL, "%s: consumed_host is NULL", who);
     *consumed_host = 0;
     if (reset != 0 && reset != 1) return fail(SMK_EINVAL, "%s: reset must be 0 or 1, got %d", who, reset);
     if (nsteps < 1) return fail(SMK_EINVAL, "%s: nsteps must be >= 1, got %d", who, nsteps);
     StepCall c;
     c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
-    c.fmul = fmul; c.frame_format = frame_format; c.csrc = sources; c.coff = offsets;
+    c.fmul = fmul; c.frame_format = frame_format; c.csrc = sources; c.coff = offsets; c.cstride = offsets_step_stride;
     c.reset = reset == 1; c.rsrc = reset_sources; c.roff = reset_offsets;
     return run_steps(who, g, st, prm, c, consumed_host, (cudaStream_t)stream);
 }

@@ -205,8 +205,9 @@ struct StepCall {
     int64_t frame_step_stride = 0, frame_batch_stride = 0;
     const float* fmul = nullptr;
     int frame_format = SMK_FRAME_F32;
-    const smk_source_t* csrc = nullptr;       // continuous emitters splatted at the head of every step (NULL: none)
-    const int32_t* coff = nullptr;
+    const smk_source_t* csrc = nullptr;       // emitters splatted at the head of every step (NULL: none); step t of simulation b
+    const int32_t* coff = nullptr;            //   adds records [coff[t * cstride + b], coff[t * cstride + b + 1])
+    int cstride = 0;                          // 0: one list for every step (continuous sources); batch: a schedule, a row per step
     bool reset = false;                       // start from a reset state splatted once with (rsrc, roff): k_step_fused only
     const smk_source_t* rsrc = nullptr;
     const int32_t* roff = nullptr;

@@ -69,6 +69,63 @@ def pack_sources(per_sim):
     return rec, np.asarray(offs, dtype=np.int32)
 
 
+def _as_tensor(name, a):
+    if isinstance(a, np.ndarray):
+        return torch.from_numpy(a)
+    if torch.is_tensor(a):
+        return a
+    raise ValueError("schedule %s must be a numpy array or a torch tensor, got %r" % (name, type(a)))
+
+
+def pack_schedule(schedule, nsteps, batch):
+    """A source schedule (xy, radius, intensity) -> (int32 records [T * B * E, 4] in the smk_source_t layout with the intensity
+    bits in column 3, E), or (None, 0) when E == 0.
+
+    xy: integer [T, B, E, 2] (column x, row y); radius: integer [T, B, E]; intensity: float32 [T, B, E]; numpy arrays, CPU
+    tensors or tensors on one CUDA device (the records are built where the inputs are).  Entry (t, b, e) is emitter e of
+    simulation b at the head of step t; an entry with radius < 0 adds nothing, which pads lists of different lengths to E.
+    The records are step-major, so the offsets of row (t, b) are arange(T * B + 1) * E (schedule_offsets).  Integer values
+    must fit int32.  ValueError for anything else, before any work; T must be nsteps and B the batch."""
+    if not isinstance(schedule, (tuple, list)) or len(schedule) != 3:
+        raise ValueError("a schedule is a tuple (xy, radius, intensity)")
+    xy, radius, inten = (_as_tensor(n, a) for n, a in zip(("xy", "radius", "intensity"), schedule))
+    if xy.dim() != 4 or xy.shape[3] != 2:
+        raise ValueError("schedule xy must be [T, B, E, 2], got shape %s" % (tuple(xy.shape),))
+    T, B, E = (int(n) for n in xy.shape[:3])
+    for name, t in (("radius", radius), ("intensity", inten)):
+        if tuple(t.shape) != (T, B, E):
+            raise ValueError("schedule %s must be [T, B, E] = %s like xy, got shape %s" % (name, (T, B, E), tuple(t.shape)))
+    for name, t in (("xy", xy), ("radius", radius)):
+        if t.dtype not in (torch.int32, torch.int64):
+            raise ValueError("schedule %s must be int32 or int64, got %s" % (name, t.dtype))
+    if inten.dtype != torch.float32:
+        raise ValueError("schedule intensity must be float32, got %s" % (inten.dtype,))
+    if len({t.device for t in (xy, radius, inten)}) != 1:
+        raise ValueError("schedule xy, radius and intensity must be on one device, got %s"
+                         % sorted({str(t.device) for t in (xy, radius, inten)}))
+    if T != int(nsteps) or B != int(batch):
+        raise ValueError("the schedule has %d steps of %d simulations; the call has %d steps of %d" % (T, B, nsteps, batch))
+    if T * B * E > 0x7fffffff or T * B + 1 > 0x7fffffff:
+        raise ValueError("a schedule of %d x %d x %d emitters does not fit int32 offsets" % (T, B, E))
+    if xy.device.type == "cpu" and E:
+        for name, t in (("xy", xy), ("radius", radius)):
+            if t.dtype == torch.int64 and (int(t.min()) < -0x80000000 or int(t.max()) > 0x7fffffff):
+                raise ValueError("schedule %s values must fit int32" % name)
+    if E == 0:
+        return None, 0
+    rec = torch.empty(T * B * E, 4, dtype=torch.int32, device=xy.device)
+    rec[:, 0:2] = xy.reshape(-1, 2)
+    rec[:, 2] = radius.reshape(-1)
+    rec[:, 3] = inten.reshape(-1).contiguous().view(torch.int32)
+    return rec, E
+
+
+def schedule_offsets(nsteps, batch, E, device):
+    """Offsets of a packed schedule: int32 [nsteps * batch + 1], row (t, b) = records [(t * batch + b) * E, (t * batch + b + 1) * E).
+    Step-major, so the steps t0 .. of a chunk read offsets[t0 * batch:] with the same records."""
+    return torch.arange(0, (nsteps * batch + 1) * E, E, dtype=torch.int32, device=device)
+
+
 class FieldLayout:
     """Where each field lives inside the single fp32 arena (pure host arithmetic, testable without a GPU).
 
@@ -327,17 +384,41 @@ class NavierStokesSimulator(nn.Module):
             # one cached pinned staging buffer (cudaHostAlloc per call costs more than the copy); the previous
             # call's H2D copy has long been consumed by the splat that followed it on the same stream
             need = src_h.numel() + 4 * off_h.numel()
-            stage = getattr(self, "_pinned_sources", None)
-            if stage is None or stage.numel() < need:
-                stage = torch.empty(max(need, 4096), dtype=torch.uint8).pin_memory()
-                self._pinned_sources = stage
-            else:
-                torch.cuda.current_stream(self._cuda).synchronize()
+            stage = self._pinned_stage("_pinned_sources", need)
             stage[:src_h.numel()].copy_(src_h)
             stage[src_h.numel():need].view(torch.int32).copy_(off_h)
             dev = stage[:need].to(self._cuda, non_blocking=True)
             return dev[:src_h.numel()], dev[src_h.numel():need].view(torch.int32), need
         return src_h.to(self._cuda), off_h.to(self._cuda), src_h.numel() + 4 * off_h.numel()
+
+    def _pinned_stage(self, attr, need):
+        """The cached pinned staging buffer `attr`, of at least `need` bytes (cudaHostAlloc per call costs more than the copy);
+        the previous call's H2D copy has long been consumed by the launch that followed it on the same stream."""
+        stage = getattr(self, attr, None)
+        if stage is None or stage.numel() < need:
+            stage = torch.empty(max(need, 4096), dtype=torch.uint8).pin_memory()
+            setattr(self, attr, stage)
+        else:
+            torch.cuda.current_stream(self._cuda).synchronize()
+        return stage
+
+    def upload_schedule(self, schedule, nsteps, pin=False):
+        """Pack a source schedule (pack_schedule) and put it on this simulator's device: (int32 records [T * B * E, 4], int32
+        offsets [T * B + 1]), or None when it has no entries (E == 0).  Host inputs travel as one H2D copy of 16 B per entry,
+        through pinned memory when pin; the offsets are built on the device."""
+        rec, E = pack_schedule(schedule, nsteps, self.batch)
+        if rec is None:
+            return None
+        if rec.device.type == "cpu":
+            if pin:
+                stage = self._pinned_stage("_pinned_schedule", rec.numel() * 4)
+                stage[:rec.numel() * 4].view(torch.int32).view(rec.shape).copy_(rec)
+                rec = stage[:rec.numel() * 4].to(self._cuda, non_blocking=True).view(torch.int32).view(rec.shape)
+            else:
+                rec = rec.to(self._cuda)
+        elif rec.device != self._cuda:
+            raise ValueError("the schedule is on %s; this simulator runs on %s" % (rec.device, self._cuda))
+        return rec, schedule_offsets(int(nsteps), self.batch, E, self._cuda)
 
     def splat_uploaded(self, src, off):
         if self._pending == []:                         # right after a reset: the fused launch that consumes it splats
@@ -471,22 +552,29 @@ class NavierStokesSimulator(nn.Module):
             return None
         return tuple(t.data_ptr() for t in self._pending[0]) if self._pending else (None, None)
 
-    def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt):
+    def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt, sched=None):
         """nsteps steps of the state, frames (a device pointer or None) at the given strides in elements of frame format fmt.
 
-        One smk_run_steps_src_ex call, with the continuous sources if any.  A pending reset is offered to it first (reset = 1,
-        on the current stream without materializing anything); when the call does not consume it (not on k_step_fused),
-        nothing was enqueued, and the reset is applied eagerly before the call is made again without it."""
+        One smk_run_steps_sched_ex call, with the continuous sources if any (offsets step stride 0) or the schedule `sched`:
+        (device records, device offsets, t0), this call's step t reading the schedule's row t0 + t (offsets step stride batch).
+        A pending reset is offered to it first (reset = 1, on the current stream without materializing anything); when the call
+        does not consume it (not on k_step_fused), nothing was enqueued, and the reset is applied eagerly before the call is made
+        again without it."""
         if nsteps == 0:
             return                                      # (a negative count goes on to the library, which refuses it)
-        src, off = (self._csrc[1].data_ptr(), self._csrc[2].data_ptr()) if self._csrc is not None else (None, None)
+        if sched is not None:
+            src, off, stride = sched[0].data_ptr(), sched[1].data_ptr() + 4 * sched[2] * self.batch, self.batch
+        elif self._csrc is not None:
+            src, off, stride = self._csrc[1].data_ptr(), self._csrc[2].data_ptr(), 0
+        else:
+            src, off, stride = None, None, 0
         fm = fmul.data_ptr() if fmul is not None else None
         done = C.c_int32(0)
         offer = self._offer_reset()
         for reset in ((True, False) if offer is not None else (False,)):
             rsrc, roff = offer if reset else (None, None)
-            _lib.call("smk_run_steps_src_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                      frames, step_stride, batch_stride, fm, fmt, src, off, int(reset), rsrc, roff, C.byref(done),
+            _lib.call("smk_run_steps_sched_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, step_stride, batch_stride, fm, fmt, src, off, stride, int(reset), rsrc, roff, C.byref(done),
                       _lib.stream_on(self._cuda) if reset else self._stream())
             if done.value:
                 self._pending = None
@@ -513,12 +601,31 @@ class NavierStokesSimulator(nn.Module):
         fmt = self._check_frame_buffer("frame", frame, (L.batch, L.h, L.pitch_c))
         self._steps(1, frame.data_ptr(), 0, L.h * L.pitch_c, fmul, fmt)
 
-    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None):
+    def _schedule(self, schedule, nsteps):
+        """_steps' schedule argument for a run_steps* schedule, None for none; ValueError before any work."""
+        if schedule is None:
+            return None
+        if self._csrc is not None:
+            raise ValueError("a source schedule and continuous sources do not combine: fold the constant emitters into the "
+                             "schedule (or set_continuous_sources(None))")
+        up = self.upload_schedule(schedule, nsteps)
+        return None if up is None else up + (0,)
+
+    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None, schedule=None):
         """nsteps consecutive steps enqueued back to back; returns frames [batch, nsteps, h, w] ([nsteps, h, w] if batch == 1).
 
         out: optional preallocated [batch, nsteps, h, pitch_c] device buffer to write the frames into (float32, float16 or
         bfloat16).  frame_dtype: the frames' dtype (default float32; with `out`, out.dtype, and a different frame_dtype is
-        an error); half-precision frames are the fp32 ones rounded once to nearest even, as in step()."""
+        an error); half-precision frames are the fp32 ones rounded once to nearest even, as in step().
+
+        schedule = (xy, radius, intensity): emitters that move or change intensity from step to step (pack_schedule gives the
+        format; T = nsteps, B = batch).  Row t is added to the density at the head of step t, before the buoyancy, exactly as
+        add_sources of that row followed by step() would add it -- bit for bit, frames and state, in one launch on the fused
+        and cluster kernels.  Frame t is the density after step t; the state left carries no trailing splat.  A schedule does
+        not combine with continuous sources (ValueError)."""
+        return self._run_steps(nsteps, fmul, return_frames, out, frame_dtype, self._schedule(schedule, nsteps))
+
+    def _run_steps(self, nsteps, fmul, return_frames, out, frame_dtype, sched):
         L = self._layout
         if out is not None:
             fmt = self._check_frame_buffer("out", out, (L.batch, nsteps, L.h, L.pitch_c))
@@ -529,15 +636,20 @@ class NavierStokesSimulator(nn.Module):
             frame_dtype = torch.float32 if frame_dtype is None else frame_dtype
             fmt = _lib.frame_format(frame_dtype)
             fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
-        self._steps(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt)
+        self._steps(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt,
+                    sched)
         return self._finish_frames(fr) if fr is not None else None
 
-    def run_steps_time_major(self, nsteps, out, fmul=None):
+    def run_steps_time_major(self, nsteps, out, fmul=None, *, schedule=None):
         """nsteps consecutive steps whose frames go to `out`, a contiguous [nsteps, batch, h, pitch_c] float32, float16 or
-        bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block)."""
+        bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block).
+        schedule: as run_steps."""
+        self._run_steps_time_major(nsteps, out, fmul, self._schedule(schedule, nsteps))
+
+    def _run_steps_time_major(self, nsteps, out, fmul, sched):
         L = self._layout
         fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
-        self._steps(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt)
+        self._steps(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt, sched)
 
     def divergence_norms(self):
         """(max|div|, ||div||_2) of the un-normalised divergence of the live (u, v), per simulation: [batch, 2] on the host."""
@@ -562,8 +674,10 @@ class NavierStokesSimulator(nn.Module):
 
 
 # every method that launches runs with the simulator's device current and restores the caller's afterwards
-for _name in ("setup_grid", "_materialize", "add_sources", "set_continuous_sources", "splat_uploaded", "upload_sources", "diffusion_step", "advection_step", "_bilerp",
-              "pressure_projection", "step", "step_into", "run_steps", "run_steps_time_major", "divergence_norms",
+for _name in ("setup_grid", "_materialize", "add_sources", "set_continuous_sources", "splat_uploaded", "upload_sources",
+              "upload_schedule", "diffusion_step", "advection_step", "_bilerp",
+              "pressure_projection", "step", "step_into", "run_steps", "_run_steps", "run_steps_time_major", "_run_steps_time_major",
+              "divergence_norms",
               "jacobi_residual_norms", "step_is_fused"):
     setattr(NavierStokesSimulator, _name, _lib.scoped(getattr(NavierStokesSimulator, _name)))
 del _name
