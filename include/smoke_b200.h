@@ -180,7 +180,7 @@ SMK_API int smk_advect_slab(const smk_grid_t* g, const float* field, float* out,
  *     [batch][nsteps][h][pitch_c] returned copies, multiplied by (1+fmul) when fmul != NULL.
  *     Not available on a slab grid (the host interleaves halo exchanges between the phases).
  *     Every step entry point (smk_step, smk_step_ex, smk_run_steps, smk_run_steps_ex, smk_run_steps_reset_ex,
- *     smk_run_steps_src_ex, smk_run_steps_sched_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
+ *     smk_run_steps_src_ex, smk_run_steps_sched_ex, smk_run_steps_force_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
  *     jacobi_iters, dt, step_kernel -- and refuses a malformed one before anything is enqueued. */
 SMK_API int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
              float* frame, int64_t frame_stride, const float* fmul, void* stream);
@@ -237,6 +237,26 @@ SMK_API int smk_run_steps_sched_ex(const smk_grid_t* g, smk_state_t* st, const s
                                    const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
                                    int32_t offsets_step_stride, int32_t reset, const smk_source_t* reset_sources,
                                    const int32_t* reset_offsets, int32_t* consumed_host, void* stream);
+/*     smk_run_steps_sched_ex with velocity forcing: increments (du, dv) added to u and v at the head of every step, after that
+ *     step's emitters and before the buoyancy -- one rounded fp32 add per cell, u's row h and v's column w included -- exactly as
+ *     `u += du; v += dv` on the live fields followed by smk_step_ex would add them (bit-identical frames and state, same frame,
+ *     emitter and reset contract as smk_run_steps_sched_ex).  force_u / force_v have the grid's pitches and per-simulation strides
+ *     (stride_u / stride_v), 16-byte aligned; step t (0 .. nsteps - 1 of this call) of simulation b reads
+ *     force_u + t * (force_per_step ? batch * stride_u : 0) + b * stride_u, and force_v likewise.  Only the cells inside each
+ *     field are read.  On k_step_fused and k_step_cluster the add is done on chip (no extra launch); on the phase kernels one
+ *     smk_add_forcing launch precedes each step.  The buffers are read during the launch and must stay valid until it completes.
+ *     Both NULL (force_per_step = 0): no forcing, which is smk_run_steps_sched_ex.  Unpaired or misaligned buffers, or a
+ *     force_per_step other than 0 and 1 or set without forcing, is SMK_EINVAL before anything is enqueued. */
+SMK_API int smk_run_steps_force_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                                   void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                                   const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
+                                   int32_t offsets_step_stride, const float* force_u, const float* force_v, int32_t force_per_step,
+                                   int32_t reset, const smk_source_t* reset_sources, const int32_t* reset_offsets,
+                                   int32_t* consumed_host, void* stream);
+/*     u = u + du, v = v + dv over the batch, the cells inside u [h+1][w] and v [h][w+1] only (pads are neither read nor
+ *     written); du / dv have the layout of u / v.  The forcing add of one step on the phase kernels; reverse mode also uses it
+ *     to accumulate gradients. */
+SMK_API int smk_add_forcing(const smk_grid_t* g, float* u, float* v, const float* du, const float* dv, void* stream);
 /*     1 when a call of nsteps steps (smk_step: 1) would take the fused single-launch path for this grid and params */
 SMK_API int smk_step_is_fused(const smk_grid_t* g, const smk_params_t* prm, int32_t nsteps, int32_t* fused_host);
 /* Host-only (no GPU needed): the time-sliced schedule smk_run_steps gives the fused kernel when `nsims` simulations of

@@ -96,6 +96,9 @@ SIGNATURES = {
     "smk_run_steps_src_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p, c_p, c_i32, c_p, c_p, C.POINTER(c_i32), c_p],
     "smk_run_steps_sched_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p, c_p, c_i32, c_i32, c_p, c_p, C.POINTER(c_i32),
                                c_p],
+    "smk_run_steps_force_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p, c_p, c_i32, c_p, c_p, c_i32, c_i32, c_p, c_p,
+                               C.POINTER(c_i32), c_p],
+    "smk_add_forcing": [GP, c_p, c_p, c_p, c_p, c_p],
     "smk_step_is_fused": [GP, PP, c_i32, C.POINTER(c_i32)],
     "smk_fused_plan": [c_i32, c_i32, c_i32, C.POINTER(c_i32), c_i32, C.POINTER(c_i32)],
     "smk_div_norms": [GP, c_p, c_p, c_p, c_p],

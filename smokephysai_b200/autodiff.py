@@ -4,6 +4,7 @@
     d0 = autodiff.add_sources(d0, emitters, intensities)       # emitters[b] = [(x, y, radius), ...]
     frames, state = autodiff.rollout(state, nsteps, sources=emitters, intensities=intensities)   # emitters at every step
     frames, state = autodiff.rollout(state, nsteps, schedule=(xy, radius), intensities=I)       # an emission history, I [T, B, E]
+    frames, state = autodiff.rollout(state, nsteps, forcing=(du, dv))                           # velocity forcing, constant or per step
 
 The reference simulator is eager PyTorch, so autograd runs through it: a user can fit emitter intensities to observed frames,
 optimise an initial state or train a model through the simulator.  This module gives the same capability on the CUDA path.
@@ -31,6 +32,12 @@ Source schedules (rollout(..., schedule=(xy, radius), intensities=I)): row t of 
 NavierStokesSimulator.run_steps(schedule=) does, and the forward is that call bit for bit.  The backward splats a copy of S_t.d with
 row t, and the gradient of step t's intensities is the splat adjoint of that step alone (smk_splat_sources_adjoint_ex on row t's
 records, not accumulating), so I.grad[t] is exactly that of step t and padded entries (radius < 0) get exactly 0.
+
+Velocity forcing (rollout(..., forcing=(du, dv))): du_t, dv_t are added to u and v at the head of step t, after the emitters, as
+NavierStokesSimulator.run_steps(forcing=) does, and the forward is that call bit for bit.  Checkpoints stay the pre-forcing S_t; the
+recompute adds row t to copies of S_t.u and S_t.v (smk_add_forcing).  The add passes the gradient unchanged, so after reverse step t
+G.u / G.v is the gradient of u / v at the head of step t: that of S_t and of du_t / dv_t alike.  A per-step forcing's gradient row t
+is that value; a constant forcing's is the sum over steps, accumulated with smk_add_forcing for t = T-1 down to 0 in that order.
 """
 import ctypes as C
 
@@ -38,7 +45,7 @@ import torch
 
 from . import _lib
 from .fractal_generator import FractalGenerator
-from .navier_stokes import FieldLayout, NavierStokesSimulator, pack_schedule, schedule_offsets
+from .navier_stokes import FieldLayout, NavierStokesSimulator, pack_forcing, pack_schedule, schedule_offsets
 
 __all__ = ["rollout", "add_sources"]
 
@@ -97,6 +104,7 @@ class _Config:
         self.B = 1 if batch is None else batch
         self.src = None                 # continuous sources: (int32 [n, 4] device records with the intensities, offsets, n)
         self.sched = None               # schedule: (int32 [T * B * E, 4] device records with the intensities, offsets [T * B + 1], E)
+        self.force = None               # forcing: (du, dv, per_step) of pack_forcing, padded [(T | 1), B, rows, pitch] device buffers
 
     def simulator(self, state):
         sim = NavierStokesSimulator((self.h, self.w), self.dt, self.viscosity, self.device, jacobi_iters=self.jacobi_iters,
@@ -114,6 +122,10 @@ class _Config:
         if self.sched is None:
             return None
         return self.sched[:2] + (t0,)
+
+    def step_force(self, t0):
+        """_steps' force argument for a call whose step 0 is step t0 of the rollout (None without forcing)."""
+        return None if self.force is None else self.force + (t0,)
 
     def fmul(self):
         if not self.add_fractal:
@@ -153,7 +165,7 @@ def _ptr(t):
 
 class _Rollout(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, cfg, u0, v0, p0, d0, intensities):
+    def forward(ctx, cfg, u0, v0, p0, d0, intensities, du, dv):
         with _lib.on_device(cfg.device):
             sim = cfg.simulator((u0, v0, p0, d0))
             L = sim._layout
@@ -166,10 +178,12 @@ class _Rollout(torch.autograd.Function):
             fmul = cfg.fmul()
             prm = sim._params()
             for t in range(T):
-                sim._steps(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0, cfg.step_sched(t))
+                sim._steps(1, frames.data_ptr() + 4 * t * L.h * L.pitch_c, 0, T * L.h * L.pitch_c, fmul, 0, cfg.step_sched(t),
+                           cfg.step_force(t))
                 for k in _FIELDS:
                     ck[k][t + 1].copy_(_arena_view(sim, k))
             ctx.cfg, ctx.ck, ctx.fmul, ctx.layout, ctx.params = cfg, ck, fmul, L, prm
+            ctx.fshapes = (du.shape, dv.shape) if du is not None else None
             out = [cfg.shape_out(frames[..., :L.w].contiguous())]
             for k in _FIELDS:
                 rows, cols, _ = L.shape_of(_layout_name(k))
@@ -182,7 +196,9 @@ class _Rollout(torch.autograd.Function):
         cfg, ck, L, prm = ctx.cfg, ctx.ck, ctx.layout, ctx.params
         with _lib.on_device(cfg.device):
             grads = _reverse(cfg, ck, L, prm, ctx.fmul, g_frames, {"u": g_u, "v": g_v, "p": g_p, "d": g_d})
-        return (None,) + grads[:4] + (grads[4] if ctx.needs_input_grad[5] else None,)
+        if ctx.fshapes is not None:
+            grads = grads[:5] + tuple(g.reshape(shape) for g, shape in zip(grads[5:], ctx.fshapes))
+        return (None,) + grads[:4] + tuple(g if ctx.needs_input_grad[k] else None for k, g in zip((5, 6, 7), grads[4:]))
 
 
 def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
@@ -217,12 +233,23 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         g_int = torch.zeros(T, B, E, dtype=torch.float32, device=dev)
         row_off = schedule_offsets(1, B, E, dev)                # one row of B lists of E entries, for the per-step adjoint
         dsp = zeros("d")
+    g_force = None
+    if cfg.force is not None:
+        fu, fv, per_step = cfg.force
+        g_force = (torch.zeros_like(fu), torch.zeros_like(fv))     # [T or 1, B, rows, pitch]: row t, or the sum over the steps
+        uf, vf = zeros("u"), zeros("v")                             # S_t.u, S_t.v with the step's forcing
     for t in range(T - 1, -1, -1):
         u0, v0, d0 = ck["u"][t], ck["v"][t], ck["d"][t]
         if g_int is not None:
             dsp.copy_(d0)
             _lib.call("smk_splat_sources", gp, dsp.data_ptr(), rec.data_ptr(), off.data_ptr() + (4 * t * B if cfg.sched else 0), s)
             d0 = dsp
+        if g_force is not None:
+            uf.copy_(u0)
+            vf.copy_(v0)
+            r = t if per_step else 0
+            _lib.call("smk_add_forcing", gp, uf.data_ptr(), vf.data_ptr(), fu[r].data_ptr(), fv[r].data_ptr(), s)
+            u0, v0 = uf, vf
         u1, v1, p1 = ck["u"][t + 1], ck["v"][t + 1], ck["p"][t + 1]
         # recompute: buoyancy + diffusions, then the gradient subtract with the pressure the step projected with
         _lib.call("smk_forces_diffuse_div", gp, u0.data_ptr(), v0.data_ptr(), d0.data_ptr(), ud.data_ptr(), vd.data_ptr(),
@@ -254,15 +281,26 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         elif cfg.sched is not None:
             _lib.call("smk_splat_sources_adjoint_ex", gp, G["d"].data_ptr(), rec.data_ptr() + 16 * t * B * E, row_off.data_ptr(),
                       B * E, 0, g_int[t].data_ptr(), s)
+        # G.u / G.v: the gradients of the forced u / v, which are also those of S_t.u / S_t.v and of the step's forcing
+        if g_force is not None:
+            if per_step:
+                g_force[0][t].copy_(G["u"])
+                g_force[1][t].copy_(G["v"])
+            else:
+                _lib.call("smk_add_forcing", gp, g_force[0][0].data_ptr(), g_force[1][0].data_ptr(), G["u"].data_ptr(),
+                          G["v"].data_ptr(), s)
     out = []
     for k in _FIELDS:
         rows, cols, _ = L.shape_of(_layout_name(k))
         out.append(cfg.shape_out(G[k][:, :, :cols].contiguous()))
-    return tuple(out) + (g_int,)
+    g_du = g_dv = None
+    if g_force is not None:
+        g_du, g_dv = (g[..., :c].contiguous() for g, c in zip(g_force, (L.w, L.w + 1)))
+    return tuple(out) + (g_int, g_du, g_dv)
 
 
 def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fractal=False, step_kernel="auto",
-            sweeps_per_launch=0, sources=None, intensities=None, schedule=None):
+            sweeps_per_launch=0, sources=None, intensities=None, schedule=None, forcing=None):
     """nsteps steps of NavierStokesSimulator from state = (u, v, p, d); differentiable with respect to all four fields.
 
     u [.., h+1, w], v [.., h, w+1], p [.., h, w], d [.., h, w]: float32 CUDA tensors on one device, with an optional leading
@@ -277,7 +315,11 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
 
     schedule = (xy, radius) / intensities: an emission history, row t added at the head of step t (run_steps(schedule=)).
     xy integer [T, B, E, 2], radius integer [T, B, E] (B = 1 for 2-D inputs; radius < 0 pads), intensities float32 [T, B, E]
-    on the state's device, differentiable.  Exclusive with sources=."""
+    on the state's device, differentiable.  Exclusive with sources=.
+
+    forcing = (du, dv): velocity increments added at the head of every step (run_steps(forcing=)), float32 tensors on the state's
+    device: du [.., h+1, w] and dv [.., h, w+1] in the state's shapes for a constant forcing, or with a leading T = nsteps axis for
+    a per-step one; differentiable with respect to du and dv.  It combines with sources= and schedule=."""
     batch, h, w, device = _check_state(state)
     if int(nsteps) < 1:
         raise ValueError("nsteps must be >= 1, got %r" % (nsteps,))
@@ -301,13 +343,19 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
         if n:
             rec.view(torch.float32)[:n, 3].copy_(intensities.detach())           # smk_source_t.intensity
             cfg.src = (rec, off, n)
+    du = dv = None
+    if forcing is not None:
+        du, dv = _check_forcing(forcing, batch is None, device)
+        cfg.force = pack_forcing((du, dv) if batch is not None else (du.unsqueeze(-3), dv.unsqueeze(-3)), cfg.nsteps, cfg.B, h, w,
+                                 device)
     differentiable = cfg.src is not None or cfg.sched is not None
-    if torch.is_grad_enabled() and (any(t.requires_grad for t in state) or (differentiable and intensities.requires_grad)):
-        frames, *final = _Rollout.apply(cfg, *state, intensities if differentiable else None)
+    wants = list(state) + ([intensities] if differentiable else []) + ([du, dv] if du is not None else [])
+    if torch.is_grad_enabled() and any(t.requires_grad for t in wants):
+        frames, *final = _Rollout.apply(cfg, *state, intensities if differentiable else None, du, dv)
         return frames, tuple(final)
     with _lib.on_device(device):
         sim = cfg.simulator(state)
-        frames = sim._run_steps(cfg.nsteps, cfg.fmul(), True, None, None, cfg.step_sched(0))
+        frames = sim._run_steps(cfg.nsteps, cfg.fmul(), True, None, None, cfg.step_sched(0), cfg.step_force(0))
         if batch is not None and cfg.B == 1:
             frames = frames.unsqueeze(0)
         final = []
@@ -352,6 +400,20 @@ def _schedule_records(schedule, intensities, T, B, device):
     rec = rec.to(device)
     rec[:, 3] = intensities.detach().reshape(-1).view(torch.int32)           # smk_source_t.intensity bits
     return rec, schedule_offsets(T, B, E, device), E
+
+
+def _check_forcing(forcing, two_d, device):
+    """rollout's forcing -> (du, dv) as given; ValueError unless they are float32 tensors on the state's device (pack_forcing checks
+    the shapes)."""
+    if not isinstance(forcing, (tuple, list)) or len(forcing) != 2:
+        raise ValueError("a forcing is a pair (du, dv)")
+    for name, t in zip(("du", "dv"), forcing):
+        if not torch.is_tensor(t) or t.dtype != torch.float32 or t.device != device:
+            raise ValueError("forcing %s must be a float32 tensor on %s" % (name, device))
+        if t.dim() not in ((2, 3) if two_d else (3, 4)):
+            raise ValueError("forcing %s must be %s, got shape %s" % (
+                name, "[rows, cols] or [T, rows, cols]" if two_d else "[B, rows, cols] or [T, B, rows, cols]", tuple(t.shape)))
+    return tuple(forcing)
 
 
 def _emitter_lists(emitters, two_d):

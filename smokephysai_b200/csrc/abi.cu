@@ -391,6 +391,10 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
         return fail(SMK_EINVAL, "%s: offsets_step_stride must be 0 or the batch (%d) with sources, got %d", who, g->batch, c.cstride);
     if ((c.rsrc == nullptr) != (c.roff == nullptr)) return fail(SMK_EINVAL, "%s: reset_sources and reset_offsets go together", who);
     if (!c.reset && c.rsrc) return fail(SMK_EINVAL, "%s: reset_sources without a reset", who);
+    if ((c.fu == nullptr) != (c.fv == nullptr)) return fail(SMK_EINVAL, "%s: force_u and force_v go together", who);
+    if ((c.fu && !aligned16(c.fu)) || (c.fv && !aligned16(c.fv))) return fail(SMK_EINVAL, "%s: force_u / force_v not 16-byte aligned", who);
+    if (c.fstep != 0 && c.fstep != 1) return fail(SMK_EINVAL, "%s: force_per_step must be 0 or 1, got %d", who, c.fstep);
+    if (c.fstep && !c.fu) return fail(SMK_EINVAL, "%s: force_per_step = 1 without forcing", who);
     SMK_TRY(check_grid(g, who));
     if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
         return fail(SMK_EUNSUPPORTED, "%s: slab grids are stepped phase by phase with halo exchanges in between", who);
@@ -407,8 +411,11 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
         return SMK_OK;
     }
     const int64_t step_bytes = c.frame_step_stride * frame_elem_size(c.frame_format);
+    const int64_t fu_step = c.fstep ? (int64_t)g->batch * g->stride_u : 0, fv_step = c.fstep ? (int64_t)g->batch * g->stride_v : 0;
     for (int t = 0; t < c.nsteps; ++t)
-        SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff ? c.coff + (int64_t)t * c.cstride : nullptr, c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
+        SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff ? c.coff + (int64_t)t * c.cstride : nullptr,
+                           c.fu ? c.fu + t * fu_step : nullptr, c.fv ? c.fv + t * fv_step : nullptr,
+                           c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
                            c.frame_batch_stride, c.fmul, c.frame_format, nullptr, nullptr, nullptr, nullptr, s));
     return SMK_OK;
 }
@@ -470,7 +477,18 @@ int smk_run_steps_sched_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
                            const smk_source_t* sources, const int32_t* offsets, int32_t offsets_step_stride, int32_t reset,
                            const smk_source_t* reset_sources, const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
 {
-    const char* who = "smk_run_steps_sched_ex";
+    return smk_run_steps_force_ex(g, st, prm, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, frame_format, sources,
+                                  offsets, offsets_step_stride, nullptr, nullptr, 0, reset, reset_sources, reset_offsets,
+                                  consumed_host, stream);
+}
+
+int smk_run_steps_force_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                           int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format,
+                           const smk_source_t* sources, const int32_t* offsets, int32_t offsets_step_stride,
+                           const float* force_u, const float* force_v, int32_t force_per_step, int32_t reset,
+                           const smk_source_t* reset_sources, const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
+{
+    const char* who = "smk_run_steps_force_ex";
     if (!consumed_host) return fail(SMK_EINVAL, "%s: consumed_host is NULL", who);
     *consumed_host = 0;
     if (reset != 0 && reset != 1) return fail(SMK_EINVAL, "%s: reset must be 0 or 1, got %d", who, reset);
@@ -478,8 +496,16 @@ int smk_run_steps_sched_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
     StepCall c;
     c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
     c.fmul = fmul; c.frame_format = frame_format; c.csrc = sources; c.coff = offsets; c.cstride = offsets_step_stride;
+    c.fu = force_u; c.fv = force_v; c.fstep = force_per_step;
     c.reset = reset == 1; c.rsrc = reset_sources; c.roff = reset_offsets;
     return run_steps(who, g, st, prm, c, consumed_host, (cudaStream_t)stream);
+}
+
+int smk_add_forcing(const smk_grid_t* g, float* u, float* v, const float* du, const float* dv, void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_add_forcing"));
+    SMK_TRY(check_ptrs("smk_add_forcing", {u, v, du, dv}));
+    return launch_add_forcing(g, u, v, du, dv, (cudaStream_t)stream);
 }
 
 int smk_div_norms(const smk_grid_t* g, const float* u, const float* v, float* out, void* stream)

@@ -164,6 +164,7 @@ int check_grid(const smk_grid_t* g, const char* who);
 
 // launchers (one per kernel family); all asynchronous on `s`
 int launch_splat(const smk_grid_t* g, float* density, const smk_source_t* src, const int32_t* off, cudaStream_t s);
+int launch_add_forcing(const smk_grid_t* g, float* u, float* v, const float* du, const float* dv, cudaStream_t s);
 int launch_diffuse(const float* in, float* out, int rows, int cols, int pitch, int batch, int64_t stride, float c, cudaStream_t s);
 int launch_forces_diffuse_div(const smk_grid_t* g, const float* u, const float* v, const float* d,
                               float* uo, float* vo, float* dout, float* div, float dt, float c_uv, float c_d, cudaStream_t s);
@@ -208,16 +209,20 @@ struct StepCall {
     const smk_source_t* csrc = nullptr;       // emitters splatted at the head of every step (NULL: none); step t of simulation b
     const int32_t* coff = nullptr;            //   adds records [coff[t * cstride + b], coff[t * cstride + b + 1])
     int cstride = 0;                          // 0: one list for every step (continuous sources); batch: a schedule, a row per step
+    const float* fu = nullptr;                // velocity forcing added to u / v at the head of every step (NULL: none), in the
+    const float* fv = nullptr;                //   grid's layout; step t of simulation b adds fu + t * (fstep ? batch * stride_u : 0)
+    int fstep = 0;                            //   + b * stride_u (v likewise).  0: one pair for every step; 1: a pair per step
     bool reset = false;                       // start from a reset state splatted once with (rsrc, roff): k_step_fused only
     const smk_source_t* rsrc = nullptr;
     const int32_t* roff = nullptr;
 };
 int launch_steps_fused(const smk_grid_t* g, const smk_state_t* st, const smk_params_t* prm, const StepCall& c, cudaStream_t s);
 // One step on the phase kernels (peer_halo.cu), for a whole grid or a row slab whose ghost rows are current: the continuous
-// emitters (csrc / coff), buoyancy + diffusion + divergence, the Jacobi sweeps, the gradient subtract and the three advections.
-// All per-call inputs may be NULL: the frame (whole grids), the reach guards chk_* and the comm of the tail push (slabs).
+// emitters (csrc / coff), the velocity forcing (fu / fv, this step's pair), buoyancy + diffusion + divergence, the Jacobi sweeps,
+// the gradient subtract and the three advections.  All per-call inputs may be NULL: the emitters, the forcing, the frame (whole
+// grids), the reach guards chk_* and the comm of the tail push (slabs).
 int phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
-               void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+               const float* fu, const float* fv, void* frame, int64_t frame_stride, const float* fmul, int frame_format,
                const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
                const smk_peer_comm_t* push_comm, cudaStream_t s);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);

@@ -289,11 +289,12 @@ static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params
 }
 
 int smk::phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
-                    void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+                    const float* fu, const float* fv, void* frame, int64_t frame_stride, const float* fmul, int frame_format,
                     const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
                     const smk_peer_comm_t* push_comm, cudaStream_t s)
 {
     if (csrc) SMK_TRY_(launch_splat(g, st->d[st->cur_d], csrc, coff, s));     // add_smoke_source, then the step (bit-equal by construction)
+    if (fu) SMK_TRY_(launch_add_forcing(g, st->u[st->cur_u], st->v[st->cur_v], fu, fv, s));      // u += du; v += dv, then the step
     const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
     // 1-2. buoyancy + diffusion + divergence                                   navier_stokes.py:154-160, :136
     SMK_TRY_(launch_forces_diffuse_div(g, st->u[cu], st->v[cv], st->d[cd], st->u[cu ^ 1], st->v[cv ^ 1], st->d[cd ^ 1], st->div,
@@ -396,7 +397,7 @@ int smk_slab_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
         SMK_TRY(peer_xfer(comm, base, false, s));
     }
     // SMK_SLAB_PUSH_TAIL: the ghost rows of the NEXT step leave from the middle of the density advection
-    return phase_step(g, st, prm, nullptr, nullptr, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d,
+    return phase_step(g, st, prm, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d,
                       (comm && (flags & SMK_SLAB_PUSH_TAIL)) ? comm : nullptr, s);
 }
 

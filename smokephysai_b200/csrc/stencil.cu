@@ -1143,6 +1143,42 @@ int launch_splat(const smk_grid_t* g, float* density, const smk_source_t* src, c
     return check_launch("k_splat");
 }
 
+// ---- velocity forcing: u = u + du, v = v + dv over the batch, one rounded add per cell ------------------------------------
+// The head of a forced step on the phase kernels (after the emitters' splat, before k_forces_diffuse_div), and in reverse mode the
+// accumulation of a constant forcing's gradient.  A thread adds one float4 of a row of u and the same float4 of v; only the cells
+// inside rows x cols are read or written (a row's last group adds its cells one by one), so pads stay as they are.
+__device__ __forceinline__ void add_row4(float* __restrict__ f, const float* __restrict__ df, const int c, const int cols)
+{
+    if (c + 4 <= cols) {
+        float4 x = *reinterpret_cast<const float4*>(f + c);
+        const float4 d = __ldg(reinterpret_cast<const float4*>(df + c));
+        x.x = x.x + d.x; x.y = x.y + d.y; x.z = x.z + d.z; x.w = x.w + d.w;
+        *reinterpret_cast<float4*>(f + c) = x;
+    } else {
+        for (int k = c; k < cols; ++k) f[k] = f[k] + __ldg(df + k);
+    }
+}
+
+__global__ void __launch_bounds__(256)
+k_add_forcing(float* __restrict__ U, float* __restrict__ V, const float* __restrict__ DU, const float* __restrict__ DV,
+              const int h, const int w, const int pu, const int pv, const long long su_, const long long sv_)
+{
+    pdl_prologue();
+    const int c = 4 * (int)(blockIdx.x * 32 + threadIdx.x), i = blockIdx.y * 8 + threadIdx.y;
+    const size_t b = blockIdx.z;
+    if (i <= h && c < w) add_row4(U + b * su_ + (size_t)i * pu, DU + b * su_ + (size_t)i * pu, c, w);
+    if (i < h && c <= w) add_row4(V + b * sv_ + (size_t)i * pv, DV + b * sv_ + (size_t)i * pv, c, w + 1);
+}
+
+int launch_add_forcing(const smk_grid_t* g, float* u, float* v, const float* du, const float* dv, cudaStream_t s)
+{
+    const dim3 grid((g->w + 1 + 127) / 128, (g->h + 1 + 7) / 8, g->batch);
+    ProfScope prof_(SMK_PH_OTHER, s);
+    launch_chain(k_add_forcing, grid, dim3(32, 8), 0, s, u, v, du, dv, g->h, g->w, g->pitch_u, g->pitch_v,
+                 (long long)g->stride_u, (long long)g->stride_v);
+    return check_launch("k_add_forcing");
+}
+
 // ---- divergence norms: per simulation max|div| and sum div^2 (un-normalised u,v differences) -------------
 __global__ void __launch_bounds__(256)
 k_div_norms(const float* __restrict__ U, const float* __restrict__ V, float* __restrict__ out,

@@ -69,12 +69,12 @@ def pack_sources(per_sim):
     return rec, np.asarray(offs, dtype=np.int32)
 
 
-def _as_tensor(name, a):
+def _as_tensor(name, a, what="schedule"):
     if isinstance(a, np.ndarray):
         return torch.from_numpy(a)
     if torch.is_tensor(a):
         return a
-    raise ValueError("schedule %s must be a numpy array or a torch tensor, got %r" % (name, type(a)))
+    raise ValueError("%s %s must be a numpy array or a torch tensor, got %r" % (what, name, type(a)))
 
 
 def pack_schedule(schedule, nsteps, batch):
@@ -124,6 +124,68 @@ def schedule_offsets(nsteps, batch, E, device):
     """Offsets of a packed schedule: int32 [nsteps * batch + 1], row (t, b) = records [(t * batch + b) * E, (t * batch + b + 1) * E).
     Step-major, so the steps t0 .. of a chunk read offsets[t0 * batch:] with the same records."""
     return torch.arange(0, (nsteps * batch + 1) * E, E, dtype=torch.int32, device=device)
+
+
+def pack_forcing(forcing, nsteps, batch, h, w, device, pin=False):
+    """A velocity forcing (du, dv) -> (du, dv) zero-padded float32 device buffers [(T | 1), batch, rows, pitch] in the simulator's
+    layout (FieldLayout: u rows h + 1, v rows h; pitches rounded up to 4), and True for a per-step forcing.
+
+    du [B, h+1, w] and dv [B, h, w+1] (the batch dimension may be dropped when batch == 1): the same increments at every step;
+    with a leading T axis, [T, B, h+1, w] and [T, B, h, w+1]: row t at step t, and T must be nsteps (nsteps=None: only the
+    constant form is accepted).  Numpy arrays, CPU tensors or tensors on `device`, float32; host inputs travel in one copy per
+    field, from pinned memory when pin.  ValueError for anything else, before any work.  The buffers are step-major, so the
+    steps t0 .. of a chunk read from element t0 * batch * (rows * pitch) of the same buffers."""
+    du, dv, T, per_step = check_forcing(forcing, nsteps, batch, h, w, device)
+    out = []
+    for t, rows, cols in ((du, h + 1, w), (dv, h, w + 1)):
+        t = t.detach().reshape(T, batch, rows, cols)
+        if t.device.type == "cpu":
+            buf = torch.zeros(T, batch, rows, _round4(cols), dtype=torch.float32, pin_memory=pin)
+            buf[..., :cols] = t
+            buf = buf.to(device, non_blocking=pin)
+        else:
+            buf = torch.zeros(T, batch, rows, _round4(cols), dtype=torch.float32, device=device)
+            buf[..., :cols] = t
+        out.append(buf)
+    return out[0], out[1], per_step
+
+
+def check_forcing(forcing, nsteps, batch, h, w, device):
+    """pack_forcing's validation alone, no work: -> (du, dv as tensors, T (1 for a constant forcing), per_step); ValueError for
+    anything pack_forcing refuses."""
+    if not isinstance(forcing, (tuple, list)) or len(forcing) != 2:
+        raise ValueError("a forcing is a pair (du, dv)")
+    du, dv = (_as_tensor(n, a, "forcing") for n, a in zip(("du", "dv"), forcing))
+    if du.dim() != dv.dim() or du.dim() not in (2, 3, 4):
+        raise ValueError("forcing du and dv must both be [B, rows, cols] (constant) or [T, B, rows, cols] (per step), got shapes %s, %s"
+                         % (tuple(du.shape), tuple(dv.shape)))
+    per_step = du.dim() == 4
+    if per_step and nsteps is None:
+        raise ValueError("this call takes a constant forcing only: du [B, h+1, w], dv [B, h, w+1]")
+    if du.dim() == 2 and batch != 1:
+        raise ValueError("a forcing without a batch dimension needs batch == 1 (batch is %d)" % batch)
+    T = int(du.shape[0]) if per_step else 1
+    lead = (T, batch) if per_step else (batch,) if du.dim() == 3 else ()
+    for name, t, rc in (("du", du, (h + 1, w)), ("dv", dv, (h, w + 1))):
+        if tuple(t.shape) != lead + rc:
+            raise ValueError("forcing %s must be %s, got %s" % (name, list(lead + rc), list(t.shape)))
+        if t.dtype != torch.float32:
+            raise ValueError("forcing %s must be float32, got %s" % (name, t.dtype))
+        if t.device.type != "cpu" and t.device != device:
+            raise ValueError("forcing %s is on %s; this simulator runs on %s" % (name, t.device, device))
+    if per_step and T != int(nsteps):
+        raise ValueError("the forcing has %d steps; the call has %d" % (T, nsteps))
+    return du, dv, T, per_step
+
+
+def forcing_pointers(force, layout):
+    """(force_u, force_v, force_per_step) of smk_run_steps_force_ex for _steps' force argument (du, dv, per_step, t0) of a call
+    whose step 0 is row t0 of a per-step forcing: the base pointers plus t0 * batch * stride; (None, None, 0) for None."""
+    if force is None:
+        return None, None, 0
+    du, dv, per_step, t0 = force
+    k = int(t0) * layout.batch if per_step else 0
+    return du.data_ptr() + 4 * k * layout.stride_u, dv.data_ptr() + 4 * k * layout.stride_v, int(per_step)
 
 
 class FieldLayout:
@@ -552,11 +614,12 @@ class NavierStokesSimulator(nn.Module):
             return None
         return tuple(t.data_ptr() for t in self._pending[0]) if self._pending else (None, None)
 
-    def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt, sched=None):
+    def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt, sched=None, force=None):
         """nsteps steps of the state, frames (a device pointer or None) at the given strides in elements of frame format fmt.
 
-        One smk_run_steps_sched_ex call, with the continuous sources if any (offsets step stride 0) or the schedule `sched`:
-        (device records, device offsets, t0), this call's step t reading the schedule's row t0 + t (offsets step stride batch).
+        One smk_run_steps_force_ex call, with the continuous sources if any (offsets step stride 0) or the schedule `sched`:
+        (device records, device offsets, t0), this call's step t reading the schedule's row t0 + t (offsets step stride batch);
+        and the forcing `force`: (du, dv, per_step, t0) of pack_forcing, this call's step t reading row t0 + t when per_step.
         A pending reset is offered to it first (reset = 1, on the current stream without materializing anything); when the call
         does not consume it (not on k_step_fused), nothing was enqueued, and the reset is applied eagerly before the call is made
         again without it."""
@@ -568,30 +631,34 @@ class NavierStokesSimulator(nn.Module):
             src, off, stride = self._csrc[1].data_ptr(), self._csrc[2].data_ptr(), 0
         else:
             src, off, stride = None, None, 0
+        fu, fv, per_step = forcing_pointers(force, self._layout)
         fm = fmul.data_ptr() if fmul is not None else None
         done = C.c_int32(0)
         offer = self._offer_reset()
         for reset in ((True, False) if offer is not None else (False,)):
             rsrc, roff = offer if reset else (None, None)
-            _lib.call("smk_run_steps_sched_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                      frames, step_stride, batch_stride, fm, fmt, src, off, stride, int(reset), rsrc, roff, C.byref(done),
-                      _lib.stream_on(self._cuda) if reset else self._stream())
+            _lib.call("smk_run_steps_force_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, step_stride, batch_stride, fm, fmt, src, off, stride, fu, fv, per_step, int(reset), rsrc, roff,
+                      C.byref(done), _lib.stream_on(self._cuda) if reset else self._stream())
             if done.value:
                 self._pending = None
                 self._stale = True
                 return
 
-    def step(self, fmul=None, *, frame_dtype=torch.float32):
+    def step(self, fmul=None, *, frame_dtype=torch.float32, forcing=None):
         """One time step; returns a copy of the new density ([h, w], or [batch, h, w]).
 
         fmul (optional, [h, pitch_c] device tensor) fuses the fractal multiply of SmokeSimulator.simulate_step
         into the returned copy: frame = d + fmul*d (fractal_generator.py:62); solver state is not perturbed.
         frame_dtype torch.float16 / torch.bfloat16 returns that copy rounded once (to nearest even) by the kernel that
         writes it, equal to the fp32 copy's .to(frame_dtype); the state is the same whatever the dtype.
+        forcing = (du, dv), du [batch, h+1, w], dv [batch, h, w+1] (pack_forcing): velocity increments added at the head of the
+        step, as run_steps(1, forcing=) does.
         """
         fmt = _lib.frame_format(frame_dtype)
+        force = self._forcing(forcing, None)
         fr = self._new_frames(dtype=frame_dtype)
-        self._steps(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt)
+        self._steps(1, fr.data_ptr(), 0, self._layout.h * self._layout.pitch_c, fmul, fmt, None, force)
         return self._finish_frames(fr)
 
     def step_into(self, frame, fmul=None):
@@ -611,7 +678,19 @@ class NavierStokesSimulator(nn.Module):
         up = self.upload_schedule(schedule, nsteps)
         return None if up is None else up + (0,)
 
-    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None, schedule=None):
+    def _check_forcing(self, forcing, nsteps):
+        """ValueError for a forcing _forcing would refuse, before any work (None passes)."""
+        if forcing is not None:
+            check_forcing(forcing, nsteps, self.batch, self.h, self.w, self._cuda)
+
+    def _forcing(self, forcing, nsteps, pin=False):
+        """_steps' force argument for a forcing (pack_forcing; nsteps None: constant only), None for none; ValueError before any
+        work."""
+        if forcing is None:
+            return None
+        return pack_forcing(forcing, nsteps, self.batch, self.h, self.w, self._cuda, pin) + (0,)
+
+    def run_steps(self, nsteps, fmul=None, return_frames=True, out=None, *, frame_dtype=None, schedule=None, forcing=None):
         """nsteps consecutive steps enqueued back to back; returns frames [batch, nsteps, h, w] ([nsteps, h, w] if batch == 1).
 
         out: optional preallocated [batch, nsteps, h, pitch_c] device buffer to write the frames into (float32, float16 or
@@ -622,10 +701,18 @@ class NavierStokesSimulator(nn.Module):
         format; T = nsteps, B = batch).  Row t is added to the density at the head of step t, before the buoyancy, exactly as
         add_sources of that row followed by step() would add it -- bit for bit, frames and state, in one launch on the fused
         and cluster kernels.  Frame t is the density after step t; the state left carries no trailing splat.  A schedule does
-        not combine with continuous sources (ValueError)."""
-        return self._run_steps(nsteps, fmul, return_frames, out, frame_dtype, self._schedule(schedule, nsteps))
+        not combine with continuous sources (ValueError).
 
-    def _run_steps(self, nsteps, fmul, return_frames, out, frame_dtype, sched):
+        forcing = (du, dv): velocity increments, du [batch, h+1, w] and dv [batch, h, w+1] at every step, or [nsteps, batch, ...]
+        with row t at step t (pack_forcing gives the format).  At the head of step t, after the emitters and before the buoyancy,
+        u = u + du_t and v = v + dv_t, one rounded fp32 add per cell: the call equals n rounds of `u += du[t]; v += dv[t]; step()`
+        bit for bit, frames and state, in one launch on the fused and cluster kernels.  It combines with continuous sources and
+        schedules."""
+        self._check_forcing(forcing, nsteps)             # both inputs are checked before either is uploaded
+        sched = self._schedule(schedule, nsteps)
+        return self._run_steps(nsteps, fmul, return_frames, out, frame_dtype, sched, self._forcing(forcing, nsteps))
+
+    def _run_steps(self, nsteps, fmul, return_frames, out, frame_dtype, sched, force=None):
         L = self._layout
         if out is not None:
             fmt = self._check_frame_buffer("out", out, (L.batch, nsteps, L.h, L.pitch_c))
@@ -637,19 +724,23 @@ class NavierStokesSimulator(nn.Module):
             fmt = _lib.frame_format(frame_dtype)
             fr = self._new_frames(nsteps, frame_dtype) if return_frames else None
         self._steps(nsteps, fr.data_ptr() if fr is not None else None, L.h * L.pitch_c, nsteps * L.h * L.pitch_c, fmul, fmt,
-                    sched)
+                    sched, force)
         return self._finish_frames(fr) if fr is not None else None
 
-    def run_steps_time_major(self, nsteps, out, fmul=None, *, schedule=None):
+    def run_steps_time_major(self, nsteps, out, fmul=None, *, schedule=None, forcing=None):
         """nsteps consecutive steps whose frames go to `out`, a contiguous [nsteps, batch, h, pitch_c] float32, float16 or
         bfloat16 device buffer owned by the caller (time-major: the frames of one step are one contiguous block).
-        schedule: as run_steps."""
-        self._run_steps_time_major(nsteps, out, fmul, self._schedule(schedule, nsteps))
+        schedule, forcing: as run_steps."""
+        L = self._layout
+        self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
+        self._check_forcing(forcing, nsteps)
+        sched = self._schedule(schedule, nsteps)
+        self._run_steps_time_major(nsteps, out, fmul, sched, self._forcing(forcing, nsteps))
 
-    def _run_steps_time_major(self, nsteps, out, fmul, sched):
+    def _run_steps_time_major(self, nsteps, out, fmul, sched, force=None):
         L = self._layout
         fmt = self._check_frame_buffer("out", out, (nsteps, L.batch, L.h, L.pitch_c))
-        self._steps(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt, sched)
+        self._steps(nsteps, out.data_ptr(), L.batch * L.h * L.pitch_c, L.h * L.pitch_c, fmul, fmt, sched, force)
 
     def divergence_norms(self):
         """(max|div|, ||div||_2) of the un-normalised divergence of the live (u, v), per simulation: [batch, 2] on the host."""

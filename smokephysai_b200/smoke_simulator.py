@@ -55,7 +55,7 @@ class SmokeSimulator(nn.Module):
 
     # -------------------------------------------------------------- batched generation (data_loader.py:37-99)
     def generate_sequences(self, emitters, sequence_length=20, add_fractal=True, to_host=False, steps_per_copy=None,
-                           frame_dtype=torch.float32, continuous=False, schedule=None):
+                           frame_dtype=torch.float32, continuous=False, schedule=None, forcing=None):
         """Reset, splat one emitter list per simulation, run sequence_length steps.
 
         emitters[b] = [((x, y), intensity), ...] for simulation b (len == batch).  Returns frames
@@ -81,37 +81,43 @@ class SmokeSimulator(nn.Module):
         that move or change intensity, row t added at the head of step t after the samples' emitters were splatted once at the
         reset.  The records are uploaded once per call (through pinned memory when to_host); the chunks of the to_host path read
         their rows of the same records.  It does not combine with continuous sources (continuous=True or the simulator's own):
-        fold constant emitters into the schedule."""
+        fold constant emitters into the schedule.
+
+        forcing = (du, dv), constant or [T, B, ...] per step (NavierStokesSimulator.run_steps): velocity increments added at the
+        head of every step.  Uploaded once per call (through pinned memory when to_host); the chunks of the to_host path read their
+        rows of the same upload.  It combines with continuous sources and schedules."""
         ns = self.ns_solver
         B, T = ns.batch, int(sequence_length)
         _lib.frame_format(frame_dtype)                     # ValueError for an unsupported dtype, before any work
+        if schedule is not None and (continuous or ns._csrc is not None):
+            raise ValueError("a source schedule and continuous sources do not combine: fold the constant emitters into "
+                             "the schedule")
+        ns._check_forcing(forcing, T)                      # both inputs are checked before either is uploaded
         sched = None
         if schedule is not None:
-            if continuous or ns._csrc is not None:
-                raise ValueError("a source schedule and continuous sources do not combine: fold the constant emitters into "
-                                 "the schedule")
             up = ns.upload_schedule(schedule, T, pin=to_host)
             sched = None if up is None else up + (0,)
+        force = ns._forcing(forcing, T, pin=to_host)
         lists = [[(x, y, 8, inten) for (x, y), inten in lst] for lst in emitters]
         ns.setup_grid()
         src, off, _ = ns.upload_sources(lists, pin=to_host)
         fmul = self.fractal_gen.multiplier((ns.h, ns.w), 0.05) if add_fractal else None
         if not continuous:
             ns.splat_uploaded(src, off)
-            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype, sched)
+            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype, sched, force)
         saved = ns._csrc
         ns._csrc = (lists, src, off)
         try:
-            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype)
+            return self._run_sequences(T, fmul, to_host, steps_per_copy, frame_dtype, None, force)
         finally:
             ns._csrc = saved
 
-    def _run_sequences(self, T, fmul, to_host, steps_per_copy, frame_dtype, sched=None):
+    def _run_sequences(self, T, fmul, to_host, steps_per_copy, frame_dtype, sched=None, force=None):
         ns = self.ns_solver
         L = ns._layout
         B = ns.batch
         if not to_host:
-            fr = ns._run_steps(T, fmul, True, None, frame_dtype, sched)
+            fr = ns._run_steps(T, fmul, True, None, frame_dtype, sched, force)
             return fr if B > 1 else fr.unsqueeze(0)
         # one (device, pinned host) buffer pair per frame dtype, keyed (T, dtype): calls that alternate dtypes each keep
         # their own buffers instead of reallocating pinned memory every call or handing one call's frames to the other
@@ -134,8 +140,10 @@ class SmokeSimulator(nn.Module):
         n = int(steps_per_copy) if steps_per_copy else (2 if ns.step_is_fused(2) else 1)
         for t in range(0, T, n):
             m = min(n, T - t)
-            # the chunk's steps t .. t + m - 1 are the schedule's rows t .. t + m - 1 (offsets from offsets[t * B] on)
-            ns._run_steps_time_major(m, dev[t:t + m], fmul, None if sched is None else sched[:2] + (t,))
+            # the chunk's steps t .. t + m - 1 are the schedule's and the forcing's rows t .. t + m - 1 (offsets from offsets[t * B]
+            # on, forcing from element t * B * stride)
+            ns._run_steps_time_major(m, dev[t:t + m], fmul, None if sched is None else sched[:2] + (t,),
+                                     None if force is None else force[:3] + (t,))
             ev = torch.cuda.Event()
             ev.record(main)
             cs.wait_event(ev)
