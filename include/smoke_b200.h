@@ -156,6 +156,13 @@ SMK_API int smk_divergence(const smk_grid_t* g, const float* u, const float* v, 
 SMK_API int smk_jacobi(const smk_grid_t* g, const float* div, float* p, float* p_scratch,
                int32_t K, int32_t T, int32_t* result_in_scratch_host, void* stream);
 
+/*     the same sweeps with solid cells (DESIGN.md s5.7): solid is uint8 [batch][h][pitch_c], non-zero = solid, zero pads, 4-byte
+ *     aligned; simulation b reads solid + b * solid_batch_stride, the stride 0 (one mask for all) or h * pitch_c.  A fluid interior
+ *     cell takes a solid neighbour's value as its own p (Neumann ghost value); solid cells and the ring get +0.0.  With no solid
+ *     cell the result is smk_jacobi's.  Every launch is the scalar masked kernel, whatever the grid size. */
+SMK_API int smk_jacobi_obst(const smk_grid_t* g, const float* div, float* p, float* p_scratch, const uint8_t* solid,
+                            int64_t solid_batch_stride, int32_t K, int32_t T, int32_t* result_in_scratch_host, void* stream);
+
 /* a7  gradient subtract in place (navier_stokes.py:148-149) */
 SMK_API int smk_project(const smk_grid_t* g, const float* p, float* u, float* v, float dt, void* stream);
 
@@ -180,7 +187,7 @@ SMK_API int smk_advect_slab(const smk_grid_t* g, const float* field, float* out,
  *     [batch][nsteps][h][pitch_c] returned copies, multiplied by (1+fmul) when fmul != NULL.
  *     Not available on a slab grid (the host interleaves halo exchanges between the phases).
  *     Every step entry point (smk_step, smk_step_ex, smk_run_steps, smk_run_steps_ex, smk_run_steps_reset_ex,
- *     smk_run_steps_src_ex, smk_run_steps_sched_ex, smk_run_steps_force_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
+ *     smk_run_steps_src_ex, smk_run_steps_sched_ex, smk_run_steps_force_ex, smk_run_steps_obst_ex) checks a call the same way -- frames, grid, all nine state pointers (div included), cur_*,
  *     jacobi_iters, dt, step_kernel -- and refuses a malformed one before anything is enqueued. */
 SMK_API int smk_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
              float* frame, int64_t frame_stride, const float* fmul, void* stream);
@@ -253,6 +260,20 @@ SMK_API int smk_run_steps_force_ex(const smk_grid_t* g, smk_state_t* st, const s
                                    int32_t offsets_step_stride, const float* force_u, const float* force_v, int32_t force_per_step,
                                    int32_t reset, const smk_source_t* reset_sources, const int32_t* reset_offsets,
                                    int32_t* consumed_host, void* stream);
+/*     smk_run_steps_force_ex with solid obstacles (DESIGN.md s5.7).  solid (may be NULL: no obstacles) is uint8 [batch][h][pitch_c],
+ *     non-zero = solid, zero pads, 4-byte aligned; simulation b reads solid + b * solid_batch_stride, the stride 0 (one mask for
+ *     every simulation) or h * pitch_c.  A face of u or v is closed when a cell it touches is solid.  Each step is the reference
+ *     step with: the closed faces of the diffused u, v set to +0.0 before the divergence; the Jacobi sweeps of smk_jacobi_obst; the
+ *     gradient subtract on open faces only; the closed faces of the advected u, v set to +0.0 before the density advection; the
+ *     density and the frame of solid cells set to +0.0 after the decay.  With a mask the call always runs on the phase kernels
+ *     (a reset is not consumed: *consumed_host = 0, nothing enqueued), and SMK_STEP_FUSED is SMK_EUNSUPPORTED.  A misaligned mask or
+ *     a bad stride is SMK_EINVAL before anything is enqueued.  smk_run_steps_force_ex is this entry with solid = NULL. */
+SMK_API int smk_run_steps_obst_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps,
+                                  void* frames, int64_t frame_step_stride, int64_t frame_batch_stride,
+                                  const float* fmul, int32_t frame_format, const smk_source_t* sources, const int32_t* offsets,
+                                  int32_t offsets_step_stride, const float* force_u, const float* force_v, int32_t force_per_step,
+                                  const uint8_t* solid, int64_t solid_batch_stride, int32_t reset, const smk_source_t* reset_sources,
+                                  const int32_t* reset_offsets, int32_t* consumed_host, void* stream);
 /*     u = u + du, v = v + dv over the batch, the cells inside u [h+1][w] and v [h][w+1] only (pads are neither read nor
  *     written); du / dv have the layout of u / v.  The forcing add of one step on the phase kernels; reverse mode also uses it
  *     to accumulate gradients. */
@@ -273,6 +294,9 @@ SMK_API int smk_div_norms(const smk_grid_t* g, const float* u, const float* v, f
 /*     per simulation {max|p' - p|, sum (p' - p)^2} where p' is one more Jacobi sweep (navier_stokes.py:139-145) over
  *     (p, div): the residual of the pressure iteration after the K sweeps of a step.  out[2*batch] zeroed by the caller. */
 SMK_API int smk_jacobi_residual(const smk_grid_t* g, const float* div, const float* p, float* out, void* stream);
+/*     the same with p' the masked sweep of smk_jacobi_obst (solid, solid_batch_stride as there); solid NULL is smk_jacobi_residual */
+SMK_API int smk_jacobi_residual_ex(const smk_grid_t* g, const float* div, const float* p, const uint8_t* solid,
+                                   int64_t solid_batch_stride, float* out, void* stream);
 
 /* a13 FractalGenerator fields (fractal_generator.py:12-62).  Output index [a][b], a < na (= w), b < nb (= h),
  *     as torch.meshgrid(x_w, y_h, indexing='ij') lays them out.  Any of the three outputs may be NULL:

@@ -98,6 +98,10 @@ SIGNATURES = {
                                c_p],
     "smk_run_steps_force_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p, c_p, c_i32, c_p, c_p, c_i32, c_i32, c_p, c_p,
                                C.POINTER(c_i32), c_p],
+    "smk_run_steps_obst_ex": [GP, SP, PP, c_i32, c_p, c_i64, c_i64, c_p, c_i32, c_p, c_p, c_i32, c_p, c_p, c_i32, c_p, c_i64, c_i32, c_p,
+                              c_p, C.POINTER(c_i32), c_p],
+    "smk_jacobi_obst": [GP, c_p, c_p, c_p, c_p, c_i64, c_i32, c_i32, C.POINTER(c_i32), c_p],
+    "smk_jacobi_residual_ex": [GP, c_p, c_p, c_p, c_i64, c_p, c_p],
     "smk_add_forcing": [GP, c_p, c_p, c_p, c_p, c_p],
     "smk_step_is_fused": [GP, PP, c_i32, C.POINTER(c_i32)],
     "smk_fused_plan": [c_i32, c_i32, c_i32, C.POINTER(c_i32), c_i32, C.POINTER(c_i32)],

@@ -257,6 +257,23 @@ int smk_jacobi(const smk_grid_t* g, const float* div, float* p, float* p_scratch
     return rc;
 }
 
+int smk_jacobi_obst(const smk_grid_t* g, const float* div, float* p, float* p_scratch, const uint8_t* solid, int64_t solid_batch_stride,
+                    int32_t K, int32_t T, int32_t* result_in_scratch_host, void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_jacobi_obst"));
+    SMK_TRY(check_ptrs("smk_jacobi_obst", {div, p, p_scratch}));
+    if (p == p_scratch) return fail(SMK_EINVAL, "smk_jacobi_obst: p and p_scratch must differ");
+    if (K < 0 || T < 0) return fail(SMK_EINVAL, "smk_jacobi_obst: negative K or T");
+    if (!result_in_scratch_host) return fail(SMK_EINVAL, "smk_jacobi_obst: result_in_scratch_host is NULL");
+    if (!solid || reinterpret_cast<uintptr_t>(solid) % 4) return fail(SMK_EINVAL, "smk_jacobi_obst: solid is NULL or not 4-byte aligned");
+    if (solid_batch_stride != 0 && solid_batch_stride != (int64_t)g->h * g->pitch_c)
+        return fail(SMK_EINVAL, "smk_jacobi_obst: solid_batch_stride must be 0 or h * pitch_c, got %lld", (long long)solid_batch_stride);
+    int flag = 0;
+    const int rc = launch_jacobi(g, div, p, p_scratch, K, T, &flag, (cudaStream_t)stream, solid, solid_batch_stride);
+    *result_in_scratch_host = flag;
+    return rc;
+}
+
 int smk_project(const smk_grid_t* g, const float* p, float* u, float* v, float dt, void* stream)
 {
     SMK_TRY(check_grid(g, "smk_project"));
@@ -313,12 +330,18 @@ enum StepPlan { PLAN_PHASES, PLAN_FUSED, PLAN_CLUSTER };
 // launch -- several steps (the state stays on chip between them), or a single step of at least 32 simulations.
 // One step of a few simulations is faster spread over all SMs by the phase kernels (tools/step_latency.py: 37 us
 // against 45 us per step() at batch 1; the fused launch also reads and writes the state, ~10 us).
-static int pick_step_kernel(const smk_grid_t* g, const smk_params_t* prm, int nsteps, StepPlan* plan)
+// Solid cells (obstacles) are applied by the phase kernels only: with them the plan is always PLAN_PHASES.
+static int pick_step_kernel(const smk_grid_t* g, const smk_params_t* prm, int nsteps, StepPlan* plan, bool solid = false)
 {
     *plan = PLAN_PHASES;
     if (prm->step_kernel == SMK_STEP_PHASES) return SMK_OK;
     if (prm->step_kernel != SMK_STEP_AUTO && prm->step_kernel != SMK_STEP_FUSED)
         return fail(SMK_EINVAL, "smk_step: step_kernel %d is not SMK_STEP_AUTO/_PHASES/_FUSED", prm->step_kernel);
+    if (solid) {
+        if (prm->step_kernel == SMK_STEP_FUSED)
+            return fail(SMK_EUNSUPPORTED, "smk_step: SMK_STEP_FUSED does not apply solid obstacles (the phase kernels do)");
+        return SMK_OK;
+    }
     if (fused_supported(g)) {
         // One simulation per SM pays when there are enough simulations to fill the SMs; a few simulations are faster on the
         // phase kernels spread over all SMs, whose launch gaps programmatic dependent launch has removed.  Measured per step
@@ -396,6 +419,10 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
     if (c.fstep != 0 && c.fstep != 1) return fail(SMK_EINVAL, "%s: force_per_step must be 0 or 1, got %d", who, c.fstep);
     if (c.fstep && !c.fu) return fail(SMK_EINVAL, "%s: force_per_step = 1 without forcing", who);
     SMK_TRY(check_grid(g, who));
+    if (c.solid && reinterpret_cast<uintptr_t>(c.solid) % 4) return fail(SMK_EINVAL, "%s: solid is not 4-byte aligned", who);
+    if (c.sstride != 0 && (!c.solid || c.sstride != (int64_t)g->h * g->pitch_c))
+        return fail(SMK_EINVAL, "%s: solid_batch_stride must be 0 or h * pitch_c (%lld) with a mask, got %lld", who,
+                    (long long)g->h * g->pitch_c, (long long)c.sstride);
     if (g->gh != 0 && (g->gh != g->h || g->row0 != 0))
         return fail(SMK_EUNSUPPORTED, "%s: slab grids are stepped phase by phase with halo exchanges in between", who);
     SMK_TRY(check_ptrs(who, {st->u[0], st->u[1], st->v[0], st->v[1], st->d[0], st->d[1], st->p[0], st->p[1], st->div}));
@@ -403,7 +430,7 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
     if (prm->jacobi_iters < 0) return fail(SMK_EINVAL, "%s: negative jacobi_iters", who);
     if (!(prm->dt != 0.0f)) return fail(SMK_EINVAL, "%s: dt must be non-zero", who);
     StepPlan plan = PLAN_PHASES;
-    SMK_TRY(pick_step_kernel(g, prm, c.nsteps, &plan));
+    SMK_TRY(pick_step_kernel(g, prm, c.nsteps, &plan, c.solid != nullptr));
     if (c.nsteps == 0 || (c.reset && plan != PLAN_FUSED)) return SMK_OK;
     if (plan != PLAN_PHASES) {
         SMK_TRY(launch_steps_fused(g, st, prm, c, s));
@@ -414,7 +441,7 @@ static int run_steps(const char* who, const smk_grid_t* g, smk_state_t* st, cons
     const int64_t fu_step = c.fstep ? (int64_t)g->batch * g->stride_u : 0, fv_step = c.fstep ? (int64_t)g->batch * g->stride_v : 0;
     for (int t = 0; t < c.nsteps; ++t)
         SMK_TRY(phase_step(g, st, prm, c.csrc, c.coff ? c.coff + (int64_t)t * c.cstride : nullptr,
-                           c.fu ? c.fu + t * fu_step : nullptr, c.fv ? c.fv + t * fv_step : nullptr,
+                           c.fu ? c.fu + t * fu_step : nullptr, c.fv ? c.fv + t * fv_step : nullptr, c.solid, c.sstride,
                            c.frames ? static_cast<char*>(c.frames) + (int64_t)t * step_bytes : nullptr,
                            c.frame_batch_stride, c.fmul, c.frame_format, nullptr, nullptr, nullptr, nullptr, s));
     return SMK_OK;
@@ -488,7 +515,19 @@ int smk_run_steps_force_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
                            const float* force_u, const float* force_v, int32_t force_per_step, int32_t reset,
                            const smk_source_t* reset_sources, const int32_t* reset_offsets, int32_t* consumed_host, void* stream)
 {
-    const char* who = "smk_run_steps_force_ex";
+    return smk_run_steps_obst_ex(g, st, prm, nsteps, frames, frame_step_stride, frame_batch_stride, fmul, frame_format, sources,
+                                 offsets, offsets_step_stride, force_u, force_v, force_per_step, nullptr, 0, reset, reset_sources,
+                                 reset_offsets, consumed_host, stream);
+}
+
+int smk_run_steps_obst_ex(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, int32_t nsteps, void* frames,
+                          int64_t frame_step_stride, int64_t frame_batch_stride, const float* fmul, int32_t frame_format,
+                          const smk_source_t* sources, const int32_t* offsets, int32_t offsets_step_stride,
+                          const float* force_u, const float* force_v, int32_t force_per_step, const uint8_t* solid,
+                          int64_t solid_batch_stride, int32_t reset, const smk_source_t* reset_sources, const int32_t* reset_offsets,
+                          int32_t* consumed_host, void* stream)
+{
+    const char* who = solid ? "smk_run_steps_obst_ex" : "smk_run_steps_force_ex";
     if (!consumed_host) return fail(SMK_EINVAL, "%s: consumed_host is NULL", who);
     *consumed_host = 0;
     if (reset != 0 && reset != 1) return fail(SMK_EINVAL, "%s: reset must be 0 or 1, got %d", who, reset);
@@ -497,6 +536,7 @@ int smk_run_steps_force_ex(const smk_grid_t* g, smk_state_t* st, const smk_param
     c.nsteps = nsteps; c.frames = frames; c.frame_step_stride = frame_step_stride; c.frame_batch_stride = frame_batch_stride;
     c.fmul = fmul; c.frame_format = frame_format; c.csrc = sources; c.coff = offsets; c.cstride = offsets_step_stride;
     c.fu = force_u; c.fv = force_v; c.fstep = force_per_step;
+    c.solid = solid; c.sstride = solid_batch_stride;
     c.reset = reset == 1; c.rsrc = reset_sources; c.roff = reset_offsets;
     return run_steps(who, g, st, prm, c, consumed_host, (cudaStream_t)stream);
 }
@@ -522,6 +562,19 @@ int smk_jacobi_residual(const smk_grid_t* g, const float* div, const float* p, f
     SMK_TRY(check_ptrs("smk_jacobi_residual", {div, p}));
     if (!out) return fail(SMK_EINVAL, "smk_jacobi_residual: out NULL");
     return launch_jacobi_residual(g, div, p, out, (cudaStream_t)stream);
+}
+
+int smk_jacobi_residual_ex(const smk_grid_t* g, const float* div, const float* p, const uint8_t* solid, int64_t solid_batch_stride,
+                           float* out, void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_jacobi_residual_ex"));
+    SMK_TRY(check_ptrs("smk_jacobi_residual_ex", {div, p}));
+    if (!out) return fail(SMK_EINVAL, "smk_jacobi_residual_ex: out NULL");
+    if (solid_batch_stride != 0 && (!solid || solid_batch_stride != (int64_t)g->h * g->pitch_c))
+        return fail(SMK_EINVAL, "smk_jacobi_residual_ex: solid_batch_stride must be 0 or h * pitch_c with a mask, got %lld",
+                    (long long)solid_batch_stride);
+    if (!solid) return launch_jacobi_residual(g, div, p, out, (cudaStream_t)stream);
+    return launch_jacobi_residual_obst(g, div, p, solid, solid_batch_stride, out, (cudaStream_t)stream);
 }
 
 int smk_fractal_fields(float* perlin, float* mandel, float* mul, int32_t na, int32_t nb, int32_t pitch, float intensity,

@@ -169,7 +169,9 @@ int launch_diffuse(const float* in, float* out, int rows, int cols, int pitch, i
 int launch_forces_diffuse_div(const smk_grid_t* g, const float* u, const float* v, const float* d,
                               float* uo, float* vo, float* dout, float* div, float dt, float c_uv, float c_d, cudaStream_t s);
 int launch_divergence(const smk_grid_t* g, const float* u, const float* v, float* div, float dt, cudaStream_t s);
-int launch_jacobi(const smk_grid_t* g, const float* div, float* p, float* scratch, int K, int T, int* in_scratch, cudaStream_t s);
+// solid (may be NULL): uint8 [batch][h][pitch_c] solid cells, simulation b at solid + b * solid_stride (k_jacobi_obst, DESIGN.md s5.7)
+int launch_jacobi(const smk_grid_t* g, const float* div, float* p, float* scratch, int K, int T, int* in_scratch, cudaStream_t s,
+                  const uint8_t* solid = nullptr, int64_t solid_stride = 0);
 int launch_project(const smk_grid_t* g, const float* p, float* u, float* v, float dt, cudaStream_t s);
 int launch_bilerp(const float* f, int rows, int cols, int pitch, const float* y, const float* x, float* out, int64_t n, int mode, cudaStream_t s);
 // part (tiled kernel only, see advect_is_tiled): band_n > 0 -> only the tile rows [band_lo, band_lo + band_n); else every tile row
@@ -189,6 +191,17 @@ bool advect_is_tiled(const smk_grid_t* g, int rows, int cols);
 int advect_tile_rows();
 int launch_div_norms(const smk_grid_t* g, const float* u, const float* v, float* out, cudaStream_t s);
 int launch_jacobi_residual(const smk_grid_t* g, const float* div, const float* p, float* out, cudaStream_t s);
+// solid obstacles (stencil.cu, DESIGN.md s5.7); solid: uint8 [batch][h][pitch_c], simulation b at solid + b * solid_stride
+// O1 (div != NULL: close the faces of u, v and rewrite div) / O4 (div == NULL: close the faces only)
+int launch_obstacle_faces(const smk_grid_t* g, float* u, float* v, float* div, const uint8_t* solid, int64_t solid_stride, float dt,
+                          cudaStream_t s);
+// O3: density and this step's frame (may be NULL) := +0.0 on solid cells
+int launch_obstacle_cells(const smk_grid_t* g, float* d, void* frame, int64_t frame_stride, int frame_format, const uint8_t* solid,
+                          int64_t solid_stride, cudaStream_t s);
+int launch_project_obst(const smk_grid_t* g, const float* p, float* u, float* v, const uint8_t* solid, int64_t solid_stride, float dt,
+                        cudaStream_t s);
+int launch_jacobi_residual_obst(const smk_grid_t* g, const float* div, const float* p, const uint8_t* solid, int64_t solid_stride,
+                                float* out, cudaStream_t s);
 int launch_fractal_fields(float* perlin, float* mandel, float* mul, int na, int nb, int pitch, float intensity, int iterations,
                           const float* px, const float* py, const float* mx, const float* my, cudaStream_t s);
 int launch_frame_features(const float* frames, int64_t frame_stride, int nframes, int h, int w, int pitch,
@@ -212,6 +225,8 @@ struct StepCall {
     const float* fu = nullptr;                // velocity forcing added to u / v at the head of every step (NULL: none), in the
     const float* fv = nullptr;                //   grid's layout; step t of simulation b adds fu + t * (fstep ? batch * stride_u : 0)
     int fstep = 0;                            //   + b * stride_u (v likewise).  0: one pair for every step; 1: a pair per step
+    const uint8_t* solid = nullptr;           // solid cells (NULL: none), uint8 [batch][h][pitch_c]; simulation b at solid + b * sstride
+    int64_t sstride = 0;                      //   (0: one mask for every simulation).  Phase kernels only (DESIGN.md s5.7)
     bool reset = false;                       // start from a reset state splatted once with (rsrc, roff): k_step_fused only
     const smk_source_t* rsrc = nullptr;
     const int32_t* roff = nullptr;
@@ -219,10 +234,12 @@ struct StepCall {
 int launch_steps_fused(const smk_grid_t* g, const smk_state_t* st, const smk_params_t* prm, const StepCall& c, cudaStream_t s);
 // One step on the phase kernels (peer_halo.cu), for a whole grid or a row slab whose ghost rows are current: the continuous
 // emitters (csrc / coff), the velocity forcing (fu / fv, this step's pair), buoyancy + diffusion + divergence, the Jacobi sweeps,
-// the gradient subtract and the three advections.  All per-call inputs may be NULL: the emitters, the forcing, the frame (whole
-// grids), the reach guards chk_* and the comm of the tail push (slabs).
+// the gradient subtract and the three advections, with the solid cells (whole grids) applied as DESIGN.md s5.7 defines.  All
+// per-call inputs may be NULL: the emitters, the forcing, the solid cells, the frame (whole grids), the reach guards chk_* and the
+// comm of the tail push (slabs).
 int phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
-               const float* fu, const float* fv, void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+               const float* fu, const float* fv, const uint8_t* solid, int64_t solid_stride,
+               void* frame, int64_t frame_stride, const float* fmul, int frame_format,
                const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
                const smk_peer_comm_t* push_comm, cudaStream_t s);
 int fused_plan(int nsims, int nsteps, int piece_len, int32_t* items, int capacity, int* count);

@@ -94,6 +94,130 @@ k_jacobi(const float* __restrict__ pin, float* __restrict__ pout, const float* _
     }
 }
 
+// ---- masked variant: solid obstacles (DESIGN.md s5.7) -------------------------------------------------------------------
+// The scalar strip of k_jacobi with a uint8 cell mask (non-zero = solid) of the pressure's pitch: per sweep a fluid interior cell
+// computes 0.25 * ((((qN + qS) + qW) + qE) - div), qX the neighbour's p when that neighbour is fluid and the cell's own p when it
+// is solid (Neumann ghost value); solid cells and the ring get +0.0.  With no solid cell this is the reference sweep bit for bit.
+// The mask does not change between sweeps, so each lane reads it once (one 32-bit word = its four cells, per strip row and the
+// rows above and below the strip, through L1) and folds it into 5 bits per cell: keep, and the four neighbours' solid flags.
+// The tile, overlap and store are k_jacobi's, so every tile configuration and multi-launch chain of run_cfg applies unchanged.
+__device__ __forceinline__ float4 stencil_row_obst(const float4 up, const float4 cur, const float4 dn, const float4 d, const unsigned f)
+{
+    const float left = __shfl_up_sync(0xffffffffu, cur.w, 1);
+    const float right = __shfl_down_sync(0xffffffffu, cur.x, 1);
+    const float c[4] = {cur.x, cur.y, cur.z, cur.w}, u[4] = {up.x, up.y, up.z, up.w}, dd[4] = {dn.x, dn.y, dn.z, dn.w};
+    const float dv[4] = {d.x, d.y, d.z, d.w};
+    float o[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const unsigned bits = f >> (5 * k);
+        const float qn = (bits & 2u) ? c[k] : u[k];
+        const float qs = (bits & 4u) ? c[k] : dd[k];
+        const float qw = (bits & 8u) ? c[k] : (k == 0 ? left : c[k - 1]);
+        const float qe = (bits & 16u) ? c[k] : (k == 3 ? right : c[k + 1]);
+        float s = qn + qs;
+        s = s + qw;
+        s = s + qe;
+        s = s - dv[k];
+        o[k] = (bits & 1u) ? 0.25f * s : 0.0f;
+    }
+    return make_float4(o[0], o[1], o[2], o[3]);
+}
+
+template <int R, int NW>
+__global__ void __launch_bounds__(NW * 32, (NW * 32 <= 256) ? 2 : 1)
+k_jacobi_obst(const float* __restrict__ pin, float* __restrict__ pout, const float* __restrict__ div,
+              const uint8_t* __restrict__ solid, const long long sstride,
+              const int h, const int w, const int pitch, const long long bstride,
+              const int T, const int HX, const int ox, const int oy)
+{
+    pdl_prologue();
+    __shared__ float4 halo[2][2][NW][32];          // [buffer][0: first row, 1: last row][warp][lane]
+
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int x0 = blockIdx.x * ox, y0 = blockIdx.y * oy;
+    const int gj = x0 + lane * 4;
+    const int gi0 = y0 + warp * R;
+    const size_t boff = (size_t)blockIdx.z * (size_t)bstride;
+    pin += boff; pout += boff; div += boff;
+    solid += (size_t)blockIdx.z * (size_t)sstride;
+
+    float4 P[R], D[R];
+    const bool colin = gj < pitch;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        const int gi = gi0 + r;
+        if (colin && gi < h) {
+            P[r] = *reinterpret_cast<const float4*>(pin + (size_t)gi * pitch + gj);
+            D[r] = __ldg(reinterpret_cast<const float4*>(div + (size_t)gi * pitch + gj));
+        } else {
+            P[r] = make_float4(0.f, 0.f, 0.f, 0.f);
+            D[r] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+    }
+    // cell flags: bit 5k keep (fluid and interior), 5k+1 .. 5k+4 the N, S, W, E neighbour is solid.  Cells outside the grid read
+    // as fluid; they are never kept, and an interior cell's neighbours are all inside.
+    unsigned F[R];
+    {
+        auto mrow = [&](const int gi) -> unsigned {
+            return (colin && gi >= 0 && gi < h) ? __ldg(reinterpret_cast<const unsigned*>(solid + (size_t)gi * pitch + gj)) : 0u;
+        };
+        unsigned above = mrow(gi0 - 1), me = mrow(gi0);
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const unsigned below = mrow(gi0 + r + 1);
+            const unsigned lw = __shfl_up_sync(0xffffffffu, me, 1), rw = __shfl_down_sync(0xffffffffu, me, 1);
+            const int gi = gi0 + r;
+            const bool rowin = gi >= 1 && gi <= h - 2;
+            unsigned f = 0;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                const bool keep = rowin && gj + k >= 1 && gj + k <= w - 2 && ((me >> (8 * k)) & 0xffu) == 0;
+                const bool sn = ((above >> (8 * k)) & 0xffu) != 0, ss = ((below >> (8 * k)) & 0xffu) != 0;
+                const bool sw = (k == 0 ? (lw >> 24) : (me >> (8 * (k - 1)))) & 0xffu;
+                const bool se = (k == 3 ? rw : (me >> (8 * (k + 1)))) & 0xffu;
+                f |= ((keep ? 1u : 0u) | (sn ? 2u : 0u) | (ss ? 4u : 0u) | (sw ? 8u : 0u) | (se ? 16u : 0u)) << (5 * k);
+            }
+            F[r] = f;
+            above = me; me = below;
+        }
+    }
+    const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
+
+    halo[0][0][warp][lane] = P[0];
+    halo[0][1][warp][lane] = P[R - 1];
+    __syncthreads();
+    for (int s = 0; s < T; ++s) {
+        const int buf = s & 1;
+        float4 prev = warp > 0 ? halo[buf][1][warp - 1][lane] : zero4;
+        const float4 dn = warp < NW - 1 ? halo[buf][0][warp + 1][lane] : zero4;
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const float4 cur = P[r];
+            P[r] = stencil_row_obst(prev, cur, r + 1 < R ? P[r + 1] : dn, D[r], F[r]);
+            prev = cur;
+        }
+        if (s + 1 < T) {
+            halo[buf ^ 1][0][warp][lane] = P[0];
+            halo[buf ^ 1][1][warp][lane] = P[R - 1];
+            __syncthreads();
+        }
+    }
+
+    const int vx0 = x0 + (blockIdx.x > 0 ? HX : 0);
+    const int vx1 = (blockIdx.x + 1 < gridDim.x) ? x0 + 128 - HX : pitch;
+    const int vy0 = y0 + (blockIdx.y > 0 ? T : 0);
+    const int vy1 = (blockIdx.y + 1 < gridDim.y) ? y0 + NW * R - T : h;
+    if (gj >= vx0 && gj < vx1 && gj < pitch) {
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const int gi = gi0 + r;
+            if (gi >= vy0 && gi < vy1 && gi < h)
+                *reinterpret_cast<float4*>(pout + (size_t)gi * pitch + gj) = P[r];
+        }
+    }
+}
+
 // Packed variant (see jacobi_core.cuh): add.f32x2 / mul.f32x2 halve the FP32 issue slots of a sweep.  The strip is
 // always 8 rows per thread (R == 8); sweeps ping-pong between two register sets, two sweeps per loop trip.
 template <int R, int NW, int PMASK>
@@ -562,8 +686,10 @@ static int launch_stream(const smk_grid_t* g, const float* src, float* dst, cons
     return check_launch("k_jacobi_stream");
 }
 
+// solid != NULL: every launch is k_jacobi_obst (the packed and streaming kernels have no masked variant)
 template <int R, int NW>
-static int run_cfg(const smk_grid_t* g, const float* div, float* a, float* b, int K, int T, int* in_scratch, cudaStream_t s, const int stream = 0)
+static int run_cfg(const smk_grid_t* g, const float* div, float* a, float* b, int K, int T, int* in_scratch, cudaStream_t s, const int stream = 0,
+                   const uint8_t* solid = nullptr, const int64_t solid_stride = 0)
 {
     const int TH = R * NW;
     const bool whole = (g->h <= TH) && (g->w <= 128);
@@ -577,7 +703,7 @@ static int run_cfg(const smk_grid_t* g, const float* div, float* a, float* b, in
         const int nx = ntiles(g->w, 128, HX), ny = ntiles(g->h, TH, t);
         dim3 grid(nx, ny, g->batch);
         int rc;
-        int stream_mode = (R == 8 && (NW == 16 || NW == 8)) ? stream : 0;
+        int stream_mode = (R == 8 && (NW == 16 || NW == 8) && !solid) ? stream : 0;
         if (stream_mode == 2 && (g->pitch_c < 128 || g->h < TH)) stream_mode = 1;       // the TMA box is 128 x TH: keep it inside the tensor
         if (stream_mode) {
             rc = launch_stream<(R == 8 && NW == 8) ? 8 : 16>(g, src, dst, div, t, HX, nx, ny, stream_mode, s);
@@ -591,7 +717,10 @@ static int run_cfg(const smk_grid_t* g, const float* div, float* a, float* b, in
             ProfScope prof_(SMK_PH_JACOBI, s);
 #define SMK_PACKED_CASE(M) case M: launch_chain(k_jacobi_packed<8, NW, M>, grid, dim3(NW * 32), 0, s, src, dst, div, g->h, g->w, g->pitch_c, \
                                                            (long long)g->stride_c, t, HX, 128 - 2 * HX, TH - 2 * t); break;
-            if (R == 8 && use_packed()) {
+            if (solid)
+                launch_chain(k_jacobi_obst<R, NW>, grid, dim3(NW * 32), 0, s, src, dst, div, solid, (long long)solid_stride, g->h, g->w,
+                             g->pitch_c, (long long)g->stride_c, t, HX, 128 - 2 * HX, TH - 2 * t);
+            else if (R == 8 && use_packed()) {
                 switch (use_packed()) {
                     SMK_PACKED_CASE(6) SMK_PACKED_CASE(9) SMK_PACKED_CASE(2) SMK_PACKED_CASE(7) SMK_PACKED_CASE(16)
                     default: launch_chain(k_jacobi_packed<8, NW, 15>, grid, dim3(NW * 32), 0, s, src, dst, div, g->h, g->w, g->pitch_c,
@@ -600,7 +729,7 @@ static int run_cfg(const smk_grid_t* g, const float* div, float* a, float* b, in
             } else
                 launch_chain(k_jacobi<R, NW>, grid, dim3(NW * 32), 0, s, src, dst, div, g->h, g->w, g->pitch_c, (long long)g->stride_c,
                                                          t, HX, 128 - 2 * HX, TH - 2 * t);
-            rc = check_launch("k_jacobi");
+            rc = check_launch(solid ? "k_jacobi_obst" : "k_jacobi");
         }
         if (rc != SMK_OK) return rc;
         float* tmp = src; src = dst; dst = tmp;
@@ -619,18 +748,21 @@ static int sm_count()
     return n;
 }
 
-int launch_jacobi(const smk_grid_t* g, const float* div, float* p, float* scratch, int K, int T, int* in_scratch, cudaStream_t s)
+int launch_jacobi(const smk_grid_t* g, const float* div, float* p, float* scratch, int K, int T, int* in_scratch, cudaStream_t s,
+                  const uint8_t* solid, int64_t solid_stride)
 {
     *in_scratch = 0;
     if (K <= 0) return SMK_OK;
     if (g->batch > 65535) return fail(SMK_EUNSUPPORTED, "smk_jacobi: batch %d > 65535", g->batch);
-    if (g->w <= 128 && g->h <= 32) return run_cfg<4, 8>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s);
-    if (g->w <= 128 && g->h <= 64) return run_cfg<8, 8>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s);
-    if (g->w <= 128 && g->h <= 128) return run_cfg<8, 16>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s);
+    const uint8_t* S = solid;
+    const int64_t ss = solid_stride;
+    if (g->w <= 128 && g->h <= 32) return run_cfg<4, 8>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s, 0, S, ss);
+    if (g->w <= 128 && g->h <= 64) return run_cfg<8, 8>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s, 0, S, ss);
+    if (g->w <= 128 && g->h <= 128) return run_cfg<8, 16>(g, div, p, scratch, K, T > 0 ? T : 8, in_scratch, s, 0, S, ss);
     // large grids: overlapped tiles.  T must leave a positive advance in both directions.
     int tile = 0;                                   // 0 auto, 1: 64 x 128 (8 warps), 2: 128 x 128 (16 warps), 3: 64 x 128 (16 warps)
     if (env().jacobi_tile != SMK_ENV_UNSET) tile = env().jacobi_tile;
-    int stream = stream_env();                      // -1 auto, 0 off, 1 LDGSTS, 2 TMA (k_jacobi_stream)
+    int stream = S ? 0 : stream_env();              // -1 auto, 0 off, 1 LDGSTS, 2 TMA (k_jacobi_stream)
     if (tile == 0) {
         // Many waves of CTAs (>= 4 per SM: 4096^2, or a 1/8 slab of 8192^2): overlap one tile's load / store with another's sweeps.
         // Without the TMA kernel: 64 x 128 tiles at two CTAs per SM (7-8 % faster than 128 x 128 tiles at 4096^2 and 8192^2, equal
@@ -649,9 +781,9 @@ int launch_jacobi(const smk_grid_t* g, const float* div, float* p, float* scratc
     }
     if (stream < 0) stream = 0;
     if (T <= 0) T = (tile == 1 || tile == 3 || stream != 0) ? 10 : pick_T(g, K, 128, 24, sm_count());
-    if (tile == 1) return run_cfg<8, 8>(g, div, p, scratch, K, min(T, 12), in_scratch, s, stream);
-    if (tile == 3) return run_cfg<4, 16>(g, div, p, scratch, K, min(T, 12), in_scratch, s);
-    return run_cfg<8, 16>(g, div, p, scratch, K, min(T, stream != 0 ? 12 : 24), in_scratch, s, stream);
+    if (tile == 1) return run_cfg<8, 8>(g, div, p, scratch, K, min(T, 12), in_scratch, s, stream, S, ss);
+    if (tile == 3) return run_cfg<4, 16>(g, div, p, scratch, K, min(T, 12), in_scratch, s, 0, S, ss);
+    return run_cfg<8, 16>(g, div, p, scratch, K, min(T, stream != 0 ? 12 : 24), in_scratch, s, stream, S, ss);
 }
 
 }  // namespace smk

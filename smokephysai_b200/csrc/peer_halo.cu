@@ -261,14 +261,27 @@ static int advect_density(const smk_grid_t* g, const float* d_in, float* d_out, 
 // frame copy (:173).  The live copies of u and density flip; so does v's, except on big fields, where the gradient subtract runs
 // inside the u advection (k_advect_tiled<.., 1>, stencil.cu), the projected v passes through the spare copy and the live v ends
 // where it was.
+// With solid cells (whole grids only, push_comm NULL) the route is always the unfused one: k_project_obst subtracts on open faces,
+// O4 closes the faces of the advected u and v before the density advection, O3 zeroes the solid cells of the density and the frame.
 static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, void* frame, int64_t frame_stride,
                           const float* fmul, int frame_format,
                           const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
-                          const smk_peer_comm_t* push_comm, cudaStream_t s)
+                          const smk_peer_comm_t* push_comm, cudaStream_t s, const uint8_t* solid = nullptr, int64_t solid_stride = 0)
 {
     const int cu = st->cur_u, cv = st->cur_v, cd = st->cur_d;
     float *u1 = st->u[cu], *u0 = st->u[cu ^ 1], *v1 = st->v[cv], *v0 = st->v[cv ^ 1], *d1 = st->d[cd], *d0 = st->d[cd ^ 1];
     float* pl = st->p[st->cur_p];
+    if (solid) {
+        SMK_TRY_(launch_project_obst(g, pl, u1, v1, solid, solid_stride, prm->dt, s));
+        SMK_TRY_(launch_advect(g, u1, u0, g->h + 1, g->w, g->pitch_u, g->stride_u, u1, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_u, s));
+        SMK_TRY_(launch_advect(g, v1, v0, g->h, g->w + 1, g->pitch_v, g->stride_v, u0, v1, prm->dt, 1.0f, nullptr, 0, nullptr, chk_v, s));
+        SMK_TRY_(launch_obstacle_faces(g, u0, v0, nullptr, solid, solid_stride, prm->dt, s));                          // O4
+        SMK_TRY_(launch_advect(g, d1, d0, g->h, g->w, g->pitch_c, g->stride_c, u0, v0, prm->dt, prm->decay, frame, frame_stride, fmul,
+                               chk_d, s, 0, nullptr, nullptr, nullptr, frame_format));
+        SMK_TRY_(launch_obstacle_cells(g, d0, frame, frame_stride, frame_format, solid, solid_stride, s));              // O3
+        st->cur_u = cu ^ 1; st->cur_v = cv ^ 1; st->cur_d = cd ^ 1;
+        return SMK_OK;
+    }
     if (advect_can_fuse_project(g)) {
         // u advection with the gradient subtract inside; it leaves the projected v in the spare copy v0, so the v advection runs
         // v0 -> v1 and the live v stays in the copy it was in
@@ -289,7 +302,8 @@ static int project_advect(const smk_grid_t* g, smk_state_t* st, const smk_params
 }
 
 int smk::phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm, const smk_source_t* csrc, const int32_t* coff,
-                    const float* fu, const float* fv, void* frame, int64_t frame_stride, const float* fmul, int frame_format,
+                    const float* fu, const float* fv, const uint8_t* solid, int64_t solid_stride,
+                    void* frame, int64_t frame_stride, const float* fmul, int frame_format,
                     const smk_slab_check_t* chk_u, const smk_slab_check_t* chk_v, const smk_slab_check_t* chk_d,
                     const smk_peer_comm_t* push_comm, cudaStream_t s)
 {
@@ -300,12 +314,15 @@ int smk::phase_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* pr
     SMK_TRY_(launch_forces_diffuse_div(g, st->u[cu], st->v[cv], st->d[cd], st->u[cu ^ 1], st->v[cv ^ 1], st->d[cd ^ 1], st->div,
                                        prm->dt, prm->c_uv, prm->c_d, s));
     st->cur_u = cu ^ 1; st->cur_v = cv ^ 1; st->cur_d = cd ^ 1;
+    // O1: close the faces next to solid cells, and the divergence from the closed faces
+    if (solid) SMK_TRY_(launch_obstacle_faces(g, st->u[st->cur_u], st->v[st->cur_v], st->div, solid, solid_stride, prm->dt, s));
     // 3. Jacobi sweeps                                                         :139-145
     int flip = 0;
-    SMK_TRY_(launch_jacobi(g, st->div, st->p[st->cur_p], st->p[st->cur_p ^ 1], prm->jacobi_iters, prm->sweeps_per_launch, &flip, s));
+    SMK_TRY_(launch_jacobi(g, st->div, st->p[st->cur_p], st->p[st->cur_p ^ 1], prm->jacobi_iters, prm->sweeps_per_launch, &flip, s,
+                           solid, solid_stride));
     st->cur_p ^= flip;
     // 4-5. gradient subtract + the three advections + decay + frame            :148-149, :166-173
-    return project_advect(g, st, prm, frame, frame_stride, fmul, frame_format, chk_u, chk_v, chk_d, push_comm, s);
+    return project_advect(g, st, prm, frame, frame_stride, fmul, frame_format, chk_u, chk_v, chk_d, push_comm, s, solid, solid_stride);
 }
 
 #define SMK_TRY(x) do { const int rc_ = (x); if (rc_ != SMK_OK) return rc_; } while (0)
@@ -397,7 +414,7 @@ int smk_slab_step(const smk_grid_t* g, smk_state_t* st, const smk_params_t* prm,
         SMK_TRY(peer_xfer(comm, base, false, s));
     }
     // SMK_SLAB_PUSH_TAIL: the ghost rows of the NEXT step leave from the middle of the density advection
-    return phase_step(g, st, prm, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d,
+    return phase_step(g, st, prm, nullptr, nullptr, nullptr, nullptr, nullptr, 0, nullptr, 0, nullptr, SMK_FRAME_F32, chk_u, chk_v, chk_d,
                       (comm && (flags & SMK_SLAB_PUSH_TAIL)) ? comm : nullptr, s);
 }
 

@@ -1355,4 +1355,168 @@ int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int
     return check_launch("k_apply_mul");
 }
 
+// ---- solid obstacles (DESIGN.md s5.7) -------------------------------------------------------------------
+// S: uint8 [batch][h][pitch_c], non-zero = solid, simulation b at S + b * ss (ss = 0: one mask for all).  u face (i, j) lies
+// between cells (i-1, j) and (i, j), v face (i, j) between (i, j-1) and (i, j); a face is closed when a cell it touches that
+// exists is solid.  Closing a face is a store of +0.0 (a multiply by 0 would give -0 or NaN).
+__device__ __forceinline__ bool u_closed(const uint8_t* S, const int h, const int pc, const int i, const int j)
+{
+    return (i >= 1 && S[(size_t)(i - 1) * pc + j] != 0) || (i < h && S[(size_t)i * pc + j] != 0);
+}
+__device__ __forceinline__ bool v_closed(const uint8_t* S, const int w, const int pc, const int i, const int j)
+{
+    return (j >= 1 && S[(size_t)i * pc + j - 1] != 0) || (j < w && S[(size_t)i * pc + j] != 0);
+}
+
+// O1 (DIV != NULL): close the faces of the diffused u, v and rewrite the divergence from them; O4 (DIV == NULL): close the faces of
+// the advected u, v.  Thread (i, j) owns u face (i, j), v face (i, j) and cell (i, j); it reads a neighbour's face only when that
+// face is open, which no thread writes.
+__global__ void __launch_bounds__(256)
+k_obstacle_faces(float* __restrict__ U, float* __restrict__ V, float* __restrict__ DIV, const uint8_t* __restrict__ S,
+                 const int h, const int w, const int pu, const int pv, const int pc,
+                 const long long su_, const long long sv_, const long long sc_, const long long ss_, const float dt)
+{
+    pdl_prologue();
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    const size_t b = blockIdx.z;
+    U += b * su_; V += b * sv_; S += b * ss_;
+    const bool cu0 = i <= h && j < w && u_closed(S, h, pc, i, j);
+    const bool cv0 = i < h && j <= w && v_closed(S, w, pc, i, j);
+    if (cu0) U[(size_t)i * pu + j] = 0.0f;
+    if (cv0) V[(size_t)i * pv + j] = 0.0f;
+    if (DIV && i < h && j < w) {
+        const float u0 = cu0 ? 0.0f : U[(size_t)i * pu + j];
+        const float u1 = u_closed(S, h, pc, i + 1, j) ? 0.0f : U[(size_t)(i + 1) * pu + j];
+        const float v0 = cv0 ? 0.0f : V[(size_t)i * pv + j];
+        const float v1 = v_closed(S, w, pc, i, j + 1) ? 0.0f : V[(size_t)i * pv + j + 1];
+        float s = u1 - u0;                                   // the divergence of navier_stokes.py:136
+        s = s + v1;
+        s = s - v0;
+        DIV[b * sc_ + (size_t)i * pc + j] = s / dt;
+    }
+}
+
+int launch_obstacle_faces(const smk_grid_t* g, float* u, float* v, float* div, const uint8_t* solid, int64_t solid_stride, float dt,
+                          cudaStream_t s)
+{
+    const dim3 grid((g->w + 1 + 31) / 32, (g->h + 1 + 7) / 8, g->batch);
+    ProfScope prof_(SMK_PH_OTHER, s);
+    launch_chain(k_obstacle_faces, grid, dim3(32, 8), 0, s, u, v, div, solid, g->h, g->w, g->pitch_u, g->pitch_v, g->pitch_c,
+                 (long long)g->stride_u, (long long)g->stride_v, (long long)g->stride_c, (long long)solid_stride, dt);
+    return check_launch("k_obstacle_faces");
+}
+
+// O3: the density of solid cells, and their element of this step's frame (any SMK_FRAME_* format), := +0.0
+__global__ void __launch_bounds__(256)
+k_obstacle_cells(float* __restrict__ D, void* frame, const long long frame_stride, const int frame_format,
+                 const uint8_t* __restrict__ S, const int h, const int w, const int pc, const long long sc_, const long long ss_)
+{
+    pdl_prologue();
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    if (i >= h || j >= w) return;
+    const size_t b = blockIdx.z;
+    if (S[b * ss_ + (size_t)i * pc + j] == 0) return;
+    D[b * sc_ + (size_t)i * pc + j] = 0.0f;
+    if (frame) frame_st1(frame, b * frame_stride + (size_t)i * pc + j, 0.0f, frame_format);
+}
+
+int launch_obstacle_cells(const smk_grid_t* g, float* d, void* frame, int64_t frame_stride, int frame_format, const uint8_t* solid,
+                          int64_t solid_stride, cudaStream_t s)
+{
+    const dim3 grid((g->w + 31) / 32, (g->h + 7) / 8, g->batch);
+    ProfScope prof_(SMK_PH_OTHER, s);
+    launch_chain(k_obstacle_cells, grid, dim3(32, 8), 0, s, d, frame, (long long)frame_stride, frame_format, solid, g->h, g->w,
+                 g->pitch_c, (long long)g->stride_c, (long long)solid_stride);
+    return check_launch("k_obstacle_cells");
+}
+
+// The gradient subtract of k_project on open faces only (u rows 1 .. h-1, v columns 1 .. w-1, as navier_stokes.py:148-149);
+// closed faces keep the +0.0 of O1.  One thread per u face (i, j) and v face (i, j).
+__global__ void __launch_bounds__(256)
+k_project_obst(const float* __restrict__ P, float* __restrict__ U, float* __restrict__ V, const uint8_t* __restrict__ S,
+               const int h, const int w, const int pu, const int pv, const int pc,
+               const long long su_, const long long sv_, const long long sc_, const long long ss_, const float dt)
+{
+    pdl_prologue();
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    if (i >= h) return;
+    const size_t b = blockIdx.z;
+    P += b * sc_; U += b * su_; V += b * sv_; S += b * ss_;
+    if (i >= 1 && j < w && !u_closed(S, h, pc, i, j)) {
+        const float g = P[(size_t)i * pc + j] - P[(size_t)(i - 1) * pc + j];
+        const float t = dt * g;
+        U[(size_t)i * pu + j] = U[(size_t)i * pu + j] - t;
+    }
+    if (j >= 1 && j < w && !v_closed(S, w, pc, i, j)) {
+        const float g = P[(size_t)i * pc + j] - P[(size_t)i * pc + j - 1];
+        const float t = dt * g;
+        V[(size_t)i * pv + j] = V[(size_t)i * pv + j] - t;
+    }
+}
+
+int launch_project_obst(const smk_grid_t* g, const float* p, float* u, float* v, const uint8_t* solid, int64_t solid_stride, float dt,
+                        cudaStream_t s)
+{
+    const dim3 grid((g->w + 31) / 32, (g->h + 7) / 8, g->batch);
+    ProfScope prof_(SMK_PH_PROJECT, s);
+    launch_chain(k_project_obst, grid, dim3(32, 8), 0, s, p, u, v, solid, g->h, g->w, g->pitch_u, g->pitch_v, g->pitch_c,
+                 (long long)g->stride_u, (long long)g->stride_v, (long long)g->stride_c, (long long)solid_stride, dt);
+    return check_launch("k_project_obst");
+}
+
+// k_jacobi_residual with p' the masked sweep of k_jacobi_obst (Neumann ghost values at solid neighbours, 0 on solid cells)
+__global__ void __launch_bounds__(256)
+k_jacobi_residual_obst(const float* __restrict__ P, const float* __restrict__ DIV, const uint8_t* __restrict__ S, float* __restrict__ out,
+                       const int h, const int w, const int pc, const long long sc_, const long long ss_)
+{
+    const size_t b = blockIdx.z;
+    P += b * sc_; DIV += b * sc_; S += b * ss_;
+    float mx = 0.f, ss = 0.f;
+    for (int i = blockIdx.y; i < h; i += gridDim.y)
+        for (int j = blockIdx.x * 256 + threadIdx.x; j < w; j += gridDim.x * 256) {
+            const size_t c = (size_t)i * pc + j;
+            const float pc0 = P[c];
+            float pn = 0.f;
+            if (i >= 1 && i <= h - 2 && j >= 1 && j <= w - 2 && S[c] == 0) {
+                float s = (S[c - pc] ? pc0 : P[c - pc]) + (S[c + pc] ? pc0 : P[c + pc]);
+                s = s + (S[c - 1] ? pc0 : P[c - 1]);
+                s = s + (S[c + 1] ? pc0 : P[c + 1]);
+                pn = 0.25f * (s - DIV[c]);
+            }
+            const float r = pn - pc0;
+            mx = fmaxf(mx, fabsf(r));
+            ss += r * r;
+        }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        ss += __shfl_xor_sync(0xffffffffu, ss, o);
+    }
+    __shared__ float smx[8], sss[8];
+    const int lane = threadIdx.x & 31, wp = threadIdx.x >> 5;
+    if (lane == 0) { smx[wp] = mx; sss[wp] = ss; }
+    __syncthreads();
+    if (wp == 0) {
+        mx = lane < 8 ? smx[lane] : 0.f; ss = lane < 8 ? sss[lane] : 0.f;
+#pragma unroll
+        for (int o = 4; o > 0; o >>= 1) {
+            mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+            ss += __shfl_xor_sync(0xffffffffu, ss, o);
+        }
+        if (lane == 0) {
+            atomicMax(reinterpret_cast<int*>(out + 2 * b), __float_as_int(mx));
+            atomicAdd(out + 2 * b + 1, ss);
+        }
+    }
+}
+
+int launch_jacobi_residual_obst(const smk_grid_t* g, const float* div, const float* p, const uint8_t* solid, int64_t solid_stride,
+                                float* out, cudaStream_t s)
+{
+    dim3 grid((g->w + 255) / 256, min(g->h, 64), g->batch);
+    ProfScope prof_(SMK_PH_OTHER, s);
+    k_jacobi_residual_obst<<<grid, 256, 0, s>>>(p, div, solid, out, g->h, g->w, g->pitch_c, g->stride_c, (long long)solid_stride);
+    return check_launch("k_jacobi_residual_obst");
+}
+
 }  // namespace smk

@@ -188,6 +188,27 @@ def forcing_pointers(force, layout):
     return du.data_ptr() + 4 * k * layout.stride_u, dv.data_ptr() + 4 * k * layout.stride_v, int(per_step)
 
 
+def check_obstacles(mask, h, w, batch, device):
+    """An obstacle mask as a tensor, validated: [h, w] or [batch, h, w], bool or integer 0 / 1, numpy, CPU or on `device`;
+    ValueError for anything else, before any work."""
+    t = _as_tensor("mask", mask, "obstacle")
+    if t.dtype != torch.bool and (t.dtype.is_floating_point or t.dtype.is_complex):
+        raise ValueError("an obstacle mask is bool or integer 0 / 1, got %s" % (t.dtype,))
+    if t.dim() not in (2, 3) or tuple(t.shape[-2:]) != (h, w) or (t.dim() == 3 and t.shape[0] != batch):
+        raise ValueError("an obstacle mask is [h, w] = [%d, %d] or [batch, h, w] = [%d, %d, %d], got %s"
+                         % (h, w, batch, h, w, list(t.shape)))
+    if t.device.type != "cpu" and t.device != device:
+        raise ValueError("the obstacle mask is on %s; this simulator runs on %s" % (t.device, device))
+    if t.dtype != torch.bool and bool(((t != 0) & (t != 1)).any()):
+        raise ValueError("an integer obstacle mask holds 0 (fluid) and 1 (solid) only")
+    return t
+
+
+def obstacle_stride(mask, layout):
+    """solid_batch_stride of smk_run_steps_obst_ex for a checked mask: 0 for one [h, w] mask, h * pitch_c for [batch, h, w]."""
+    return 0 if mask.dim() == 2 else layout.h * layout.pitch_c
+
+
 class FieldLayout:
     """Where each field lives inside the single fp32 arena (pure host arithmetic, testable without a GPU).
 
@@ -277,6 +298,9 @@ class NavierStokesSimulator(nn.Module):
         # Continuous sources (set_continuous_sources): None, or (per-simulation lists, device records, device offsets), uploaded once
         # and splatted at the head of every step by the kernels.
         self._csrc = None
+        # Solid obstacles (set_obstacles): None, or (the mask as given, as a bool numpy copy; device uint8 [1 | batch, h, pitch_c];
+        # batch stride in elements), uploaded once and applied by every step on the phase kernels.
+        self._solid = None
         self.setup_grid()
 
     # ------------------------------------------------------------------ state (navier_stokes.py:24-35)
@@ -395,7 +419,10 @@ class NavierStokesSimulator(nn.Module):
                       _lib.STEP_KERNELS[self.step_kernel])
 
     def step_is_fused(self, nsteps=1):
-        """True when a call of nsteps steps (step(): 1, run_steps(n): n) takes the single-launch on-chip path."""
+        """True when a call of nsteps steps (step(): 1, run_steps(n): n) takes the single-launch on-chip path (never with
+        obstacles: they run on the phase kernels)."""
+        if self._solid is not None:
+            return False
         flag = C.c_int32(0)
         prm = self._params()
         _lib.call("smk_step_is_fused", C.byref(self._grid), C.byref(prm), int(nsteps), C.byref(flag))
@@ -510,6 +537,39 @@ class NavierStokesSimulator(nn.Module):
         """The per-simulation lists of set_continuous_sources (a copy), or None when no simulation has one."""
         return None if self._csrc is None else [list(l) for l in self._csrc[0]]
 
+    def set_obstacles(self, mask):
+        """Solid obstacles: mask [h, w] (one for every simulation) or [batch, h, w], bool or integers that are 0 / 1 (1 = solid), as
+        a numpy array, a CPU tensor or a CUDA tensor.  Every later step (step, step_into, run_steps, run_steps_time_major) applies
+        it on the phase kernels (DESIGN.md s5.7): the faces of u and v next to a solid cell are closed (+0.0) before the divergence
+        and after the advection of u and v, the Jacobi sweeps take Neumann ghost values at solid neighbours, the gradient subtract
+        skips closed faces, and the density and frame of solid cells are +0.0 after the step.  It combines with continuous
+        sources, schedules, forcing, frame dtypes and fmul; it does not combine with step_kernel="fused" (ValueError).  The mask is
+        uploaded once, here, into a zero-padded uint8 buffer; setup_grid() keeps it, and setting it leaves the state as it is (the
+        next step closes the faces).  None clears it.  The reference's per-phase methods (diffusion_step, advection_step,
+        pressure_projection, ...) do not apply it.  ValueError for anything else, before any work."""
+        if mask is None:
+            self._solid = None
+            return
+        if self.step_kernel == "fused":
+            raise ValueError('obstacles run on the phase kernels: they do not combine with step_kernel="fused"')
+        if self._layout.gh != 0:
+            raise ValueError("obstacles are not available on row slabs")
+        L = self._layout
+        t = check_obstacles(mask, L.h, L.w, L.batch, self._cuda)
+        n = 1 if t.dim() == 2 else L.batch
+        buf = torch.zeros(n, L.h, L.pitch_c, dtype=torch.uint8, device=self._cuda)
+        buf[:, :, :L.w] = t.reshape(n, L.h, L.w).to(device=self._cuda, dtype=torch.uint8)
+        self._solid = ((t != 0).cpu().numpy().copy(), buf, obstacle_stride(t, L))
+
+    @property
+    def obstacles(self):
+        """The mask of set_obstacles as a bool numpy array of the shape it was given (a copy), or None."""
+        return None if self._solid is None else self._solid[0].copy()
+
+    def _solid_args(self):
+        """(solid pointer, batch stride) of smk_run_steps_obst_ex; (None, 0) without obstacles."""
+        return (None, 0) if self._solid is None else (self._solid[1].data_ptr(), self._solid[2])
+
     def add_sources(self, per_sim):
         """Batched splat: per_sim[b] is the ordered emitter list [(x, y, radius, intensity), ...] of simulation b."""
         if not any(len(l) for l in per_sim):
@@ -617,9 +677,10 @@ class NavierStokesSimulator(nn.Module):
     def _steps(self, nsteps, frames, step_stride, batch_stride, fmul, fmt, sched=None, force=None):
         """nsteps steps of the state, frames (a device pointer or None) at the given strides in elements of frame format fmt.
 
-        One smk_run_steps_force_ex call, with the continuous sources if any (offsets step stride 0) or the schedule `sched`:
-        (device records, device offsets, t0), this call's step t reading the schedule's row t0 + t (offsets step stride batch);
-        and the forcing `force`: (du, dv, per_step, t0) of pack_forcing, this call's step t reading row t0 + t when per_step.
+        One smk_run_steps_obst_ex call, with the obstacles if any, the continuous sources if any (offsets step stride 0) or the
+        schedule `sched`: (device records, device offsets, t0), this call's step t reading the schedule's row t0 + t (offsets step
+        stride batch); and the forcing `force`: (du, dv, per_step, t0) of pack_forcing, this call's step t reading row t0 + t when
+        per_step.
         A pending reset is offered to it first (reset = 1, on the current stream without materializing anything); when the call
         does not consume it (not on k_step_fused), nothing was enqueued, and the reset is applied eagerly before the call is made
         again without it."""
@@ -632,14 +693,17 @@ class NavierStokesSimulator(nn.Module):
         else:
             src, off, stride = None, None, 0
         fu, fv, per_step = forcing_pointers(force, self._layout)
+        if self._solid is not None and self.step_kernel == "fused":
+            raise ValueError('obstacles run on the phase kernels: they do not combine with step_kernel="fused"')
+        solid, sstride = self._solid_args()
         fm = fmul.data_ptr() if fmul is not None else None
         done = C.c_int32(0)
         offer = self._offer_reset()
         for reset in ((True, False) if offer is not None else (False,)):
             rsrc, roff = offer if reset else (None, None)
-            _lib.call("smk_run_steps_force_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
-                      frames, step_stride, batch_stride, fm, fmt, src, off, stride, fu, fv, per_step, int(reset), rsrc, roff,
-                      C.byref(done), _lib.stream_on(self._cuda) if reset else self._stream())
+            _lib.call("smk_run_steps_obst_ex", C.byref(self._grid), C.byref(self._state), C.byref(self._params()), int(nsteps),
+                      frames, step_stride, batch_stride, fm, fmt, src, off, stride, fu, fv, per_step, solid, sstride, int(reset), rsrc,
+                      roff, C.byref(done), _lib.stream_on(self._cuda) if reset else self._stream())
             if done.value:
                 self._pending = None
                 self._stale = True
@@ -753,9 +817,12 @@ class NavierStokesSimulator(nn.Module):
     def jacobi_residual_norms(self):
         """(max|p' - p|, ||p' - p||_2) per simulation, p' = one more Jacobi sweep (navier_stokes.py:139-145) over the live
         pressure and the divergence of the last projection: [batch, 2] on the host.  Meaningful right after
-        pressure_projection() or a step() of the phase-per-kernel path (the fused kernel keeps the divergence in registers)."""
+        pressure_projection() or a step() of the phase-per-kernel path (the fused kernel keeps the divergence in registers).
+        With obstacles p' is the masked sweep the step uses (Neumann ghost values at solid neighbours, 0 on solid cells)."""
         out = torch.zeros(self.batch, 2, dtype=torch.float32, device=self._cuda)
-        _lib.call("smk_jacobi_residual", C.byref(self._grid), self._state.div, self._ptr("p"), out.data_ptr(), self._stream())
+        solid, sstride = self._solid_args()
+        _lib.call("smk_jacobi_residual_ex", C.byref(self._grid), self._state.div, self._ptr("p"), solid, sstride, out.data_ptr(),
+                  self._stream())
         out = out.cpu().double()
         out[:, 1] = out[:, 1].sqrt()
         return out
@@ -765,8 +832,8 @@ class NavierStokesSimulator(nn.Module):
 
 
 # every method that launches runs with the simulator's device current and restores the caller's afterwards
-for _name in ("setup_grid", "_materialize", "add_sources", "set_continuous_sources", "splat_uploaded", "upload_sources",
-              "upload_schedule", "diffusion_step", "advection_step", "_bilerp",
+for _name in ("setup_grid", "_materialize", "add_sources", "set_continuous_sources", "set_obstacles", "splat_uploaded",
+              "upload_sources", "upload_schedule", "diffusion_step", "advection_step", "_bilerp",
               "pressure_projection", "step", "step_into", "run_steps", "_run_steps", "run_steps_time_major", "_run_steps_time_major",
               "divergence_norms",
               "jacobi_residual_norms", "step_is_fused"):

@@ -43,6 +43,10 @@ class SmokeSimulator(nn.Module):
         lists = ns.continuous_sources or [[] for _ in range(ns.batch)]
         ns.set_continuous_sources([lst + new for lst in lists])
 
+    def set_obstacles(self, mask):
+        """Solid obstacles of every later step: NavierStokesSimulator.set_obstacles (None clears them)."""
+        self.ns_solver.set_obstacles(mask)
+
     def simulate_step(self, add_fractal=True):
         """One simulation step; returns the (fractal-scaled) density frame (smoke_simulator.py:31-45)."""
         ns = self.ns_solver
@@ -55,7 +59,7 @@ class SmokeSimulator(nn.Module):
 
     # -------------------------------------------------------------- batched generation (data_loader.py:37-99)
     def generate_sequences(self, emitters, sequence_length=20, add_fractal=True, to_host=False, steps_per_copy=None,
-                           frame_dtype=torch.float32, continuous=False, schedule=None, forcing=None):
+                           frame_dtype=torch.float32, continuous=False, schedule=None, forcing=None, obstacles=None):
         """Reset, splat one emitter list per simulation, run sequence_length steps.
 
         emitters[b] = [((x, y), intensity), ...] for simulation b (len == batch).  Returns frames
@@ -85,7 +89,24 @@ class SmokeSimulator(nn.Module):
 
         forcing = (du, dv), constant or [T, B, ...] per step (NavierStokesSimulator.run_steps): velocity increments added at the
         head of every step.  Uploaded once per call (through pinned memory when to_host); the chunks of the to_host path read their
-        rows of the same upload.  It combines with continuous sources and schedules."""
+        rows of the same upload.  It combines with continuous sources and schedules.
+
+        obstacles: a solid mask for this call ([h, w] or [batch, h, w], NavierStokesSimulator.set_obstacles); the simulator's own
+        obstacles (if any) apply when it is None, and are restored after the call.  With obstacles the steps run on the phase
+        kernels, and steps_per_copy defaults to 1."""
+        ns = self.ns_solver
+        if obstacles is None:
+            return self._generate(emitters, sequence_length, add_fractal, to_host, steps_per_copy, frame_dtype, continuous, schedule,
+                                  forcing)
+        saved = ns._solid
+        ns.set_obstacles(obstacles)                        # ValueError for a bad mask, before any work
+        try:
+            return self._generate(emitters, sequence_length, add_fractal, to_host, steps_per_copy, frame_dtype, continuous, schedule,
+                                  forcing)
+        finally:
+            ns._solid = saved
+
+    def _generate(self, emitters, sequence_length, add_fractal, to_host, steps_per_copy, frame_dtype, continuous, schedule, forcing):
         ns = self.ns_solver
         B, T = ns.batch, int(sequence_length)
         _lib.frame_format(frame_dtype)                     # ValueError for an unsupported dtype, before any work
