@@ -165,6 +165,20 @@ SMK_API int smk_jacobi_obst(const smk_grid_t* g, const float* div, float* p, flo
 
 /* a7  gradient subtract in place (navier_stokes.py:148-149) */
 SMK_API int smk_project(const smk_grid_t* g, const float* p, float* u, float* v, float dt, void* stream);
+/*     the same with solid cells (DESIGN.md s5.7): solid as smk_jacobi_obst (may be NULL: smk_project); with a mask the subtract
+ *     runs on open faces only (a face of u or v is closed when a cell it touches is solid).  A misaligned mask or a stride other
+ *     than 0 or h * pitch_c is SMK_EINVAL before anything is enqueued; a mask on a slab grid is SMK_EUNSUPPORTED. */
+SMK_API int smk_project_ex(const smk_grid_t* g, const float* p, float* u, float* v, float dt, const uint8_t* solid,
+                           int64_t solid_batch_stride, void* stream);
+/*     the closed faces of u and v := +0.0 (solid as smk_project_ex, required).  div != NULL: then div := the divergence of the closed
+ *     fields ((u[i+1][j] - u[i][j]) + v[i][j+1]) - v[i][j]) / dt (O1 of a masked step); div == NULL: the faces only (O4).  On
+ *     gradients of u and v it is its own transpose (a store of +0.0). */
+SMK_API int smk_obstacle_faces(const smk_grid_t* g, float* u, float* v, float* div, const uint8_t* solid, int64_t solid_batch_stride,
+                               float dt, void* stream);
+/*     d and frame (may be NULL; [batch][h][pitch_c] in frame_format, frame_stride elements apart) := +0.0 on solid cells (O3 of a
+ *     masked step, and its transpose on gradients). */
+SMK_API int smk_obstacle_cells(const smk_grid_t* g, float* d, void* frame, int64_t frame_stride, int32_t frame_format,
+                               const uint8_t* solid, int64_t solid_batch_stride, void* stream);
 
 /* a8  bilinear_interpolate (navier_stokes.py:111-131) at n arbitrary (y, x); mode 0 plain,
  *     1 = interpolate_velocity_u (x+0.5 clamped, :97-102), 2 = interpolate_velocity_v (y+0.5 clamped, :104-109) */
@@ -414,16 +428,29 @@ SMK_API int smk_advect_adjoint(const smk_grid_t* g, const float* field, int32_t 
  *     The gradients of u and v pass through unchanged. */
 SMK_API int smk_project_adjoint(const smk_grid_t* g, const float* g_u, const float* g_v, const float* g_p_in, float* g_p, float dt,
                                 void* stream);
+/*     the same through smk_project_ex with solid cells (solid as there; NULL is smk_project_adjoint): closed faces add nothing. */
+SMK_API int smk_project_adjoint_ex(const smk_grid_t* g, const float* g_u, const float* g_v, const float* g_p_in, float* g_p, float dt,
+                                   const uint8_t* solid, int64_t solid_batch_stride, void* stream);
 /*     adjoint of K Jacobi sweeps (smk_jacobi): from the gradient g_p_in of the swept pressure, g_p (of the pressure before the sweeps,
  *     ring cells included) and g_div (of the divergence).  T as smk_jacobi.  workspace: 5 fields of batch * F floats, F = stride_c
  *     (h * pitch_c when batch == 1), 16-byte aligned; NULL allowed when K == 0. */
 SMK_API int smk_jacobi_adjoint(const smk_grid_t* g, const float* g_p_in, float* g_p, float* g_div, int32_t K, int32_t T,
                                float* workspace, void* stream);
+/*     adjoint of smk_jacobi_obst (solid as there; NULL is smk_jacobi_adjoint): the same two sweep chains on the masked sweep, with
+ *     r = g_p_in on fluid interior cells; g_p and g_div are exactly 0 on solid cells (g_p for K >= 1). */
+SMK_API int smk_jacobi_adjoint_ex(const smk_grid_t* g, const float* g_p_in, float* g_p, float* g_div, int32_t K, int32_t T,
+                                  float* workspace, const uint8_t* solid, int64_t solid_batch_stride, void* stream);
 /*     adjoint of smk_forces_diffuse_div: from the gradients of (u_out, v_out, d_out, div), those of (u, v, d) before the buoyancy and
  *     the diffusions.  Outputs must not alias inputs. */
 SMK_API int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u_diff, const float* g_v_diff, const float* g_d_diff,
                                            const float* g_div, float* g_u, float* g_v, float* g_d, float dt, float c_uv, float c_d,
                                            void* stream);
+/*     the same for a masked step, whose diffused u and v had their closed faces set to +0.0 before the divergence (solid as
+ *     smk_project_ex; NULL is smk_forces_diffuse_div_adjoint): the total gradient of a closed face is +0.0 before the diffusion
+ *     transpose gathers it. */
+SMK_API int smk_forces_diffuse_div_adjoint_ex(const smk_grid_t* g, const float* g_u_diff, const float* g_v_diff, const float* g_d_diff,
+                                              const float* g_div, float* g_u, float* g_v, float* g_d, float dt, float c_uv, float c_d,
+                                              const uint8_t* solid, int64_t solid_batch_stride, void* stream);
 /*     intensity gradient of smk_splat_sources: g_intensity[k] = sum over emitter k's footprint of g_density * its splat weight,
  *     for the nsources = offsets[batch] emitters of (sources, offsets); a fixed-order tree per emitter. */
 SMK_API int smk_splat_sources_adjoint(const smk_grid_t* g, const float* g_density, const smk_source_t* sources,

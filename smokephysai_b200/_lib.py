@@ -103,6 +103,9 @@ SIGNATURES = {
     "smk_jacobi_obst": [GP, c_p, c_p, c_p, c_p, c_i64, c_i32, c_i32, C.POINTER(c_i32), c_p],
     "smk_jacobi_residual_ex": [GP, c_p, c_p, c_p, c_i64, c_p, c_p],
     "smk_add_forcing": [GP, c_p, c_p, c_p, c_p, c_p],
+    "smk_project_ex": [GP, c_p, c_p, c_p, c_f, c_p, c_i64, c_p],
+    "smk_obstacle_faces": [GP, c_p, c_p, c_p, c_p, c_i64, c_f, c_p],
+    "smk_obstacle_cells": [GP, c_p, c_p, c_i64, c_i32, c_p, c_i64, c_p],
     "smk_step_is_fused": [GP, PP, c_i32, C.POINTER(c_i32)],
     "smk_fused_plan": [c_i32, c_i32, c_i32, C.POINTER(c_i32), c_i32, C.POINTER(c_i32)],
     "smk_div_norms": [GP, c_p, c_p, c_p, c_p],
@@ -128,6 +131,9 @@ SIGNATURES = {
     "smk_project_adjoint": [GP, c_p, c_p, c_p, c_p, c_f, c_p],
     "smk_jacobi_adjoint": [GP, c_p, c_p, c_p, c_i32, c_i32, c_p, c_p],
     "smk_forces_diffuse_div_adjoint": [GP, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_f, c_f, c_p],
+    "smk_project_adjoint_ex": [GP, c_p, c_p, c_p, c_p, c_f, c_p, c_i64, c_p],
+    "smk_jacobi_adjoint_ex": [GP, c_p, c_p, c_p, c_i32, c_i32, c_p, c_p, c_i64, c_p],
+    "smk_forces_diffuse_div_adjoint_ex": [GP, c_p, c_p, c_p, c_p, c_p, c_p, c_p, c_f, c_f, c_f, c_p, c_i64, c_p],
     "smk_splat_sources_adjoint": [GP, c_p, c_p, c_p, c_i32, c_p, c_p],
     "smk_splat_sources_adjoint_ex": [GP, c_p, c_p, c_p, c_i32, c_i32, c_p, c_p],
 }

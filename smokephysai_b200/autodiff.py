@@ -38,6 +38,13 @@ NavierStokesSimulator.run_steps(forcing=) does, and the forward is that call bit
 recompute adds row t to copies of S_t.u and S_t.v (smk_add_forcing).  The add passes the gradient unchanged, so after reverse step t
 G.u / G.v is the gradient of u / v at the head of step t: that of S_t and of du_t / dv_t alike.  A per-step forcing's gradient row t
 is that value; a constant forcing's is the sum over steps, accumulated with smk_add_forcing for t = T-1 down to 0 in that order.
+
+Solid obstacles (rollout(..., obstacles=mask)): the simulator applies the mask (set_obstacles), so the forward is set_obstacles +
+run_steps bit for bit.  The recompute adds O1 (smk_obstacle_faces), the masked subtract (smk_project_ex) and the advected u before O4
+(smk_advect; S_{t+1}.u is after O4, and the v advection read the u before it): one extra u-shaped buffer.  The reverse zeroes the
+solid cells of G.d and of the step's frame gradient (O3^T, smk_obstacle_cells) before the density advection's adjoint and the closed
+faces of G.u, G.v (O4^T) after it, and runs the masked project, Jacobi and diffusion adjoints (the *_adjoint_ex entries, DESIGN.md
+s5.7).  The mask is not differentiable.
 """
 import ctypes as C
 
@@ -45,7 +52,7 @@ import torch
 
 from . import _lib
 from .fractal_generator import FractalGenerator
-from .navier_stokes import FieldLayout, NavierStokesSimulator, pack_forcing, pack_schedule, schedule_offsets
+from .navier_stokes import FieldLayout, NavierStokesSimulator, check_obstacles, pack_forcing, pack_schedule, schedule_offsets
 
 __all__ = ["rollout", "add_sources"]
 
@@ -105,6 +112,8 @@ class _Config:
         self.src = None                 # continuous sources: (int32 [n, 4] device records with the intensities, offsets, n)
         self.sched = None               # schedule: (int32 [T * B * E, 4] device records with the intensities, offsets [T * B + 1], E)
         self.force = None               # forcing: (du, dv, per_step) of pack_forcing, padded [(T | 1), B, rows, pitch] device buffers
+        self.obstacles = None           # solid cells: the mask checked by check_obstacles, [h, w] or [B, h, w]
+        self.solid = None               # (device buffer, batch stride) of the mask set_obstacles uploaded, set by simulator()
 
     def simulator(self, state):
         sim = NavierStokesSimulator((self.h, self.w), self.dt, self.viscosity, self.device, jacobi_iters=self.jacobi_iters,
@@ -115,6 +124,9 @@ class _Config:
             live[:, :, :cols] = t.detach().reshape(self.B, rows, cols)
         if self.src is not None:
             sim._csrc = (None, self.src[0], self.src[1])          # set_continuous_sources with records already on the device
+        if self.obstacles is not None:
+            sim.set_obstacles(self.obstacles)
+            self.solid = sim._solid[1:]                           # the reverse reads this buffer after the simulator is gone
         return sim
 
     def step_sched(self, t0):
@@ -233,6 +245,9 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         g_int = torch.zeros(T, B, E, dtype=torch.float32, device=dev)
         row_off = schedule_offsets(1, B, E, dev)                # one row of B lists of E entries, for the per-step adjoint
         dsp = zeros("d")
+    solid = (cfg.solid[0].data_ptr(), cfg.solid[1]) if cfg.obstacles is not None else None
+    if solid is not None:
+        ua = zeros("u")                                         # the advected u before O4, the v advection's velocity
     g_force = None
     if cfg.force is not None:
         fu, fv, per_step = cfg.force
@@ -254,14 +269,27 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
         # recompute: buoyancy + diffusions, then the gradient subtract with the pressure the step projected with
         _lib.call("smk_forces_diffuse_div", gp, u0.data_ptr(), v0.data_ptr(), d0.data_ptr(), ud.data_ptr(), vd.data_ptr(),
                   dd.data_ptr(), None, dt, c_uv, c_d, s)
-        _lib.call("smk_project", gp, p1.data_ptr(), ud.data_ptr(), vd.data_ptr(), dt, s)
+        if solid is None:
+            _lib.call("smk_project", gp, p1.data_ptr(), ud.data_ptr(), vd.data_ptr(), dt, s)
+            u_adv = u1
+        else:
+            # O1 on the diffused u, v; the subtract on open faces; the advected u before O4 (S_{t+1}.u is after it)
+            _lib.call("smk_obstacle_faces", gp, ud.data_ptr(), vd.data_ptr(), None, *solid, dt, s)
+            _lib.call("smk_project_ex", gp, p1.data_ptr(), ud.data_ptr(), vd.data_ptr(), dt, *solid, s)
+            _lib.call("smk_advect", gp, ud.data_ptr(), ua.data_ptr(), rows_u, L.w, L.pitch_u, L.stride_u, ud.data_ptr(), vd.data_ptr(),
+                      dt, 1.0, None, 0, None, s)
+            u_adv = ua
         gft = gF[:, t] if gF is not None else None
+        if solid is not None:                                   # O3^T: the solid cells' density and frame were set to +0.0
+            _lib.call("smk_obstacle_cells", gp, G["d"].data_ptr(), _ptr(gft), T * L.h * L.pitch_c, 0, *solid, s)
         # 1. density advection (+ decay, frame, fractal): field d_diff by (u_adv, v_adv) = (S_{t+1}.u, S_{t+1}.v)
         _lib.call("smk_advect_adjoint", gp, dd.data_ptr(), rows_c, L.w, L.pitch_c, L.stride_c, u1.data_ptr(), v1.data_ptr(),
                   dt, prm.decay, G["d"].data_ptr(), _ptr(gft), T * L.h * L.pitch_c, _ptr(fmul) if gft is not None else None,
                   gdd.data_ptr(), 0, G["u"].data_ptr(), G["v"].data_ptr(), ws_adv.data_ptr(), s)
+        if solid is not None:                                   # O4^T: the closed faces of the advected u, v were set to +0.0
+            _lib.call("smk_obstacle_faces", gp, G["u"].data_ptr(), G["v"].data_ptr(), None, *solid, dt, s)
         # 2. v advection: field v_proj by (u_adv, v_proj)
-        _lib.call("smk_advect_adjoint", gp, vd.data_ptr(), rows_v, L.w + 1, L.pitch_v, L.stride_v, u1.data_ptr(), vd.data_ptr(),
+        _lib.call("smk_advect_adjoint", gp, vd.data_ptr(), rows_v, L.w + 1, L.pitch_v, L.stride_v, u_adv.data_ptr(), vd.data_ptr(),
                   dt, 1.0, G["v"].data_ptr(), None, 0, None, gvp.data_ptr(), 0, G["u"].data_ptr(), gvp.data_ptr(),
                   ws_adv.data_ptr(), s)
         # 3. u advection: field u_proj by (u_proj, v_proj); G.u is complete now
@@ -269,11 +297,19 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
                   dt, 1.0, G["u"].data_ptr(), None, 0, None, gup.data_ptr(), 0, gup.data_ptr(), gvp.data_ptr(),
                   ws_adv.data_ptr(), s)
         # 4. gradient subtract, 5. Jacobi sweeps, 6. divergence + diffusions + buoyancy
-        _lib.call("smk_project_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), G["p"].data_ptr(), gpk.data_ptr(), dt, s)
-        _lib.call("smk_jacobi_adjoint", gp, gpk.data_ptr(), Gn["p"].data_ptr(), gdiv.data_ptr(), cfg.jacobi_iters,
-                  cfg.sweeps_per_launch, ws_jac.data_ptr(), s)
-        _lib.call("smk_forces_diffuse_div_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), gdd.data_ptr(), gdiv.data_ptr(),
-                  Gn["u"].data_ptr(), Gn["v"].data_ptr(), Gn["d"].data_ptr(), dt, c_uv, c_d, s)
+        #    (with solid cells: open faces only, the masked sweeps, and O1^T inside the diffusion transpose)
+        if solid is None:
+            _lib.call("smk_project_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), G["p"].data_ptr(), gpk.data_ptr(), dt, s)
+            _lib.call("smk_jacobi_adjoint", gp, gpk.data_ptr(), Gn["p"].data_ptr(), gdiv.data_ptr(), cfg.jacobi_iters,
+                      cfg.sweeps_per_launch, ws_jac.data_ptr(), s)
+            _lib.call("smk_forces_diffuse_div_adjoint", gp, gup.data_ptr(), gvp.data_ptr(), gdd.data_ptr(), gdiv.data_ptr(),
+                      Gn["u"].data_ptr(), Gn["v"].data_ptr(), Gn["d"].data_ptr(), dt, c_uv, c_d, s)
+        else:
+            _lib.call("smk_project_adjoint_ex", gp, gup.data_ptr(), gvp.data_ptr(), G["p"].data_ptr(), gpk.data_ptr(), dt, *solid, s)
+            _lib.call("smk_jacobi_adjoint_ex", gp, gpk.data_ptr(), Gn["p"].data_ptr(), gdiv.data_ptr(), cfg.jacobi_iters,
+                      cfg.sweeps_per_launch, ws_jac.data_ptr(), *solid, s)
+            _lib.call("smk_forces_diffuse_div_adjoint_ex", gp, gup.data_ptr(), gvp.data_ptr(), gdd.data_ptr(), gdiv.data_ptr(),
+                      Gn["u"].data_ptr(), Gn["v"].data_ptr(), Gn["d"].data_ptr(), dt, c_uv, c_d, *solid, s)
         G, Gn = Gn, G
         # G.d: the gradient of the splatted density, which is also that of S_t.d
         if cfg.src is not None:
@@ -300,7 +336,7 @@ def _reverse(cfg, ck, L, prm, fmul, g_frames, g_out):
 
 
 def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fractal=False, step_kernel="auto",
-            sweeps_per_launch=0, sources=None, intensities=None, schedule=None, forcing=None):
+            sweeps_per_launch=0, sources=None, intensities=None, schedule=None, forcing=None, obstacles=None):
     """nsteps steps of NavierStokesSimulator from state = (u, v, p, d); differentiable with respect to all four fields.
 
     u [.., h+1, w], v [.., h, w+1], p [.., h, w], d [.., h, w]: float32 CUDA tensors on one device, with an optional leading
@@ -319,7 +355,12 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
 
     forcing = (du, dv): velocity increments added at the head of every step (run_steps(forcing=)), float32 tensors on the state's
     device: du [.., h+1, w] and dv [.., h, w+1] in the state's shapes for a constant forcing, or with a leading T = nsteps axis for
-    a per-step one; differentiable with respect to du and dv.  It combines with sources= and schedule=."""
+    a per-step one; differentiable with respect to du and dv.  It combines with sources= and schedule=.
+
+    obstacles: solid cells, [h, w] (every simulation) or [B, h, w], bool or integers 0 / 1 (1 = solid), as a numpy array, a CPU
+    tensor or a tensor on the state's device, applied at every step as NavierStokesSimulator.set_obstacles does (DESIGN.md s5.7);
+    the mask is not differentiable.  It combines with sources=, schedule=, forcing= and add_fractal, not with
+    step_kernel="fused" (ValueError)."""
     batch, h, w, device = _check_state(state)
     if int(nsteps) < 1:
         raise ValueError("nsteps must be >= 1, got %r" % (nsteps,))
@@ -328,6 +369,10 @@ def rollout(state, nsteps, *, dt=0.01, viscosity=0.001, jacobi_iters=20, add_fra
     if step_kernel not in _lib.STEP_KERNELS:
         raise ValueError("step_kernel must be one of %s, got %r" % (sorted(_lib.STEP_KERNELS), step_kernel))
     cfg = _Config(batch, h, w, device, nsteps, dt, viscosity, jacobi_iters, add_fractal, step_kernel, sweeps_per_launch)
+    if obstacles is not None:
+        if step_kernel == "fused":
+            raise ValueError('obstacles run on the phase kernels: they do not combine with step_kernel="fused"')
+        cfg.obstacles = check_obstacles(obstacles, h, w, cfg.B, device)
     if sources is not None and schedule is not None:
         raise ValueError("sources= and schedule= do not combine: fold the constant emitters into the schedule")
     if sources is None and schedule is None and intensities is not None:

@@ -117,6 +117,16 @@ int check_grid(const smk_grid_t* g, const char* who)
     return SMK_OK;
 }
 
+int check_solid(const smk_grid_t* g, const uint8_t* solid, int64_t solid_stride, const char* who)
+{
+    if (solid && reinterpret_cast<uintptr_t>(solid) % 4) return fail(SMK_EINVAL, "%s: solid is not 4-byte aligned", who);
+    if (solid_stride != 0 && (!solid || solid_stride != (int64_t)g->h * g->pitch_c))
+        return fail(SMK_EINVAL, "%s: solid_batch_stride must be 0 or h * pitch_c (%lld) with a mask, got %lld", who,
+                    (long long)g->h * g->pitch_c, (long long)solid_stride);
+    if (solid && g->gh != 0) return fail(SMK_EUNSUPPORTED, "%s: solid cells are not available on a slab grid (gh != 0)", who);
+    return SMK_OK;
+}
+
 static int check_ptrs(const char* who, std::initializer_list<const void*> ps)
 {
     int k = 0;
@@ -279,6 +289,42 @@ int smk_project(const smk_grid_t* g, const float* p, float* u, float* v, float d
     SMK_TRY(check_grid(g, "smk_project"));
     SMK_TRY(check_ptrs("smk_project", {p, u, v}));
     return launch_project(g, p, u, v, dt, (cudaStream_t)stream);
+}
+
+int smk_project_ex(const smk_grid_t* g, const float* p, float* u, float* v, float dt, const uint8_t* solid, int64_t solid_batch_stride,
+                   void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_project_ex"));
+    SMK_TRY(check_ptrs("smk_project_ex", {p, u, v}));
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_project_ex"));
+    if (!solid) return launch_project(g, p, u, v, dt, (cudaStream_t)stream);
+    return launch_project_obst(g, p, u, v, solid, solid_batch_stride, dt, (cudaStream_t)stream);
+}
+
+int smk_obstacle_faces(const smk_grid_t* g, float* u, float* v, float* div, const uint8_t* solid, int64_t solid_batch_stride, float dt,
+                       void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_obstacle_faces"));
+    SMK_TRY(check_ptrs("smk_obstacle_faces", {u, v}));
+    if (!solid) return fail(SMK_EINVAL, "smk_obstacle_faces: solid is NULL");
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_obstacle_faces"));
+    if (div && !aligned16(div)) return fail(SMK_EINVAL, "smk_obstacle_faces: div is not 16-byte aligned");
+    if (div && !(dt != 0.0f)) return fail(SMK_EINVAL, "smk_obstacle_faces: dt must be non-zero");
+    return launch_obstacle_faces(g, u, v, div, solid, solid_batch_stride, dt, (cudaStream_t)stream);
+}
+
+int smk_obstacle_cells(const smk_grid_t* g, float* d, void* frame, int64_t frame_stride, int32_t frame_format, const uint8_t* solid,
+                       int64_t solid_batch_stride, void* stream)
+{
+    SMK_TRY(check_grid(g, "smk_obstacle_cells"));
+    SMK_TRY(check_ptrs("smk_obstacle_cells", {d}));
+    if (!solid) return fail(SMK_EINVAL, "smk_obstacle_cells: solid is NULL");
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_obstacle_cells"));
+    if (frame_format != SMK_FRAME_F32 && frame_format != SMK_FRAME_F16 && frame_format != SMK_FRAME_BF16)
+        return fail(SMK_EINVAL, "smk_obstacle_cells: bad frame_format %d", frame_format);
+    if (frame && g->batch > 1 && frame_stride < (int64_t)g->h * g->pitch_c)
+        return fail(SMK_EINVAL, "smk_obstacle_cells: frame_stride smaller than one frame");
+    return launch_obstacle_cells(g, d, frame, frame_stride, frame_format, solid, solid_batch_stride, (cudaStream_t)stream);
 }
 
 int smk_bilerp(const float* field, int32_t rows, int32_t cols, int32_t pitch, const float* y, const float* x,

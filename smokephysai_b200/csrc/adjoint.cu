@@ -179,6 +179,25 @@ k_project_adj(const float* __restrict__ gU, const float* __restrict__ gV, const 
     gP[k] = gp + dt * ((un - uc) + (vn - vc));
 }
 
+// With solid cells (k_project_obst subtracts on open faces only): a closed face contributes nothing to g_p.
+__global__ void __launch_bounds__(256)
+k_project_adj_obst(const float* __restrict__ gU, const float* __restrict__ gV, const float* __restrict__ gPin, float* __restrict__ gP,
+                   const uint8_t* __restrict__ S, const int h, const int w, const int pu, const int pv, const int pc,
+                   const long long su, const long long sv, const long long sc, const long long ss, const float dt)
+{
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    if (i >= h || j >= w) return;
+    const size_t b = blockIdx.z;
+    gU += b * su; gV += b * sv; S += b * ss;
+    const float un = i + 1 <= h - 1 && !u_closed(S, h, pc, i + 1, j) ? gU[(size_t)(i + 1) * pu + j] : 0.0f;
+    const float uc = i >= 1 && !u_closed(S, h, pc, i, j) ? gU[(size_t)i * pu + j] : 0.0f;
+    const float vn = j + 1 <= w - 1 && !v_closed(S, w, pc, i, j + 1) ? gV[(size_t)i * pv + j + 1] : 0.0f;
+    const float vc = j >= 1 && !v_closed(S, w, pc, i, j) ? gV[(size_t)i * pv + j] : 0.0f;
+    const size_t k = b * sc + (size_t)i * pc + j;
+    const float gp = gPin ? gPin[k] : 0.0f;
+    gP[k] = gp + dt * ((un - uc) + (vn - vc));
+}
+
 // ---- a6 adjoint: K Jacobi sweeps (navier_stokes.py:139-145) ------------------------------------------------------------
 // A sweep is p' = J0 p - 0.25*M*div with J0 = M*0.25*S (M: interior mask, S: 4-neighbour sum).  With r = M*g:
 //   g_div = -0.25 * sum_{j<K} J0^j r          g_p = 0.25 * S * J0^(K-1) r   (ring cells of p included)
@@ -214,6 +233,48 @@ k_jacobi_adj_out(const float* __restrict__ y, const float* __restrict__ sum, flo
     gDiv[k] = -0.25f * sum[k];
 }
 
+// With solid cells (k_jacobi_obst, DESIGN.md s5.7).  A masked sweep is p' = J p - 0.25*M*div with M the fluid-interior mask and
+// J = M*A, A[c][n] = 0.25 for each fluid neighbour n of c and A[c][c] = 0.25 * (the number of solid neighbours of c).  A restricted
+// to fluid-interior cells is symmetric, so M J^T M = M J M and, with r = M*g, the two chains above carry over on k_jacobi_obst:
+//   g_div = -0.25 * sum_{j<K} J^j r          g_p = J^T J^(K-1) r
+// y = J^(K-1) r is 0 off the fluid interior, so J^T y at a fluid cell n is the forward's stencil read backwards: each neighbour
+// slot takes y of a fluid neighbour, or y_n itself where the neighbour is solid (its Neumann ghost value); solid cells get 0.
+__global__ void __launch_bounds__(256)
+k_jacobi_adj_prep_obst(const float* __restrict__ g, float* __restrict__ r, float* __restrict__ nd, const uint8_t* __restrict__ S,
+                       const int h, const int w, const int pc, const long long sc, const long long ss)
+{
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    if (i >= h || j >= w) return;
+    const size_t k = blockIdx.z * (size_t)sc + (size_t)i * pc + j;
+    const bool keep = i >= 1 && i <= h - 2 && j >= 1 && j <= w - 2 && S[blockIdx.z * (size_t)ss + (size_t)i * pc + j] == 0;
+    const float x = keep ? g[k] : 0.0f;
+    r[k] = x;
+    if (nd) nd[k] = -4.0f * x;
+}
+
+__global__ void __launch_bounds__(256)
+k_jacobi_adj_out_obst(const float* __restrict__ y, const float* __restrict__ sum, float* __restrict__ gP, float* __restrict__ gDiv,
+                      const uint8_t* __restrict__ S, const int h, const int w, const int pc, const long long sc, const long long ss)
+{
+    const int j = blockIdx.x * 32 + threadIdx.x, i = blockIdx.y * 8 + threadIdx.y;
+    if (i >= h || j >= w) return;
+    const size_t base = blockIdx.z * (size_t)sc, c = (size_t)i * pc + j, k = base + c;
+    const float* Y = y + base;
+    S += blockIdx.z * (size_t)ss;
+    gDiv[k] = -0.25f * sum[k];
+    if (S[c]) {
+        gP[k] = 0.0f;
+        return;
+    }
+    const float yc = Y[c];
+    const float up = i >= 1 ? (S[c - pc] ? yc : Y[c - pc]) : 0.0f, dn = i + 1 < h ? (S[c + pc] ? yc : Y[c + pc]) : 0.0f;
+    const float lf = j >= 1 ? (S[c - 1] ? yc : Y[c - 1]) : 0.0f, rt = j + 1 < w ? (S[c + 1] ? yc : Y[c + 1]) : 0.0f;
+    float s = up + dn;
+    s = s + lf;
+    s = s + rt;
+    gP[k] = 0.25f * s;
+}
+
 // ---- a3 + a4 + a5 adjoint: buoyancy (:154-155), the three diffusions (:158-160) and the divergence (:136) --------------
 // Divergence: div[i][j] = (((u[i+1][j] - u[i][j]) + v[i][j+1]) - v[i][j]) / dt, so the u_diff / v_diff gradients gain the
 // shifted differences of q = g_div / dt.  Diffusion f' = f + c*(S_clamped f - 4f) with replicate padding: its transpose
@@ -240,25 +301,30 @@ __device__ __forceinline__ float gtot_v(const DiffAdjIn& A, int a, int b)
 }
 __device__ __forceinline__ float gtot_d(const DiffAdjIn& A, int a, int b) { return A.gDd[(size_t)a * A.pc + b]; }
 
-template <int KIND>
-__device__ __forceinline__ float gtot(const DiffAdjIn& A, int a, int b)
+// OBST (solid cells S of this simulation): O1 set the closed faces of u_diff / v_diff to +0.0 before the divergence and the
+// gradient subtract read them, so the total gradient of a closed face is +0.0 before the diffusion transpose gathers it
+template <int KIND, bool OBST = false>
+__device__ __forceinline__ float gtot(const DiffAdjIn& A, int a, int b, const uint8_t* S = nullptr)
 {
+    if (OBST && KIND == 0 && u_closed(S, A.h, A.pc, a, b)) return 0.0f;
+    if (OBST && KIND == 1 && v_closed(S, A.w, A.pc, a, b)) return 0.0f;
     return KIND == 0 ? gtot_u(A, a, b) : (KIND == 1 ? gtot_v(A, a, b) : gtot_d(A, a, b));
 }
 
 // transpose of diffusion_step (navier_stokes.py:50-72) on a rows x cols field at (a, b)
-template <int KIND>
-__device__ __forceinline__ float diffuse_adj(const DiffAdjIn& A, int rows, int cols, int a, int b, float c)
+template <int KIND, bool OBST = false>
+__device__ __forceinline__ float diffuse_adj(const DiffAdjIn& A, int rows, int cols, int a, int b, float c,
+                                             const uint8_t* S = nullptr)
 {
-    const float g = gtot<KIND>(A, a, b), t = c * g;
+    const float g = gtot<KIND, OBST>(A, a, b, S), t = c * g;
     float s = 0.0f;
-    if (a + 1 < rows) s = s + c * gtot<KIND>(A, a + 1, b);          // (a, b) is the upper tap of (a+1, b)
+    if (a + 1 < rows) s = s + c * gtot<KIND, OBST>(A, a + 1, b, S);          // (a, b) is the upper tap of (a+1, b)
     if (a == 0) s = s + t;                                           // ... and its own, clamped
-    if (a >= 1) s = s + c * gtot<KIND>(A, a - 1, b);                 // lower tap of (a-1, b)
+    if (a >= 1) s = s + c * gtot<KIND, OBST>(A, a - 1, b, S);                 // lower tap of (a-1, b)
     if (a == rows - 1) s = s + t;
-    if (b + 1 < cols) s = s + c * gtot<KIND>(A, a, b + 1);           // left tap of (a, b+1)
+    if (b + 1 < cols) s = s + c * gtot<KIND, OBST>(A, a, b + 1, S);           // left tap of (a, b+1)
     if (b == 0) s = s + t;
-    if (b >= 1) s = s + c * gtot<KIND>(A, a, b - 1);                 // right tap of (a, b-1)
+    if (b >= 1) s = s + c * gtot<KIND, OBST>(A, a, b - 1, S);                 // right tap of (a, b-1)
     if (b == cols - 1) s = s + t;
     return g + (s - 4.0f * t);
 }
@@ -278,6 +344,30 @@ k_forces_diffuse_div_adj(DiffAdjIn A, float* __restrict__ gU, float* __restrict_
         gV[n * sv + (size_t)a * A.pv + b] = gv;
         if (b <= w - 1) {
             const float gd = diffuse_adj<2>(A, h, w, a, b, c_d);
+            gD[n * sc + (size_t)a * A.pc + b] = gd + (A.dt * gv) * 0.1f;
+        }
+    }
+}
+
+// k_forces_diffuse_div_adj of a masked step (solid cells S, simulation n at S + n * ss); kept a separate kernel so that the one
+// above, which runs on every unmasked reverse step, compiles exactly as it did
+__global__ void __launch_bounds__(256)
+k_forces_diffuse_div_adj_obst(DiffAdjIn A, float* __restrict__ gU, float* __restrict__ gV, float* __restrict__ gD,
+                              const long long su, const long long sv, const long long sc, const float c_uv, const float c_d,
+                              const uint8_t* __restrict__ S, const long long ss)
+{
+    const int b = blockIdx.x * 32 + threadIdx.x, a = blockIdx.y * 8 + threadIdx.y;
+    const size_t n = blockIdx.z;
+    const int h = A.h, w = A.w;
+    if (a > h || b > w) return;
+    A.gUd += n * su; A.gVd += n * sv; A.gDd += n * sc; A.gDiv += n * sc;
+    S += n * ss;
+    if (b <= w - 1) gU[n * su + (size_t)a * A.pu + b] = diffuse_adj<0, true>(A, h + 1, w, a, b, c_uv, S);
+    if (a <= h - 1) {
+        const float gv = diffuse_adj<1, true>(A, h, w + 1, a, b, c_uv, S);
+        gV[n * sv + (size_t)a * A.pv + b] = gv;
+        if (b <= w - 1) {
+            const float gd = diffuse_adj<2, true>(A, h, w, a, b, c_d, S);
             gD[n * sc + (size_t)a * A.pc + b] = gd + (A.dt * gv) * 0.1f;
         }
     }
@@ -382,28 +472,50 @@ int smk_advect_adjoint(const smk_grid_t* g, const float* field, int32_t rows, in
 
 int smk_project_adjoint(const smk_grid_t* g, const float* g_u, const float* g_v, const float* g_p_in, float* g_p, float dt, void* stream)
 {
+    return smk_project_adjoint_ex(g, g_u, g_v, g_p_in, g_p, dt, nullptr, 0, stream);
+}
+
+int smk_project_adjoint_ex(const smk_grid_t* g, const float* g_u, const float* g_v, const float* g_p_in, float* g_p, float dt,
+                           const uint8_t* solid, int64_t solid_batch_stride, void* stream)
+{
     SMK_TRY(adj_grid(g, "smk_project_adjoint"));
     if (!g_u || !g_v || !g_p) return fail(SMK_EINVAL, "smk_project_adjoint: NULL pointer");
     if (g_p == g_u || g_p == g_v) return fail(SMK_EINVAL, "smk_project_adjoint: g_p aliases g_u or g_v");
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_project_adjoint_ex"));
     cudaStream_t s = (cudaStream_t)stream;
     ProfScope prof_(SMK_PH_OTHER, s);
-    k_project_adj<<<cells_grid(g->h, g->w, g->batch), dim3(32, 8), 0, s>>>(g_u, g_v, g_p_in, g_p, g->h, g->w, g->pitch_u, g->pitch_v,
-                                                                          g->pitch_c, g->stride_u, g->stride_v, g->stride_c, dt);
+    const dim3 grid = cells_grid(g->h, g->w, g->batch), blk(32, 8);
+    if (solid) {
+        k_project_adj_obst<<<grid, blk, 0, s>>>(g_u, g_v, g_p_in, g_p, solid, g->h, g->w, g->pitch_u, g->pitch_v, g->pitch_c,
+                                                g->stride_u, g->stride_v, g->stride_c, solid_batch_stride, dt);
+        return check_launch("k_project_adj_obst");
+    }
+    k_project_adj<<<grid, blk, 0, s>>>(g_u, g_v, g_p_in, g_p, g->h, g->w, g->pitch_u, g->pitch_v, g->pitch_c, g->stride_u, g->stride_v,
+                                       g->stride_c, dt);
     return check_launch("k_project_adj");
 }
 
 int smk_jacobi_adjoint(const smk_grid_t* g, const float* g_p_in, float* g_p, float* g_div, int32_t K, int32_t T,
                        float* workspace, void* stream)
 {
+    return smk_jacobi_adjoint_ex(g, g_p_in, g_p, g_div, K, T, workspace, nullptr, 0, stream);
+}
+
+// With solid cells: the prep and output kernels take the mask (k_jacobi_adj_*_obst) and both chains run on k_jacobi_obst.
+int smk_jacobi_adjoint_ex(const smk_grid_t* g, const float* g_p_in, float* g_p, float* g_div, int32_t K, int32_t T,
+                          float* workspace, const uint8_t* solid, int64_t solid_batch_stride, void* stream)
+{
     SMK_TRY(adj_grid(g, "smk_jacobi_adjoint"));
     if (!g_p_in || !g_p || !g_div) return fail(SMK_EINVAL, "smk_jacobi_adjoint: NULL pointer");
     if (K < 0 || T < 0) return fail(SMK_EINVAL, "smk_jacobi_adjoint: negative K or T");
     if (g_p == g_p_in || g_div == g_p_in || g_p == g_div) return fail(SMK_EINVAL, "smk_jacobi_adjoint: outputs must not alias");
     if (K >= 1 && (!workspace || !aligned16(workspace))) return fail(SMK_EINVAL, "smk_jacobi_adjoint: workspace NULL or not 16-byte aligned");
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_jacobi_adjoint_ex"));
     cudaStream_t s = (cudaStream_t)stream;
     const int64_t field = g->batch > 1 ? g->stride_c : (int64_t)g->h * g->pitch_c;
     const size_t bytes = sizeof(float) * (size_t)field * g->batch;
     const dim3 blk(32, 8), grid = cells_grid(g->h, g->w, g->batch);
+    const long long ss = solid_batch_stride;
     cudaError_t e;
     if (K == 0) {                                    // no sweep: p passes through, the divergence has no effect
         e = cudaMemcpyAsync(g_p, g_p_in, bytes, cudaMemcpyDeviceToDevice, s);
@@ -413,6 +525,12 @@ int smk_jacobi_adjoint(const smk_grid_t* g, const float* g_p_in, float* g_p, flo
     if (K == 1) {                                    // J0^0 r = sum_{j<1} J0^j r = r: no sweep
         ProfScope prof_(SMK_PH_OTHER, s);
         float* r = workspace;
+        if (solid) {
+            k_jacobi_adj_prep_obst<<<grid, blk, 0, s>>>(g_p_in, r, nullptr, solid, g->h, g->w, g->pitch_c, field, ss);
+            SMK_TRY(check_launch("k_jacobi_adj_prep_obst"));
+            k_jacobi_adj_out_obst<<<grid, blk, 0, s>>>(r, r, g_p, g_div, solid, g->h, g->w, g->pitch_c, field, ss);
+            return check_launch("k_jacobi_adj_out_obst");
+        }
         k_jacobi_adj_prep<<<grid, blk, 0, s>>>(g_p_in, r, nullptr, g->h, g->w, g->pitch_c, field);
         SMK_TRY(check_launch("k_jacobi_adj_prep"));
         k_jacobi_adj_out<<<grid, blk, 0, s>>>(r, r, g_p, g_div, g->h, g->w, g->pitch_c, field);
@@ -429,21 +547,35 @@ int smk_jacobi_adjoint(const smk_grid_t* g, const float* g_p_in, float* g_p, flo
     if (e != cudaSuccess) return fail((int)e, "smk_jacobi_adjoint: %s", cudaGetErrorString(e));
     {
         ProfScope prof_(SMK_PH_OTHER, s);
-        k_jacobi_adj_prep<<<grid, blk, 0, s>>>(g_p_in, A, ND, g->h, g->w, g->pitch_c, field);
-        SMK_TRY(check_launch("k_jacobi_adj_prep"));
+        if (solid)
+            k_jacobi_adj_prep_obst<<<grid, blk, 0, s>>>(g_p_in, A, ND, solid, g->h, g->w, g->pitch_c, field, ss);
+        else
+            k_jacobi_adj_prep<<<grid, blk, 0, s>>>(g_p_in, A, ND, g->h, g->w, g->pitch_c, field);
+        SMK_TRY(check_launch(solid ? "k_jacobi_adj_prep_obst" : "k_jacobi_adj_prep"));
     }
     smk_grid_t gg = *g;
     gg.stride_c = field;
     int in_b = 0, in_z2 = 0;
-    SMK_TRY(launch_jacobi(&gg, g_div, A, B, K - 1, T, &in_b, s));       // J0^(K-1) r
-    SMK_TRY(launch_jacobi(&gg, ND, Z, Z2, K, T, &in_z2, s));            // sum_{j<K} J0^j r
+    SMK_TRY(launch_jacobi(&gg, g_div, A, B, K - 1, T, &in_b, s, solid, ss));       // J0^(K-1) r
+    SMK_TRY(launch_jacobi(&gg, ND, Z, Z2, K, T, &in_z2, s, solid, ss));            // sum_{j<K} J0^j r
     ProfScope prof_(SMK_PH_OTHER, s);
+    if (solid) {
+        k_jacobi_adj_out_obst<<<grid, blk, 0, s>>>(in_b ? B : A, in_z2 ? Z2 : Z, g_p, g_div, solid, g->h, g->w, g->pitch_c, field, ss);
+        return check_launch("k_jacobi_adj_out_obst");
+    }
     k_jacobi_adj_out<<<grid, blk, 0, s>>>(in_b ? B : A, in_z2 ? Z2 : Z, g_p, g_div, g->h, g->w, g->pitch_c, field);
     return check_launch("k_jacobi_adj_out");
 }
 
 int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u_diff, const float* g_v_diff, const float* g_d_diff,
                                    const float* g_div, float* g_u, float* g_v, float* g_d, float dt, float c_uv, float c_d, void* stream)
+{
+    return smk_forces_diffuse_div_adjoint_ex(g, g_u_diff, g_v_diff, g_d_diff, g_div, g_u, g_v, g_d, dt, c_uv, c_d, nullptr, 0, stream);
+}
+
+int smk_forces_diffuse_div_adjoint_ex(const smk_grid_t* g, const float* g_u_diff, const float* g_v_diff, const float* g_d_diff,
+                                      const float* g_div, float* g_u, float* g_v, float* g_d, float dt, float c_uv, float c_d,
+                                      const uint8_t* solid, int64_t solid_batch_stride, void* stream)
 {
     SMK_TRY(adj_grid(g, "smk_forces_diffuse_div_adjoint"));
     if (!g_u_diff || !g_v_diff || !g_d_diff || !g_div || !g_u || !g_v || !g_d)
@@ -452,11 +584,17 @@ int smk_forces_diffuse_div_adjoint(const smk_grid_t* g, const float* g_u_diff, c
     for (const float* p : ins)
         if (p == g_u || p == g_v || p == g_d) return fail(SMK_EINVAL, "smk_forces_diffuse_div_adjoint: outputs must not alias inputs");
     if (!(dt != 0.0f)) return fail(SMK_EINVAL, "smk_forces_diffuse_div_adjoint: dt must be non-zero");
+    SMK_TRY(check_solid(g, solid, solid_batch_stride, "smk_forces_diffuse_div_adjoint_ex"));
     cudaStream_t s = (cudaStream_t)stream;
     DiffAdjIn A{g_u_diff, g_v_diff, g_d_diff, g_div, g->h, g->w, g->pitch_u, g->pitch_v, g->pitch_c, dt};
     ProfScope prof_(SMK_PH_OTHER, s);
-    k_forces_diffuse_div_adj<<<cells_grid(g->h + 1, g->w + 1, g->batch), dim3(32, 8), 0, s>>>(A, g_u, g_v, g_d, g->stride_u, g->stride_v,
-                                                                                             g->stride_c, c_uv, c_d);
+    const dim3 grid = cells_grid(g->h + 1, g->w + 1, g->batch), blk(32, 8);
+    if (solid) {
+        k_forces_diffuse_div_adj_obst<<<grid, blk, 0, s>>>(A, g_u, g_v, g_d, g->stride_u, g->stride_v, g->stride_c, c_uv, c_d, solid,
+                                                           solid_batch_stride);
+        return check_launch("k_forces_diffuse_div_adj_obst");
+    }
+    k_forces_diffuse_div_adj<<<grid, blk, 0, s>>>(A, g_u, g_v, g_d, g->stride_u, g->stride_v, g->stride_c, c_uv, c_d);
     return check_launch("k_forces_diffuse_div_adj");
 }
 

@@ -45,6 +45,19 @@ __device__ __forceinline__ int clampi(int a, int lo, int hi) { return min(max(a,
 // torch.clamp(x, lo, hi) == min(max(x, lo), hi)
 __device__ __forceinline__ float clampf(float a, float lo, float hi) { return fminf(fmaxf(a, lo), hi); }
 
+// ---- solid obstacles (DESIGN.md s5.7) -------------------------------------------------------------------
+// S: uint8 [batch][h][pitch_c], non-zero = solid, simulation b at S + b * ss (ss = 0: one mask for all).  u face (i, j) lies
+// between cells (i-1, j) and (i, j), v face (i, j) between (i, j-1) and (i, j); a face is closed when a cell it touches that
+// exists is solid.  Closing a face is a store of +0.0 (a multiply by 0 would give -0 or NaN).
+__device__ __forceinline__ bool u_closed(const uint8_t* S, const int h, const int pc, const int i, const int j)
+{
+    return (i >= 1 && S[(size_t)(i - 1) * pc + j] != 0) || (i < h && S[(size_t)i * pc + j] != 0);
+}
+__device__ __forceinline__ bool v_closed(const uint8_t* S, const int w, const int pc, const int i, const int j)
+{
+    return (j >= 1 && S[(size_t)i * pc + j - 1] != 0) || (j < w && S[(size_t)i * pc + j] != 0);
+}
+
 // a8: bilinear_interpolate (navier_stokes.py:111-131) with a sampler f(row, col) over a Hg x Wg field.
 // Corner indices are clamped AFTER the +1 (:116-123), weights come from the clamped corners (:125-128),
 // the sum is ((wa*f00 + wb*f01) + wc*f10) + wd*f11 (:130-131).
@@ -161,6 +174,8 @@ struct ProfScope {
 };
 bool aligned16(const void* p);
 int check_grid(const smk_grid_t* g, const char* who);
+// a solid-cell mask argument pair (solid may be NULL): 4-byte aligned, stride 0 or h * pitch_c, whole grids only
+int check_solid(const smk_grid_t* g, const uint8_t* solid, int64_t solid_stride, const char* who);
 
 // launchers (one per kernel family); all asynchronous on `s`
 int launch_splat(const smk_grid_t* g, float* density, const smk_source_t* src, const int32_t* off, cudaStream_t s);

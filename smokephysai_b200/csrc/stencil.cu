@@ -1355,19 +1355,7 @@ int launch_apply_mul(const float* f, const float* mul, float* out, int rows, int
     return check_launch("k_apply_mul");
 }
 
-// ---- solid obstacles (DESIGN.md s5.7) -------------------------------------------------------------------
-// S: uint8 [batch][h][pitch_c], non-zero = solid, simulation b at S + b * ss (ss = 0: one mask for all).  u face (i, j) lies
-// between cells (i-1, j) and (i, j), v face (i, j) between (i, j-1) and (i, j); a face is closed when a cell it touches that
-// exists is solid.  Closing a face is a store of +0.0 (a multiply by 0 would give -0 or NaN).
-__device__ __forceinline__ bool u_closed(const uint8_t* S, const int h, const int pc, const int i, const int j)
-{
-    return (i >= 1 && S[(size_t)(i - 1) * pc + j] != 0) || (i < h && S[(size_t)i * pc + j] != 0);
-}
-__device__ __forceinline__ bool v_closed(const uint8_t* S, const int w, const int pc, const int i, const int j)
-{
-    return (j >= 1 && S[(size_t)i * pc + j - 1] != 0) || (j < w && S[(size_t)i * pc + j] != 0);
-}
-
+// ---- solid obstacles (DESIGN.md s5.7); u_closed / v_closed are in common.cuh --------------------------------------------
 // O1 (DIV != NULL): close the faces of the diffused u, v and rewrite the divergence from them; O4 (DIV == NULL): close the faces of
 // the advected u, v.  Thread (i, j) owns u face (i, j), v face (i, j) and cell (i, j); it reads a neighbour's face only when that
 // face is open, which no thread writes.
